@@ -2,7 +2,7 @@
 """
 bench.py — denoiser frame-steps/s (sampling) of the FDM hot path on N B200s of one node.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is one diffusion step of the sampler over one batch: UNetVideoModel forward (the whole kernel schedule)
 + the fused posterior update + the step's Gaussian noise draw, i.e. what `diffusion.p_sample` does.  One step
@@ -220,6 +220,24 @@ def config_dict(workload, wl, world):
             "sharding": f"video batch over {world} rank(s), no collective",
             "l2": "flushed between timed steps (192 MB memset outside the event pairs)",
             "weights": "random non-zero init (zero_module tensors re-randomised)"}
+
+
+DUMP_LIMIT_BYTES = 64_000_000 - 4096  # 64 MB in all, .npy headers (128 bytes each) included
+
+
+def dump_outputs(directory, arrays):
+    """Write each tensor as DIR/<name>.npy in float32, in its own shape.  When all of them together exceed DUMP_LIMIT_BYTES, each
+    is cut to a fixed, seeded sample of its flat elements (the same elements on every run for the same shapes)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    total = sum(4 * a.numel() for a in arrays.values())
+    for name, a in arrays.items():
+        out = a.detach().float().cpu()
+        if total > DUMP_LIMIT_BYTES:
+            keep = out.numel() * DUMP_LIMIT_BYTES // total
+            idx = th.randperm(out.numel(), generator=th.Generator().manual_seed(0))[:keep].sort().values
+            out = out.flatten()[idx]
+        np.save(os.path.join(directory, name + ".npy"), out.numpy())
 
 
 def cpu_port_steps(over, B, K, batch, sd, n_steps, warmup, threads):
@@ -637,6 +655,9 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-train", action="store_true")
     ap.add_argument("--no-gpu-eager", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write rank 0's sample and eps of the last timed step to DIR/<name>.npy (float32), so that two builds "
+                         "run with the same arguments can be compared output for output")
     args = ap.parse_args()
     wl = dict(WORKLOADS[args.workload])
     if args.batch > 0:
@@ -647,6 +668,8 @@ def main():
         os.environ["FDM_BENCH_GPU_EAGER"] = "0"
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes what the native timed path computed; --impl reference has no such output")
         run_reference(args, wl, rank, world)
         return
 
@@ -730,6 +753,7 @@ def main():
         errs = [v for k, v in parity.items() if k.startswith("eps_rel_l2")]
         parity["ok"] = bool(errs) and all(e <= tol for e in errs)
 
+    th.manual_seed(1000 + rank)  # the sampler state and step noise below: the same inputs on every run with the same arguments
     P.x_view.normal_()
     P.t_index_view.fill_(diffusion.num_timesteps - 1)
     nbuf.normal_()
@@ -764,6 +788,9 @@ def main():
         evs[k][1].record()
     th.cuda.synchronize()
     clocks.mark_end()
+    if args.dump_outputs and rank == 0:
+        # what p_sample returns for the last timed step, read before the informational passes below reuse the plan's buffers
+        dump_outputs(args.dump_outputs, {"sample": P.x_view, "eps": P.eps_view})
     if world > 1:
         dist.barrier()
     th.cuda.synchronize()

@@ -287,11 +287,14 @@ def factorized_attention(sd, p, x, temb, attn_mask, T, frame_indices, heads, col
     return x.reshape(BT, C, H, W)
 
 
-def unet_forward(sd, cfg, x, x0, timesteps, frame_indices, obs_mask, latent_mask, taps=None):
+def unet_forward(sd, cfg, x, x0, timesteps, frame_indices, obs_mask, latent_mask, taps=None, attns=None):
     """UNetVideoModel.forward, unet.py:428-464.  Returns eps [B,T,C_out,H,W] (fp32).
 
     `taps`, if a dict, receives intermediate activations {layer prefix: NCHW tensor} for kernel-level tests.
+    `attns`, if a dict, receives the attention maps of return_attn_weights=True under "temporal" and "spatial" (rpe.py:128-130: per
+    attention block in forward order, mean over heads, absolute value: [B*HW, T, T] and [B*T, HW, HW]).
     """
+    collect = [] if attns is not None else None
     B, T, C, H, W = x.shape
     mc, heads = cfg["num_channels"], cfg["num_heads"]
     lay = unet_layout(cfg)
@@ -311,7 +314,7 @@ def unet_forward(sd, cfg, x, x0, timesteps, frame_indices, obs_mask, latent_mask
             elif kind == "res":
                 h = res_block(sd, p, h, emb, cfg["use_scale_shift_norm"])
             elif kind == "attn":
-                h = factorized_attention(sd, p, h, emb, mask, T, frame_indices, heads)
+                h = factorized_attention(sd, p, h, emb, mask, T, frame_indices, heads, collect)
             elif kind == "down":
                 h = F.conv2d(h, sd[p + ".op.weight"], sd[p + ".op.bias"], stride=2, padding=1)
             elif kind == "up":
@@ -330,6 +333,9 @@ def unet_forward(sd, cfg, x, x0, timesteps, frame_indices, obs_mask, latent_mask
         h = run(blk, torch.cat([h, hs.pop()], dim=1))
     h = silu(gn32(h, sd["out.0.weight"], sd["out.0.bias"]))
     out = F.conv2d(h, sd["out.2.weight"], sd["out.2.bias"], padding=1)
+    for _, a_t, a_s in collect or ():
+        attns.setdefault("temporal", []).append(a_t.flatten(0, 1).mean(dim=1).abs())
+        attns.setdefault("spatial", []).append(a_s.flatten(0, 1).mean(dim=1).abs())
     return out.view(B, T, -1, H, W)
 
 

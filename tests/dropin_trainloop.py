@@ -1,4 +1,4 @@
-"""Helper run as a SUBPROCESS by tests/test_host_cpu.py (needs /root/reference): the reference's own TrainLoop
+"""Helper run as a SUBPROCESS by tests/test_host_cpu.py (needs a reference checkout, named by FDM_REFERENCE_PATH): the reference's own TrainLoop
 (improved_diffusion/train_util.py, unmodified) driving THIS repo's model + diffusion for two optimizer steps on CPU.
 mpi4py / blobfile / wandb are absent or unwanted here and are stubbed; everything else is the reference's code."""
 import os
@@ -23,7 +23,7 @@ import improved_diffusion  # noqa: E402  (this repo's package; FDM_REFERENCE_PAT
 from improved_diffusion import train_util, unet  # noqa: E402
 from improved_diffusion.script_util import create_model_and_diffusion, model_and_diffusion_defaults  # noqa: E402
 
-assert train_util.__file__.startswith("/root/reference"), train_util.__file__
+assert train_util.__file__.startswith(os.environ["FDM_REFERENCE_PATH"]), train_util.__file__
 assert "_b200" in unet.__file__
 
 os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=sys.argv[1], DIFFUSION_TRAINING_TEST="1")

@@ -1,14 +1,14 @@
 """
-GPU parity against the UNMODIFIED reference running on the same B200 (oracle/_ref, shipped by oracle/make_ref.sh):
+GPU parity at real shapes, and against the UNMODIFIED reference running on the same B200 where a copy of it is present (oracle/_ref):
 
   * eps at the REAL BASELINE.json shapes (cfg4 shard B=8/K=20/nc=64 — the shape bench.py times —, cfg2, cfg3 128 px/nc=128/K=20/B=2,
     cfg5 64 px/nc=128/K=40 at B = 1, 2, 16, and num_res_blocks=2, the reference default): native fp32 mode <= 1e-4, bf16 mode
-    <= 2e-2 against the reference in PyTorch-eager fp32 (TF32 off) — the GPU-side oracle of SURVEY §8c;
-  * the reference's own `sample_video` (scripts/video_sample.py:28-85) driving the native model + diffusion, against the same
-    function driving the reference model + diffusion, same seeds;
-  * the reference's own `TrainLoop` (train_util.py:267-275 run_step) over the native model on the GPU (subprocess helper).
-
-/root/reference is never read here: oracle/ref_loader.py resolves oracle/_ref.
+    <= 2e-2 against the oracle's network (oracle/fdm_oracle.py, the restatement of the reference's forward that the committed goldens
+    of tests/golden pin to the live reference) in PyTorch-eager fp32 on the same GPU (TF32 off) — the GPU-side oracle of SURVEY §8c;
+  * with the reference present: its own `sample_video` (scripts/video_sample.py:28-85) driving the native model + diffusion, against
+    the same function driving the reference model + diffusion, same seeds; its attention maps; its own `TrainLoop`
+    (train_util.py:267-275 run_step) over the native model on the GPU (subprocess helper).  These run the reference's own code, which
+    is not part of this repository, and skip without it.
 """
 import os
 import subprocess
@@ -21,9 +21,9 @@ import torch
 from oracle import fdm_oracle as O
 from oracle import ref_loader as R
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(R.find_ref() is None, reason="oracle/_ref missing: run __graft_entry__.build() (oracle/make_ref.sh) "
-                                                               "in the build container so that the reference travels to the GPU box")]
+pytestmark = pytest.mark.gpu
+needs_reference = pytest.mark.skipif(R.find_ref() is None, reason="runs the reference's own code: needs a reference checkout "
+                                                                  "(oracle/make_ref.sh copies it into oracle/_ref)")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PIXEL = dict(diffusion_space="pixel", pre_encoded=False, pre_encoded_stats_dict=None)
 TOL = {"fp32": 1e-4, "bf16": 2e-2}
@@ -39,19 +39,33 @@ def _exact_fp32_reference():
     torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = old
 
 
-def build_pair(over, seed=1):
-    """(native model, native diffusion, reference model, reference diffusion) with the same deterministic non-zero weights."""
+def build_native(over, seed=1):
+    """(native model, native diffusion, oracle cfg, state dict) with deterministic non-zero weights."""
     from improved_diffusion.script_util import create_model_and_diffusion, model_and_diffusion_defaults
     d = model_and_diffusion_defaults()
     d.update(over)
     d["diffusion_space_kwargs"] = dict(PIXEL)
     model, diffusion = create_model_and_diffusion(**d)
-    ref_model, ref_diffusion = R.create_reference(over)
     cfg = O.make_cfg(**{**{k: d[k] for k in ("image_size", "in_channels", "num_channels", "num_res_blocks")}, **over})
     sd = O.init_state_dict(cfg, seed=seed)
     model.load_state_dict(sd, strict=True)
+    return model.cuda().eval(), diffusion, cfg, sd
+
+
+def build_pair(over, seed=1):
+    """(native model, native diffusion, reference model, reference diffusion) with the same deterministic non-zero weights."""
+    model, diffusion, cfg, sd = build_native(over, seed)
+    ref_model, ref_diffusion = R.create_reference(over)
     ref_model.load_state_dict(sd, strict=True)  # the reference's own strict load: pins the state-dict contract on the way
-    return model.cuda().eval(), diffusion, ref_model.cuda().eval(), ref_diffusion, cfg, sd
+    return model, diffusion, ref_model.cuda().eval(), ref_diffusion, cfg, sd
+
+
+def oracle_eps_on_gpu(sd, cfg, inp, ts):
+    """eps of the oracle's network in fp32 on the GPU (the fixture disables TF32): the reference's forward as restated by
+    oracle/fdm_oracle.py, held to the live reference's outputs by tests/test_oracle_golden.py."""
+    sd_gpu = {k: v.cuda() for k, v in sd.items()}
+    return O.unet_forward(sd_gpu, cfg, inp["x"].cuda(), inp["x0"].cuda(), ts.cuda(), inp["frame_indices"].cuda(),
+                          inp["obs_mask"].cuda(), inp["latent_mask"].cuda())
 
 
 def cuda_kw(inp):
@@ -74,31 +88,51 @@ REAL_SHAPES = [
 ]
 
 
+def _check_eps(label, model, inp, ts, ref):
+    """native fp32 and bf16 eps against `ref` (an fp32 eps on the GPU) at the TOL bounds"""
+    kw = cuda_kw(inp)
+    assert float(ref.abs().mean()) > 1e-2, "vacuous parity: eps ~ 0"
+    for precision in ("fp32", "bf16"):
+        model.precision = precision
+        eps, attn = model(inp["x"].cuda(), timesteps=ts.cuda(), **kw)
+        e = O.rel_l2(eps.cpu(), ref.cpu())
+        print(f"{label} [{precision}] eps rel-L2 = {e:.3e}")
+        assert attn is None and eps.shape == ref.shape
+        assert e <= TOL[precision], (label, precision, e)
+
+
+def _real_shape_inputs(cfg, B, K, n_obs, pads):
+    inp = O.synthetic_inputs(cfg, B, K, n_obs, seed=7, video_len=300, pad_rows=pads)
+    return inp, O.model_timesteps(O.Tables(cfg), torch.tensor([(97 * (b + 1)) % 1000 for b in range(B)]))
+
+
+@needs_reference
 @pytest.mark.parametrize("name,over,B,K,n_obs,pads", REAL_SHAPES, ids=[c[0] for c in REAL_SHAPES])
 def test_eps_at_real_shapes_vs_reference_on_gpu(name, over, B, K, n_obs, pads):
     model, diffusion, ref_model, ref_diffusion, cfg, sd = build_pair(over)
-    inp = O.synthetic_inputs(cfg, B, K, n_obs, seed=7, video_len=300, pad_rows=pads)
-    t = torch.tensor([(97 * (b + 1)) % 1000 for b in range(B)])
-    ts = O.model_timesteps(O.Tables(cfg), t)
-    kw = cuda_kw(inp)
+    inp, ts = _real_shape_inputs(cfg, B, K, n_obs, pads)
     with torch.no_grad():
-        ref, _ = ref_model(inp["x"].cuda(), timesteps=ts.cuda(), **kw)
-        assert float(ref.abs().mean()) > 1e-2, "vacuous parity: reference eps ~ 0"
-        for precision in ("fp32", "bf16"):
-            model.precision = precision
-            eps, attn = model(inp["x"].cuda(), timesteps=ts.cuda(), **kw)
-            e = O.rel_l2(eps.cpu(), ref.cpu())
-            print(f"{name} [{precision}] eps rel-L2 vs reference-on-GPU = {e:.3e}")
-            assert attn is None and eps.shape == ref.shape
-            assert e <= TOL[precision], (name, precision, e)
+        ref, _ = ref_model(inp["x"].cuda(), timesteps=ts.cuda(), **cuda_kw(inp))
+        _check_eps(f"{name} vs reference-on-GPU", model, inp, ts, ref)
     del model, ref_model
     torch.cuda.empty_cache()
 
 
+@pytest.mark.parametrize("name,over,B,K,n_obs,pads", REAL_SHAPES, ids=[c[0] for c in REAL_SHAPES])
+def test_eps_at_real_shapes_vs_oracle_on_gpu(name, over, B, K, n_obs, pads):
+    """The same shapes against the oracle's network (oracle/fdm_oracle.py) in fp32 on the GPU: runs without a reference checkout."""
+    model, diffusion, cfg, sd = build_native(over)
+    inp, ts = _real_shape_inputs(cfg, B, K, n_obs, pads)
+    with torch.no_grad():
+        _check_eps(f"{name} vs oracle-on-GPU", model, inp, ts, oracle_eps_on_gpu(sd, cfg, inp, ts))
+    del model
+    torch.cuda.empty_cache()
+
+
 def test_bench_shape_also_matches_cpu_oracle():
-    """The benchmarked shape once more against the CPU oracle (the restatement pinned by the goldens), closing the chain
-    native == reference-on-GPU == oracle == reference-on-CPU at B=8, K=20, nc=64."""
-    model, diffusion, ref_model, _, cfg, sd = build_pair(LATENT32)
+    """The benchmarked shape once more against the CPU oracle (the restatement of the reference's forward that the goldens pin at
+    the cfg1 shapes), at B=8, K=20, nc=64."""
+    model, diffusion, cfg, sd = build_native(LATENT32)
     inp = O.synthetic_inputs(cfg, 8, 20, 10, seed=0, video_len=300)
     ts = torch.full((8,), 999.0)
     with torch.no_grad():
@@ -116,6 +150,7 @@ def _args(scheme, n_obs, max_frames, max_latent):
                                  max_latent_frames=max_latent, device=torch.device("cuda"), clip_denoised=True, eval_dir=None)
 
 
+@needs_reference
 @pytest.mark.parametrize("scheme,T,n_obs,max_frames,max_latent", [("autoreg", 12, 3, 5, 2), ("hierarchy-2", 20, 4, 8, 4),
                                                                   ("long-range", 11, 2, 6, 3)])
 def test_reference_sample_video_runs_over_the_native_model(scheme, T, n_obs, max_frames, max_latent):
@@ -177,6 +212,7 @@ class _ContentAdaptiveScheme:
         return obs, [lat] * self.B
 
 
+@needs_reference
 def test_adaptive_scheme_on_the_device_resident_buffer():
     """An adaptive scheme (per-row observed sets chosen from the CURRENT samples via set_videos) through video_sampler on the
     device buffer, against the reference's host-loop `sample_video` procedure given the same scheme object type."""
@@ -207,6 +243,7 @@ def test_adaptive_scheme_on_the_device_resident_buffer():
     assert e <= 2e-3
 
 
+@needs_reference
 def test_reference_trainloop_runs_over_the_native_model_on_gpu():
     """The reference's unmodified TrainLoop (forward_backward + optimize_normal + log_step, DDP-wrapped on CUDA) over the native
     model, against the same loop over the reference model on the same GPU: see tests/dropin_trainloop_gpu.py."""
@@ -259,7 +296,7 @@ def test_philox_sampler_matches_torch_noise_sampler_in_distribution():
     """diffusion.noise_mode = 'philox' through p_sample_loop: finite, observed frames untouched, same per-frame statistics as
     the torch-noise sampler on the same weights (different stream, same distribution)."""
     over = dict(image_size=32, in_channels=4, num_channels=32, num_res_blocks=1, diffusion_steps=32, timestep_respacing="8")
-    model, diffusion, _, _, cfg, sd = build_pair(over)
+    model, diffusion, cfg, sd = build_native(over)
     model.precision = "bf16"
     inp = O.synthetic_inputs(cfg, 4, 6, 2, seed=9, video_len=40)
     kw = cuda_kw(inp)
@@ -279,28 +316,28 @@ def test_philox_sampler_matches_torch_noise_sampler_in_distribution():
     assert abs(sa - sb) <= 0.1 * sa
 
 
-@pytest.mark.parametrize("over,B,T,n_obs,pads", [
+ATTN_CASES = [
     (dict(image_size=32, in_channels=4, num_channels=32, num_res_blocks=1, diffusion_steps=32), 2, 5, 2, (1,)),
     (dict(image_size=32, in_channels=4, num_channels=64, num_res_blocks=1, diffusion_steps=1000), 2, 20, 10, ()),
     (dict(image_size=64, in_channels=4, num_channels=128, num_res_blocks=1, diffusion_steps=1000), 1, 40, 20, ()),
-])
-def test_native_attention_maps_match_the_reference(over, B, T, n_obs, pads):
-    """model(..., return_attn_weights=True) (unet.py:454-464, rpe.py:126-131): the head-averaged attention maps of every attention
-    block, produced by the materialising variants of the tcgen05 attention kernels, against the unmodified reference on the GPU."""
-    model, diffusion, ref_model, ref_diffusion, cfg, sd = build_pair(over)
-    model.precision = "bf16"
+]
+
+
+def _attn_inputs(cfg, B, T, n_obs, pads):
     inp = O.synthetic_inputs(cfg, B, T, n_obs, seed=3, video_len=300, pad_rows=pads)
-    ts = O.model_timesteps(O.Tables(cfg), torch.tensor([(53 * (b + 1)) % cfg["diffusion_steps"] for b in range(B)]))
+    return inp, O.model_timesteps(O.Tables(cfg), torch.tensor([(53 * (b + 1)) % cfg["diffusion_steps"] for b in range(B)]))
+
+
+def _check_native_maps(label, model, inp, ts, eps_r, attn_r, attn_c):
+    """model(..., return_attn_weights=True) in bf16 against fp32 maps `attn_r`; `attn_c` = the same maps with bf16 GEMM operands
+    (torch autocast), the calibration of the bound."""
     kw = cuda_kw(inp)
     with torch.no_grad():
-        eps_r, attn_r = ref_model(inp["x"].cuda(), timesteps=ts.cuda(), return_attn_weights=True, **kw)
-        with torch.autocast("cuda", dtype=torch.bfloat16):  # calibration: what bf16 GEMM operands cost the reference's own maps
-            _, attn_c = ref_model(inp["x"].cuda(), timesteps=ts.cuda(), return_attn_weights=True, **kw)
         eps_n, attn_n = model(inp["x"].cuda(), timesteps=ts.cuda(), return_attn_weights=True, **kw)
         eps_plain, none = model(inp["x"].cuda(), timesteps=ts.cuda(), **kw)
     assert none is None and O.rel_l2(eps_n.cpu(), eps_plain.cpu()) <= 1e-3  # the logging plan computes the same eps
     assert O.rel_l2(eps_n.cpu(), eps_r.cpu()) <= TOL["bf16"]
-    assert set(attn_n) == set(attn_r) == {"spatial", "temporal", "mixed"} and attn_n["mixed"] == []
+    assert set(attn_n) == {"spatial", "temporal", "mixed"} and attn_n["mixed"] == []
     plans = model.engine().plans
     assert any(k[-1] for k in plans), "the maps must come from a collect_attn kernel plan, not from the PyTorch expression"
     worst = worst_c = 0.0
@@ -310,14 +347,50 @@ def test_native_attention_maps_match_the_reference(over, B, T, n_obs, pads):
             assert a.shape == r.shape and a.dtype == torch.float32
             e, e_c = O.rel_l2(a.cpu(), r.cpu()), O.rel_l2(c.float().cpu(), r.cpu())
             worst, worst_c = max(worst, e), max(worst_c, e_c)
-            # softmax maps amplify score errors; the bound is what torch's own autocast-bf16 run of the reference gives on
-            # the same map (x1.5), with north_star's 2e-2 as the floor
+            # softmax maps amplify score errors; the bound is what torch's own autocast-bf16 run gives on the same map (x1.5), with
+            # north_star's 2e-2 as the floor
             assert e <= max(2e-2, 1.5 * e_c), (key, tuple(a.shape), e, e_c)
             rows = a.sum(dim=-1)
             assert float((rows - 1).abs().max()) <= 2e-3  # every row of a head-averaged softmax sums to 1
-    print(f"attention maps vs reference-on-GPU: worst rel-L2 {worst:.3e} over 14 maps (B={B}, T={T}); torch autocast-bf16: {worst_c:.3e}")
+    print(f"attention maps vs {label}: worst rel-L2 {worst:.3e} over 14 maps; torch autocast-bf16: {worst_c:.3e}")
 
 
+@needs_reference
+@pytest.mark.parametrize("over,B,T,n_obs,pads", ATTN_CASES)
+def test_native_attention_maps_match_the_reference(over, B, T, n_obs, pads):
+    """model(..., return_attn_weights=True) (unet.py:454-464, rpe.py:126-131): the head-averaged attention maps of every attention
+    block, produced by the materialising variants of the tcgen05 attention kernels, against the unmodified reference on the GPU."""
+    model, diffusion, ref_model, ref_diffusion, cfg, sd = build_pair(over)
+    model.precision = "bf16"
+    inp, ts = _attn_inputs(cfg, B, T, n_obs, pads)
+    kw = cuda_kw(inp)
+    with torch.no_grad():
+        eps_r, attn_r = ref_model(inp["x"].cuda(), timesteps=ts.cuda(), return_attn_weights=True, **kw)
+        with torch.autocast("cuda", dtype=torch.bfloat16):
+            _, attn_c = ref_model(inp["x"].cuda(), timesteps=ts.cuda(), return_attn_weights=True, **kw)
+    assert set(attn_r) == {"spatial", "temporal", "mixed"}
+    _check_native_maps("reference-on-GPU", model, inp, ts, eps_r, attn_r, attn_c)
+
+
+@pytest.mark.parametrize("over,B,T,n_obs,pads", ATTN_CASES)
+def test_native_attention_maps_match_the_oracle(over, B, T, n_obs, pads):
+    """The same maps against the oracle's network on the GPU (unet_forward(attns=...): mean over heads, absolute value, as
+    rpe.py:128-130), fp32 and under autocast-bf16 for the bound: runs without a reference checkout."""
+    model, diffusion, cfg, sd = build_native(over)
+    model.precision = "bf16"
+    inp, ts = _attn_inputs(cfg, B, T, n_obs, pads)
+    sd_gpu = {k: v.cuda() for k, v in sd.items()}
+    args = (sd_gpu, cfg, inp["x"].cuda(), inp["x0"].cuda(), ts.cuda(), inp["frame_indices"].cuda(), inp["obs_mask"].cuda(),
+            inp["latent_mask"].cuda())
+    attn_r, attn_c = {}, {}
+    with torch.no_grad():
+        eps_r = O.unet_forward(*args, attns=attn_r)
+        with torch.autocast("cuda", dtype=torch.bfloat16):
+            O.unet_forward(*args, attns=attn_c)
+    _check_native_maps("oracle-on-GPU", model, inp, ts, eps_r, attn_r, attn_c)
+
+
+@needs_reference
 def test_sample_loop_attention_logging_matches_the_reference():
     """p_sample_loop(return_attn_weights=True): the per-quartile running means of the maps (gaussian_diffusion.py:448-469) through
     the native maps, against the reference loop with the same seeds (TrainLoop.log_samples' path, train_util.py:451-463)."""
@@ -338,24 +411,73 @@ def test_sample_loop_attention_logging_matches_the_reference():
     assert O.rel_l2(s_n.cpu(), s_r.cpu()) <= 8 * TOL["bf16"]
 
 
+def test_sample_loop_attention_logging_matches_reference_golden_on_gpu(golden):
+    """p_sample_loop(return_attn_weights=True) on the GPU with the native bf16 map kernels against the reference's own run stored in
+    tests/golden/attn_cfg1.pt (same weights, inputs and noises): the final sample and the per-quartile running means of the maps
+    (gaussian_diffusion.py:448-469)."""
+    g = golden("attn_cfg1")
+    model, diffusion, cfg, sd = build_native(g["over"])
+    model.precision = "bf16"
+    inp = g["inputs"]
+    kw = cuda_kw(inp)
+    it = iter([n.cuda() for n in g["noises"][1:]])
+    diffusion._noise_fn = lambda x: next(it)
+    with torch.no_grad():
+        final, attns = diffusion.p_sample_loop(model, tuple(inp["x0"].shape), noise=g["noises"][0].cuda(), model_kwargs=kw,
+                                               latent_mask=kw["latent_mask"], return_attn_weights=True)
+    # calibration, as in the per-forward map tests: what bf16 GEMM operands (torch autocast) cost the oracle's maps of this model on
+    # the loop's first-step inputs; the bound is 1.5x that, with 3e-2 as the floor
+    tab = O.Tables(cfg)
+    ts0 = O.model_timesteps(tab, torch.full((inp["x0"].shape[0],), tab.num_timesteps - 1))
+    args = ({k: v.cuda() for k, v in sd.items()}, cfg, g["noises"][0].cuda(), kw["x0"], ts0.cuda(), kw["frame_indices"],
+            kw["obs_mask"], kw["latent_mask"])
+    a32, a16 = {}, {}
+    with torch.no_grad():
+        O.unet_forward(*args, attns=a32)
+        with torch.autocast("cuda", dtype=torch.bfloat16):
+            O.unet_forward(*args, attns=a16)
+    e_c = max(O.rel_l2(c.float().cpu(), r.cpu()) for key in ("spatial", "temporal") for c, r in zip(a16[key], a32[key]))
+    assert set(attns) == set(g["attns"]) and len(attns) == 8  # 4 quartiles x {spatial, temporal}
+    for tag, ref in g["attns"].items():
+        e = O.rel_l2(attns[tag].cpu(), ref)
+        assert attns[tag].shape == ref.shape and e <= max(3e-2, 1.5 * e_c), (tag, e, e_c)
+    print(f"quartile maps vs the reference's stored run: worst rel-L2 "
+          f"{max(O.rel_l2(attns[t].cpu(), r) for t, r in g['attns'].items()):.3e}; oracle autocast-bf16 calibration {e_c:.3e}")
+    assert O.rel_l2(final.cpu(), g["final"]) <= 8 * TOL["bf16"]
+
+
+ADDITIVE = dict(image_size=32, in_channels=4, num_channels=64, num_res_blocks=1, diffusion_steps=1000, use_scale_shift_norm=False)
+
+
+def _additive_inputs(cfg, sd):
+    assert sd["input_blocks.1.0.emb_layers.1.weight"].shape[0] == 64  # C outputs, not 2C
+    inp = O.synthetic_inputs(cfg, 2, 6, 2, seed=12, video_len=100, pad_rows=(0,))
+    return inp, O.model_timesteps(O.Tables(cfg), torch.tensor([17, 803]))
+
+
+@needs_reference
 def test_additive_embedding_resblocks_match_the_reference():
     """use_scale_shift_norm=False (unet.py:204-206): h = out_layers(h + emb_out) — the embedding is added BEFORE the second
     GroupNorm.  Served by fdm_gn_apply's film_add mode (statistics of h + e derived from those of h in fp64); native training of
     this variant raises (the GroupNorm backward kernels implement the scale/shift form)."""
-    over = dict(image_size=32, in_channels=4, num_channels=64, num_res_blocks=1, diffusion_steps=1000, use_scale_shift_norm=False)
-    model, diffusion, ref_model, ref_diffusion, cfg, sd = build_pair(over)
-    assert sd["input_blocks.1.0.emb_layers.1.weight"].shape[0] == 64  # C outputs, not 2C
-    inp = O.synthetic_inputs(cfg, 2, 6, 2, seed=12, video_len=100, pad_rows=(0,))
-    ts = O.model_timesteps(O.Tables(cfg), torch.tensor([17, 803]))
+    model, diffusion, ref_model, ref_diffusion, cfg, sd = build_pair(ADDITIVE)
+    inp, ts = _additive_inputs(cfg, sd)
     kw = cuda_kw(inp)
     with torch.no_grad():
         ref, _ = ref_model(inp["x"].cuda(), timesteps=ts.cuda(), **kw)
-        for precision in ("fp32", "bf16"):
-            model.precision = precision
-            eps, _ = model(inp["x"].cuda(), timesteps=ts.cuda(), **kw)
-            e = O.rel_l2(eps.cpu(), ref.cpu())
-            print(f"additive-embedding ResBlocks [{precision}] eps rel-L2 = {e:.3e}")
-            assert e <= TOL[precision], (precision, e)
+        _check_eps("additive-embedding ResBlocks vs reference-on-GPU", model, inp, ts, ref)
     model.train()
     with pytest.raises(NotImplementedError, match="use_scale_shift_norm"):
         diffusion.training_losses(model, inp["x0"].cuda(), torch.tensor([3, 5]).cuda(), model_kwargs=kw)
+
+
+def test_additive_embedding_resblocks_match_the_oracle():
+    """The additive-embedding ResBlocks against the oracle's network in fp32 on the GPU (res_block(scale_shift=False)), and native
+    training of the variant raising: runs without a reference checkout."""
+    model, diffusion, cfg, sd = build_native(ADDITIVE)
+    inp, ts = _additive_inputs(cfg, sd)
+    with torch.no_grad():
+        _check_eps("additive-embedding ResBlocks vs oracle-on-GPU", model, inp, ts, oracle_eps_on_gpu(sd, cfg, inp, ts))
+    model.train()
+    with pytest.raises(NotImplementedError, match="use_scale_shift_norm"):
+        diffusion.training_losses(model, inp["x0"].cuda(), torch.tensor([3, 5]).cuda(), model_kwargs=cuda_kw(inp))

@@ -8,6 +8,7 @@ import pytest
 import torch
 
 from oracle import fdm_oracle as O
+from oracle import ref_loader as R
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PIXEL = dict(diffusion_space="pixel", pre_encoded=False, pre_encoded_stats_dict=None)
@@ -144,22 +145,35 @@ def test_training_losses_and_grads_match_reference(golden):
         assert abs(float(grads[k].grad.norm()) - nrm) <= 1e-3 * nrm + floor, k
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/improved_diffusion"), reason="reference checkout only exists in the build container")
-def test_drop_in_package_path_resolution():
+def test_drop_in_package_path_resolution(tmp_path):
     """FDM_REFERENCE_PATH: hot-path modules come from this repo, every other improved_diffusion module from the reference
-    (INTEGRATION.md §2).  Runs the reference's own hierarchy-2 sampling-scheme iterator through the mixed package."""
+    (INTEGRATION.md §2).  The reference checkout is a stand-in tree: its `unet` / `gaussian_diffusion` refuse to be imported, and its
+    `sampling_schemes` replays the hierarchy-2 stages that the live reference's iterator produced (tests/golden/make_stages.py)."""
     import subprocess
     import sys
+    pkg = tmp_path / "improved_diffusion"
+    pkg.mkdir()
+    (pkg / "__init__.py").write_text("")
+    for name in ("unet", "gaussian_diffusion"):
+        (pkg / f"{name}.py").write_text(f"raise ImportError('{name} must come from the drop-in package')\n")
+    (pkg / "sampling_schemes.py").write_text(
+        "import json\n"
+        f"_fx = json.load(open({os.path.join(ROOT, 'tests', 'golden', 'stages_hierarchy-2_T300.json')!r}))\n"
+        "def _hierarchy_2(video_length, num_obs, max_frames, step_size, optimal_schedule_path=None):\n"
+        "    assert (video_length, num_obs, max_frames, step_size) == "
+        "(_fx['video_length'], _fx['n_obs'], _fx['max_frames'], _fx['step_size'])\n"
+        "    return iter([tuple(s) for s in _fx['stages']])\n"
+        "sampling_schemes = {'hierarchy-2': _hierarchy_2}\n")
     code = (
         "import sys, improved_diffusion\n"
         "from improved_diffusion import sampling_schemes, unet, gaussian_diffusion\n"
-        "assert sampling_schemes.__file__.startswith('/root/reference'), sampling_schemes.__file__\n"
+        f"assert sampling_schemes.__file__.startswith({str(tmp_path)!r}), sampling_schemes.__file__\n"
         "assert '_b200' in unet.__file__ and '_b200' in gaussian_diffusion.__file__\n"
         "it = sampling_schemes.sampling_schemes['hierarchy-2'](video_length=300, num_obs=36, max_frames=20, step_size=10)\n"
         "stages = [(len(o), len(l)) for o, l in it]\n"
         "assert len(stages) == 27 and sum(o + l for o, l in stages) == 534, (len(stages), sum(o + l for o, l in stages))\n"
     )
-    env = dict(os.environ, FDM_REFERENCE_PATH="/root/reference",
+    env = dict(os.environ, FDM_REFERENCE_PATH=str(tmp_path),
                PYTHONPATH=os.path.join(ROOT, "latent-flexible-video-diffusion-modeling_b200"))
     r = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True)
     assert r.returncode == 0, r.stderr[-2000:]
@@ -186,7 +200,8 @@ def test_attention_map_logging_matches_reference(golden):
         assert attns[k].shape == ref.shape and O.rel_l2(attns[k], ref) <= 1e-5, k
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/improved_diffusion"), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(R.find_ref() is None, reason="runs the reference's own TrainLoop: needs a reference checkout "
+                                                "(oracle/make_ref.sh copies it into oracle/_ref)")
 def test_drop_in_under_reference_trainloop():
     """The reference's unmodified TrainLoop (train_util.py) runs two optimizer steps over this repo's model + diffusion
     (mask sampling, training_losses, backward, AdamW, EMA, loss logging): tests/dropin_trainloop.py in a subprocess."""
@@ -197,7 +212,7 @@ def test_drop_in_under_reference_trainloop():
     s.bind(("127.0.0.1", 0))
     port = s.getsockname()[1]
     s.close()
-    env = dict(os.environ, FDM_REFERENCE_PATH="/root/reference",
+    env = dict(os.environ, FDM_REFERENCE_PATH=R.find_ref(),
                PYTHONPATH=os.path.join(ROOT, "latent-flexible-video-diffusion-modeling_b200"))
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "dropin_trainloop.py"), str(port)], env=env,
                        capture_output=True, text=True, timeout=600)
