@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define FDM_ABI_VERSION 1
+#define FDM_ABI_VERSION 2
 
 enum { FDM_F32 = 0, FDM_BF16 = 1 };
 
@@ -110,11 +110,6 @@ typedef struct {
   const double* rn_stats;  /* [N][Cout][2] */
   const float* rn_gamma;   /* [Cout] */
   const float* rn_beta;
-  /* segment 1 read from TWO tensors (the ResBlock skip_connection over th.cat([h, skip]), unet.py:460,180, without materialising the
-   * concat): channels [0, C1a) come from a1 ([N][Ho][Wo][C1a]), channels [C1a, C1) from a1b ([N][Ho][Wo][C1 - C1a]); C1a % 64 == 0.
-   * NULL: a1 holds all C1 channels.  tcgen05 halo kernel only (3x3 stride 1 on 16/32/64/128-wide maps). */
-  const void* a1b;
-  int32_t C1a;
 } fdm_conv_args; /* which = 1 */
 int fdm_conv(const fdm_conv_args* a, void* stream);
 

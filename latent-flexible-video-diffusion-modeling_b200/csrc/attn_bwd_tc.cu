@@ -52,7 +52,6 @@ __global__ void __launch_bounds__(128) attn_spatial_bwd_tc_kernel(const __grid_c
   __shared__ uint32_t tmem_slot;
   __shared__ float col_lse[128], col_d[128];
 
-  pdl_launch_dependents();
   const int tid = threadIdx.x, warp = tid >> 5;
   const int r0 = blockIdx.x * 128, h = blockIdx.y, n = blockIdx.z;
   const int L = p.L, F = p.F, C = p.C, cf = p.cf;

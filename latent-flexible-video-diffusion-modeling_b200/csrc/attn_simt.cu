@@ -64,7 +64,6 @@ struct KvTile<__nv_bfloat16> {
 // (then Rv[t,:,chunk]) into a private slice with lane-parallel loads and reads them back as float4 broadcasts.
 template <int TP, int TPW, typename QT, typename OT>
 __global__ void __launch_bounds__(TA_MAX_WARPS * 32) attn_temporal_kernel(TAParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   extern __shared__ __align__(16) float ta_smem[];
   using KV = KvTile<QT>;
@@ -263,7 +262,6 @@ struct SAParams {
 
 template <int FQ, typename QT, typename OT>
 __global__ void __launch_bounds__(256) attn_spatial_kernel(SAParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   constexpr int V = (FQ % 4 == 0) ? 4 : 2;   // vector width of shared-memory accesses (F = 24 -> FQ = 6 -> float2)
   constexpr int SUB = FQ + V;                // padded sub-vector stride: lane `sub` starts at sub*SUB

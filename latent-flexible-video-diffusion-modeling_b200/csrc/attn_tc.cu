@@ -17,7 +17,6 @@
 //                      -> TMEM columns [0, F) (aliasing S, which every thread has finished reading)
 //   5. O / rowsum -> bf16 -> out[N][L][C]
 #include "tc_common.cuh"
-#include <cstdlib>
 #include <mutex>
 
 namespace fdm {
@@ -30,7 +29,6 @@ struct SaTcParams {
   int rows;     // TMA box rows = min(L, 128)
   int cf;       // 64-wide channel chunks per head = ceil(F / 64)
   int tmem_cols;
-  int vbar;     // V on its own barrier (S = Q K^T starts when Q and K have landed)
   float scale_log2e;
   float* lse;   // optional [N][heads][L]: natural-log sum-exp of each scaled score row (saved for the backward pass)
   float* attn_mean;  // optional [N][L][L]: += softmax weights / heads (attention-map logging, rpe.py:128-130)
@@ -59,7 +57,6 @@ __global__ void __launch_bounds__(256) attn_spatial_tc_kernel(const __grid_const
   __shared__ uint32_t tmem_slot;
   __shared__ float xch[2][2][128];  // split rows: [max | sum][column half][row]
 
-  pdl_launch_dependents();
   const int tid = threadIdx.x, warp = tid >> 5;
   const bool split = blockDim.x == 256;
   const int hh = warp >> 2;                 // column half of this thread (0 when not split)
@@ -92,28 +89,16 @@ __global__ void __launch_bounds__(256) attn_spatial_tc_kernel(const __grid_const
 
   if (tid == 0) {
     const int loads_kv = L / p.rows;
-    if (p.vbar) {
-      mbar_expect_tx(&bar_load, (uint32_t)(p.cf * (p.rows * 128 + kv_tile)));
-      mbar_expect_tx(&bar_v, (uint32_t)(p.cf * kv_tile));
-      for (int c = 0; c < p.cf; ++c) {
-        const int ch = h * F + c * 64;
-        tma_load_3d(q_s + c * 16384, &tq, &bar_load, ch, q0, n);
-        for (int j = 0; j < loads_kv; ++j) tma_load_3d(k_s + c * kv_tile + j * p.rows * 128, &tq, &bar_load, C + ch, j * p.rows, n);
-      }
-      for (int c = 0; c < p.cf; ++c)
-        for (int j = 0; j < loads_kv; ++j)
-          tma_load_3d(v_s + c * kv_tile + j * p.rows * 128, &tq, &bar_v, 2 * C + h * F + c * 64, j * p.rows, n);
-    } else {
-      mbar_expect_tx(&bar_load, (uint32_t)(p.cf * (p.rows * 128 + 2 * kv_tile)));
-      for (int c = 0; c < p.cf; ++c) {
-        const int ch = h * F + c * 64;
-        tma_load_3d(q_s + c * 16384, &tq, &bar_load, ch, q0, n);
-        for (int j = 0; j < loads_kv; ++j) {
-          tma_load_3d(k_s + c * kv_tile + j * p.rows * 128, &tq, &bar_load, C + ch, j * p.rows, n);
-          tma_load_3d(v_s + c * kv_tile + j * p.rows * 128, &tq, &bar_load, 2 * C + ch, j * p.rows, n);
-        }
-      }
+    mbar_expect_tx(&bar_load, (uint32_t)(p.cf * (p.rows * 128 + kv_tile)));
+    mbar_expect_tx(&bar_v, (uint32_t)(p.cf * kv_tile));
+    for (int c = 0; c < p.cf; ++c) {
+      const int ch = h * F + c * 64;
+      tma_load_3d(q_s + c * 16384, &tq, &bar_load, ch, q0, n);
+      for (int j = 0; j < loads_kv; ++j) tma_load_3d(k_s + c * kv_tile + j * p.rows * 128, &tq, &bar_load, C + ch, j * p.rows, n);
     }
+    for (int c = 0; c < p.cf; ++c)
+      for (int j = 0; j < loads_kv; ++j)
+        tma_load_3d(v_s + c * kv_tile + j * p.rows * 128, &tq, &bar_v, 2 * C + h * F + c * 64, j * p.rows, n);
     mbar_wait(&bar_load, 0);
     tcgen05_fence_after();
     // ---- S = Q K^T
@@ -229,7 +214,7 @@ __global__ void __launch_bounds__(256) attn_spatial_tc_kernel(const __grid_const
   __syncthreads();
   if (split) sum = xch[1][0][row] + xch[1][1][row];
   if (tid == 0) {
-    if (p.vbar) mbar_wait(&bar_v, 0);
+    mbar_wait(&bar_v, 0);
     tcgen05_fence_after();
     // ---- O = P V   (N chunks of <= 64 head dims; K = L keys in steps of 16)
     for (int c = 0; c < p.cf; ++c) {
@@ -312,8 +297,6 @@ int attn_spatial_tc_launch(const fdm_attn_spatial_args* a, cudaStream_t st) {
   p.tmem_cols = pow2_at_least(L > F ? L : F, 32);
   p.scale_log2e = 1.4426950408889634f / sqrtf((float)F);
   p.lse = a->lse;
-  static const int vbar = [] { const char* e = getenv("FDM_SA_VBAR"); return e ? atoi(e) : 1; }();  // A/B switch; default on
-  p.vbar = vbar;
   p.attn_mean = a->attn_mean;
   EncodeTiledFn enc = get_tensormap_encoder();
   FDM_REQUIRE(enc != nullptr, FDM_ERR_UNSUPPORTED);
@@ -340,13 +323,8 @@ int attn_spatial_tc_launch(const fdm_attn_spatial_args* a, cudaStream_t st) {
   }
   FDM_REQUIRE(smem <= 200 * 1024, FDM_ERR_UNSUPPORTED);
   dim3 grid((L + 127) / 128, a->heads, a->N);
-  // rows of >= SA_SPLIT_MIN_L keys: two threads per query row (256-thread CTAs).  FDM_SA_SPLIT_MIN_L overrides (A/B; 0 = never).
-  static const int split_min_l = [] {
-    const char* e = getenv("FDM_SA_SPLIT_MIN_L");
-    const int v = e ? atoi(e) : SA_SPLIT_MIN_L;
-    return v <= 0 ? 1 << 30 : (v < 64 ? 64 : v);
-  }();
-  fdm::launch(attn_spatial_tc_kernel, dim3(grid), dim3(L >= split_min_l ? 256 : 128), smem, st, tq, p);
+  // rows of >= SA_SPLIT_MIN_L keys: two threads per query row (256-thread CTAs)
+  fdm::launch(attn_spatial_tc_kernel, dim3(grid), dim3(L >= SA_SPLIT_MIN_L ? 256 : 128), smem, st, tq, p);
   return check_launch();
 }
 

@@ -88,7 +88,6 @@ __global__ void __launch_bounds__(128) rpe_bias_kernel(const __grid_constant__ C
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   __shared__ __align__(8) uint64_t bar_load, bar_d;
   __shared__ uint32_t tmem_slot;
-  pdl_launch_dependents();
   const int tid = threadIdx.x, warp = tid >> 5;
   const int px0 = blockIdx.x * 128, j = blockIdx.y, bh = blockIdx.z;
   const int b = bh / p.heads, h = bh - b * p.heads;
@@ -214,7 +213,6 @@ __global__ void __launch_bounds__(128) attn_rows_kernel(const __grid_constant__ 
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   __shared__ __align__(8) uint64_t bar_load, bar_s, bar_o;
   __shared__ uint32_t tmem_slot;
-  pdl_launch_dependents();
   const int tid = threadIdx.x, warp = tid >> 5;
   const int px0 = blockIdx.x * PL, h = blockIdx.y, b = blockIdx.z;
   const int T = p.T, F = p.F, C = p.C, HW = p.HW;
@@ -460,7 +458,6 @@ __global__ void __launch_bounds__(128) rpe_pv_kernel(const __grid_constant__ CUt
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   __shared__ __align__(8) uint64_t bar_load, bar_d;
   __shared__ uint32_t tmem_slot;
-  pdl_launch_dependents();
   const int tid = threadIdx.x, warp = tid >> 5;
   const int px0 = blockIdx.x * 128, t = blockIdx.y, bh = blockIdx.z;
   const int b = bh / p.heads, h = bh - b * p.heads;

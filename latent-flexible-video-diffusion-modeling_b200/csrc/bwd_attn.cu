@@ -8,7 +8,6 @@
 // Two kernels per attention: a row-owner pass (log-sum-exp, D, dq, dRk) and a column-owner pass (dk, dv, dRq, dRv) that
 // re-forms P from the stored log-sum-exp — no cross-CTA reduction except the pixel sums of the RPE tables (fp32 atomics).
 #include "common.cuh"
-#include <stdlib.h>
 
 namespace fdm {
 
@@ -48,7 +47,6 @@ __device__ __forceinline__ float warp_max(float v) {
 // grid (ceil(L/32), heads, N), block 256.  Warp w owns query rows i0 + w*4 .. +3.
 template <typename QT>
 __global__ void __launch_bounds__(256) attn_spatial_bwd_q_kernel(SABwdParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   extern __shared__ __align__(16) float sa_smem[];
   const int F = p.F, ld = F + 1, L = p.L, C = p.C;
@@ -185,7 +183,6 @@ __global__ void __launch_bounds__(256) attn_spatial_bwd_q_kernel(SABwdParams p) 
 // grid (ceil(L/32), heads, N), block 256.  Warp w owns key rows j0 + w*4 .. +3; queries are streamed in blocks of 64.
 template <typename QT>
 __global__ void __launch_bounds__(256) attn_spatial_bwd_kv_kernel(SABwdParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   extern __shared__ __align__(16) float sa_smem[];
   const int F = p.F, ld = F + 1, L = p.L, C = p.C;
@@ -384,7 +381,6 @@ __device__ __forceinline__ void tb_pixel_gemm(const float* rows, const float* co
 // Row-owner pass.  grid (ceil(HW/32), heads, B), block 256: warp w owns query frames t = w, w+8, ...
 template <int TP, typename QT>
 __global__ void __launch_bounds__(TB_WARPS * 32, (TP <= 24 ? 2 : 1)) attn_temporal_bwd_q_kernel(TABwdParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   extern __shared__ __align__(16) float tb_smem[];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -569,7 +565,6 @@ __global__ void __launch_bounds__(TB_WARPS * 32, (TP <= 24 ? 2 : 1)) attn_tempor
 // Column-owner pass.  warp w owns key frames s = w, w+8, ...
 template <int TP, typename QT>
 __global__ void __launch_bounds__(TB_WARPS * 32, (TP <= 24 ? 2 : 1)) attn_temporal_bwd_kv_kernel(TABwdParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   extern __shared__ __align__(16) float tb_smem[];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -776,18 +771,14 @@ static void launch_ta_bwd(const TABwdParams& p, cudaStream_t st) {
   const int T = p.T;
   // frames (warps) per CTA.  Fewer warps per CTA (more CTAs on the small feature maps, where 8-warp CTAs number only 48-192) was
   // measured SLOWER on B200 (cfg3: 3.7 -> 4.9 ms per step): every CTA re-stages all T key/value frames, so halving the frames
-  // per CTA doubles the staging traffic and the serial stage -> sync -> compute chain stays as long.  FDM_TA_BWD_WARPS overrides.
-  static const int nw_env = [] { const char* e = getenv("FDM_TA_BWD_WARPS"); return e ? atoi(e) : 0; }();
-  const int nw = (nw_env == 2 || nw_env == 4) ? nw_env : TB_WARPS;
-  const size_t smem_q = ((size_t)2 * T * TB_FC * TB_LD + (size_t)nw * (3 * T * TB_FC + T * TB_LD + TB_FC * TB_LD)) * sizeof(float);
-  const size_t smem_kv = ((size_t)2 * T * TB_FC * TB_LD + (size_t)nw * (3 * T * TB_FC + 2 * T * TB_LD + TB_FC * TB_LD)) * sizeof(float);
-  const size_t smem_q_max = ((size_t)2 * T * TB_FC * TB_LD + (size_t)TB_WARPS * (3 * T * TB_FC + T * TB_LD + TB_FC * TB_LD)) * sizeof(float);
-  const size_t smem_kv_max = ((size_t)2 * T * TB_FC * TB_LD + (size_t)TB_WARPS * (3 * T * TB_FC + 2 * T * TB_LD + TB_FC * TB_LD)) * sizeof(float);
-  dim3 grid((p.HW + 31) / 32, p.heads, p.B * ((T + nw - 1) / nw));
-  cudaFuncSetAttribute(attn_temporal_bwd_q_kernel<TP, QT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_q_max);
-  cudaFuncSetAttribute(attn_temporal_bwd_kv_kernel<TP, QT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_kv_max);
-  fdm::launch(attn_temporal_bwd_q_kernel<TP, QT>, grid, dim3(nw * 32), smem_q, st, p);
-  fdm::launch(attn_temporal_bwd_kv_kernel<TP, QT>, grid, dim3(nw * 32), smem_kv, st, p);
+  // per CTA doubles the staging traffic and the serial stage -> sync -> compute chain stays as long.
+  const size_t smem_q = ((size_t)2 * T * TB_FC * TB_LD + (size_t)TB_WARPS * (3 * T * TB_FC + T * TB_LD + TB_FC * TB_LD)) * sizeof(float);
+  const size_t smem_kv = ((size_t)2 * T * TB_FC * TB_LD + (size_t)TB_WARPS * (3 * T * TB_FC + 2 * T * TB_LD + TB_FC * TB_LD)) * sizeof(float);
+  dim3 grid((p.HW + 31) / 32, p.heads, p.B * ((T + TB_WARPS - 1) / TB_WARPS));
+  cudaFuncSetAttribute(attn_temporal_bwd_q_kernel<TP, QT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_q);
+  cudaFuncSetAttribute(attn_temporal_bwd_kv_kernel<TP, QT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_kv);
+  fdm::launch(attn_temporal_bwd_q_kernel<TP, QT>, grid, dim3(TB_WARPS * 32), smem_q, st, p);
+  fdm::launch(attn_temporal_bwd_kv_kernel<TP, QT>, grid, dim3(TB_WARPS * 32), smem_kv, st, p);
 }
 
 extern "C" int fdm_attn_temporal_bwd(const fdm_attn_temporal_bwd_args* a, void* stream) {

@@ -25,7 +25,6 @@ struct WgradParams {
 
 template <typename AT, typename DT>
 __global__ void __launch_bounds__(WG_NT) wgrad_simt_kernel(WgradParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   __shared__ __align__(16) float As[WG_BK][WG_BM + 4];
   __shared__ __align__(16) float Bs[WG_BK][WG_BN + 4];
@@ -116,7 +115,6 @@ constexpr int WG_NARROW = 8;
 
 template <typename AT, typename DT>
 __global__ void __launch_bounds__(128) wgrad_narrow_in_kernel(WgradParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   const int co = blockIdx.x * 128 + threadIdx.x;
   const bool ok = co < p.Cout;
@@ -173,7 +171,6 @@ __global__ void __launch_bounds__(128) wgrad_narrow_in_kernel(WgradParams p) {
 
 template <typename AT, typename DT>
 __global__ void __launch_bounds__(128) wgrad_narrow_out_kernel(WgradParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   const int ci = blockIdx.x * 128 + threadIdx.x;
   const bool ok = ci < p.C;
@@ -222,7 +219,6 @@ __global__ void __launch_bounds__(128) wgrad_narrow_out_kernel(WgradParams p) {
 // dw[co][ci < Cw][kh][kw] = sum_split part[split][tap = kh*k+kw][ci][co]
 __global__ void wgrad_reduce_kernel(const float* __restrict__ part, float* __restrict__ dw, int splits, int taps, int C, int Cw,
                                     int Cout) {
-  pdl_launch_dependents();
   pdl_wait();
   const long long total = (long long)taps * Cw * Cout;
   const size_t sstride = (size_t)taps * C * Cout;
@@ -256,7 +252,6 @@ __global__ void wgrad_reduce_kernel(const float* __restrict__ part, float* __res
 template <typename DT>
 __global__ void __launch_bounds__(256) colsum_kernel(const DT* __restrict__ x, float* __restrict__ part, long long rows, int C,
                                                      long long rows_per_block) {
-  pdl_launch_dependents();
   pdl_wait();
   __shared__ float4 cs_red[256];
   const long long r0 = (long long)blockIdx.x * rows_per_block;
@@ -300,7 +295,6 @@ __global__ void __launch_bounds__(256) colsum_kernel(const DT* __restrict__ x, f
 }
 __global__ void colsum_final_kernel(const float* __restrict__ part, float* __restrict__ out, float* __restrict__ out2, int blocks,
                                     int C) {
-  pdl_launch_dependents();
   pdl_wait();
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= C) return;

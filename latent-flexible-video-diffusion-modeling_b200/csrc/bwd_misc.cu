@@ -20,7 +20,6 @@ __device__ __forceinline__ float dsilu(float u) {
 
 // ---------------- B0 weight packing ---------------------------------------------------------------------------------
 __global__ void pack_weights_kernel(const fdm_pack_problem* __restrict__ probs) {
-  pdl_launch_dependents();
   pdl_wait();
   const fdm_pack_problem pr = probs[blockIdx.y];
   const int k = pr.k, kk = k * k;
@@ -94,7 +93,6 @@ __global__ void pack_weights_kernel(const fdm_pack_problem* __restrict__ probs) 
 // ---------------- B6 accumulate / 2x2 sum-pool ----------------------------------------------------------------------
 template <typename ST>
 __global__ void accum_kernel(const ST* __restrict__ src, float* __restrict__ dst, int N, int H, int W, int C, int pool, int acc) {
-  pdl_launch_dependents();
   pdl_wait();
   const int quads = C / 4;
   const long long total = (long long)N * H * W * quads;
@@ -124,7 +122,6 @@ __global__ void accum_kernel(const ST* __restrict__ src, float* __restrict__ dst
 
 template <typename OT>
 __global__ void nchw_to_nhwc_kernel(const float* __restrict__ src, OT* __restrict__ dst, int N, int C, int HW, int Cpad) {
-  pdl_launch_dependents();
   pdl_wait();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (long long)N * HW) return;
@@ -136,7 +133,6 @@ __global__ void nchw_to_nhwc_kernel(const float* __restrict__ src, OT* __restric
 
 __global__ void sum_parts_kernel(const float* __restrict__ parts, float* __restrict__ out, long long stride, long long n,
                                  int count, int acc) {
-  pdl_launch_dependents();
   pdl_wait();
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     float s = acc ? out[i] : 0.f;
@@ -150,7 +146,6 @@ __global__ void sum_parts_kernel(const float* __restrict__ parts, float* __restr
 // per k (coalesced dW rows), blockIdx.y walks n.  (2) dx_part[m][k] = silu'(x) * sum_n dy[m][n] W[n][k]: one thread per k, the
 // n loop streams W rows coalesced; 8 rows of M per pass.
 __global__ void __launch_bounds__(128) linear_bwd_w_kernel(const fdm_linear_bwd_problem* __restrict__ probs) {
-  pdl_launch_dependents();
   pdl_wait();
   const fdm_linear_bwd_problem pr = probs[blockIdx.z];
   const int k = blockIdx.x * 128 + threadIdx.x;
@@ -172,7 +167,6 @@ __global__ void __launch_bounds__(128) linear_bwd_w_kernel(const fdm_linear_bwd_
 }
 
 __global__ void __launch_bounds__(128) linear_bwd_x_kernel(const fdm_linear_bwd_problem* __restrict__ probs) {
-  pdl_launch_dependents();
   pdl_wait();
   const fdm_linear_bwd_problem pr = probs[blockIdx.y];
   if (pr.dx_part == nullptr) return;
@@ -216,7 +210,6 @@ template <typename DT>
 __global__ void __launch_bounds__(256) rpe_hidden_bwd_kernel(const float* __restrict__ te, const int64_t* __restrict__ fi,
                                                              const fdm_rpe_hidden_bwd_problem* __restrict__ probs,
                                                              float* __restrict__ dte, int T, int te_stride) {
-  pdl_launch_dependents();
   pdl_wait();
   const fdm_rpe_hidden_bwd_problem pr = probs[blockIdx.z];
   const int c = blockIdx.x * 32 + threadIdx.x, b = blockIdx.y;
@@ -259,7 +252,6 @@ __global__ void __launch_bounds__(256) rpe_hidden_bwd_kernel(const float* __rest
 
 // ---------------- B7 fused AdamW (+EMA) over flat buffers -----------------------------------------------------------
 __global__ void __launch_bounds__(256) adamw_flat_kernel(fdm_adamw_args a) {
-  pdl_launch_dependents();
   pdl_wait();
   const long long n4 = a.n >> 2;
   const float decay = 1.f - a.lr * a.weight_decay, step = a.lr / a.bias_correction1;
@@ -296,7 +288,6 @@ __global__ void __launch_bounds__(256) adamw_flat_kernel(fdm_adamw_args a) {
 
 // ---------------- B8 masked MSE backward: grid (chunks, B*T) ----------------------------------------------------------
 __global__ void __launch_bounds__(256) masked_mse_bwd_kernel(fdm_masked_mse_bwd_args a) {
-  pdl_launch_dependents();
   pdl_wait();
   const int f = blockIdx.y, b = f / a.T;
   float w = 0.f;

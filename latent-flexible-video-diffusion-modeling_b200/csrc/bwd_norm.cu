@@ -47,7 +47,6 @@ __device__ __forceinline__ void gn_group_stats(const GnBwdParams& p, int n, int 
 // MODE 0: statistics pass; MODE 1: apply pass.  grid (ceil(HW / pix_per_block), N); block (C/4) * ppi threads.
 template <typename OT, int MODE>
 __global__ void __launch_bounds__(256, 3) gn_bwd_kernel(GnBwdParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   __shared__ float s_mean[32], s_rstd[32], s_m1[32], s_m2[32];
   __shared__ float s_red[MODE == 0 ? 1024 * 8 : 1024];  // MODE 1: block partials of the fused bias-gradient column sums
@@ -202,7 +201,6 @@ __global__ void __launch_bounds__(256, 3) gn_bwd_kernel(GnBwdParams p) {
 // parameter gradients from the per-(n, c) sums.  block (32 channels, 8 frame slices): the frames of a video are split over
 // threadIdx.y and combined in shared memory (one thread per channel walking all N frames took 45 us per launch at N = 160).
 __global__ void __launch_bounds__(256) gn_bwd_params_kernel(GnBwdParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   __shared__ double redA[8][33], redB[8][33];
   const int c = blockIdx.x * 32 + threadIdx.x, sl = threadIdx.y;
@@ -258,7 +256,6 @@ constexpr int TGN_MAX_CPG = 16;
 // warp <-> (b, pixel) (grid-stride), lane <-> group.  Three passes over the group's T * C/32 values (L1/L2 resident).
 template <typename OT>
 __global__ void __launch_bounds__(256) temporal_gn_bwd_kernel(TgnBwdParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   extern __shared__ float tg_red[];  // [8 warps][2][C]
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;

@@ -59,27 +59,15 @@ struct OpType<__nv_bfloat16> {
 };
 
 // ---- programmatic dependent launch (PDL).  Every kernel of the library is launched with the programmatic-stream-
-// serialization attribute and calls pdl_wait() before it touches global memory (blocks until the PREVIOUS kernel of the
-// stream has completed and its writes are visible), so the launch latency of each of the ~160 short dependent launches of
-// a diffusion step overlaps its predecessor.  Measured on B200 (cfg4 step): 2.47 -> 2.40 ms.  Triggering the dependents
-// EARLY (griddepcontrol.launch_dependents at kernel start, -DFDM_PDL_EARLY_TRIGGER) was measured SLOWER (2.60 ms): kernels
-// that are themselves still waiting release their successors, and chains of waiting CTAs take the SM slots.  Releasing them
-// right AFTER the own dependency wait (FDM_PDL_TRIGGER_AFTER_WAIT, the default build) is the version that pays: the next
-// kernel becomes resident — TMEM allocation, barrier init, tensor-map prefetch — during this grid's last wave, at most one
-// kernel deep: cfg4 step 1.84 -> 1.75 ms, cfg5 / cfg3 -0.5 % (with the persistent halo conv kernel excluded, conv_halo.cu).
-// FDM_PDL=0 disables the attribute.
-__device__ __forceinline__ void pdl_launch_dependents() {
-#ifdef FDM_PDL_EARLY_TRIGGER
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
+// serialization attribute and calls pdl_wait() before it touches global memory: it blocks until the PREVIOUS kernel of the
+// stream has completed and its writes are visible, then releases the NEXT kernel.  The release comes after the wait, not at
+// kernel start, so a kernel that is itself still waiting never releases its successor: the next kernel becomes resident
+// (TMEM allocation, barrier init, tensor-map prefetch) during this grid's last wave, at most one kernel deep.  DESIGN.md has
+// the measurements.  FDM_PDL=0 disables the attribute.
+__device__ __forceinline__ void pdl_wait_only() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() {
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-#if defined(FDM_PDL_TRIGGER_AFTER_WAIT) && !defined(FDM_PDL_NO_TRIGGER)
-  // let the NEXT kernel of the stream become resident (its prologue: TMEM allocation, barrier init, tensor-map prefetch, up to its own
-  // griddepcontrol.wait) as soon as every CTA of this grid has got past its dependency wait — i.e. during this grid's last wave
+  pdl_wait_only();
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
 }
 
 bool pdl_enabled();  // api.cu

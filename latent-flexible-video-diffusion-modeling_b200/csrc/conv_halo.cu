@@ -21,10 +21,9 @@
 //     channels) as ONE stream of M = 256 MMAs issued by the leader.  Each CTA stages its own A box and only HALF of the weight
 //     tile (BN/2 rows per tap): single-CTA MMAs at N <= 128 are bound by shared-memory operand reads (A + B per MMA, measured
 //     86 clk per 128x128x16 against a tensor floor of 64); the pair reads A + B/2 per SM and halves the weight TMA traffic.
-// This kernel does not release its dependents after its dependency wait (common.cuh, pdl_wait): it is ONE wave of persistent CTAs, so
-// the release would come at kernel start and the next kernel's CTAs would sit on the SMs for the whole run (measured: +4 % on the
-// cfg5 / cfg3 steps).  FDM_HALO_LATE_TRIGGER: release when the MMA warp has issued its last work item instead.
-#define FDM_PDL_NO_TRIGGER
+// This kernel does not release its dependents after its dependency wait (common.cuh, pdl_wait_only): it is ONE wave of persistent
+// CTAs, so the release would come at kernel start and the next kernel's CTAs would sit on the SMs for the whole run (measured: +4 %
+// on the cfg5 / cfg3 steps).
 #include "tc_common.cuh"
 #include <mutex>
 
@@ -42,7 +41,6 @@ struct HaloParams {
   int Cout, W, HW, hbox;
   int pairs_per_frame, n_items, ntiles;
   int kchunks0, kchunks1, klast0, klast1;
-  int kchunks1a;  // chunks of the skip segment that come from its first tensor (ta1); the rest from ta1b.  = kchunks1: one tensor
   int stages, a_bytes, stage_bytes;
   int tpi;       // M tiles per work item: 2 (B shared by two tiles) or 1 (finer items when 2-tile items quantise badly on 148 SMs)
   int a_bytes0;  // bytes of the segment-0 A box ((2*hbox + ks - 1) rows); a_bytes is the slot size
@@ -60,7 +58,6 @@ __global__ void __launch_bounds__(HALO_THREADS, 1) conv_halo_kernel(const __grid
                                                                    const __grid_constant__ CUtensorMap tw0,
                                                                    const __grid_constant__ CUtensorMap ta1,
                                                                    const __grid_constant__ CUtensorMap tw1,
-                                                                   const __grid_constant__ CUtensorMap ta1b,
                                                                    const HaloParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -80,7 +77,6 @@ __global__ void __launch_bounds__(HALO_THREADS, 1) conv_halo_kernel(const __grid
   const int per_pair = p.ntiles * p.nph;
   auto item_of = [&](int q) { return CG == 2 ? ((2 * (q / per_pair) + (int)rank) * per_pair + q % per_pair) : q; };
 
-  pdl_launch_dependents();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float* staging = reinterpret_cast<float*>(smem + (size_t)p.stages * p.stage_bytes);  // [8 warps][32][16], XOR-swizzled
   float* statbuf = staging + 8 * 32 * 16;                                              // [2 buffers][2 tiles][4 lane groups][BN][2]
@@ -91,7 +87,6 @@ __global__ void __launch_bounds__(HALO_THREADS, 1) conv_halo_kernel(const __grid
     if (p.kchunks1) {
       asm volatile("prefetch.tensormap [%0];" ::"l"(&ta1) : "memory");
       asm volatile("prefetch.tensormap [%0];" ::"l"(&tw1) : "memory");
-      if (p.kchunks1a < p.kchunks1) asm volatile("prefetch.tensormap [%0];" ::"l"(&ta1b) : "memory");
     }
   }
   if (warp == 1 && lane == 0) {
@@ -119,7 +114,7 @@ __global__ void __launch_bounds__(HALO_THREADS, 1) conv_halo_kernel(const __grid
   if (CG == 2) cluster_sync_all();  // the peer's barriers are initialised before anything signals them
   tcgen05_fence_after();
   const uint32_t tmem_base = tmem_base_slot;
-  pdl_wait();  // everything above (barriers, TMEM, tensor-map prefetch) overlapped the previous kernel's tail
+  pdl_wait_only();  // everything above (barriers, TMEM, tensor-map prefetch) overlapped the previous kernel's tail
 
   if (warp == 0) {
     // ===================== TMA producer (whole warp converged; one elected lane issues) =====================
@@ -161,18 +156,14 @@ __global__ void __launch_bounds__(HALO_THREADS, 1) conv_halo_kernel(const __grid
           const int stage = it % p.stages;
           mbar_wait(&empty_bar[stage], ((it / p.stages) & 1) ^ 1);
           uint8_t* a_dst = smem + (size_t)stage * p.stage_bytes;
-          // the skip segment's input may be split over two tensors (virtual concat): the weights are one [Cout][C1] matrix
-          const bool second = kc >= p.kchunks1a;
-          const CUtensorMap* tsrc = second ? &ta1b : &ta1;
-          const int ch = (second ? kc - p.kchunks1a : kc) * 64;
           if (elect_one_sync()) {
             if (CG == 2) {
               if (rank == 0) mbar_expect_tx(&full_bar[stage], 2 * (TPI * 128 * 128 + B_TAP_BYTES));
-              tma_load_4d_cg2(a_dst, tsrc, full0 + stage * 8, ch, 0, h0, n);
+              tma_load_4d_cg2(a_dst, &ta1, full0 + stage * 8, kc * 64, 0, h0, n);
               tma_load_3d_cg2(a_dst + p.a_bytes, &tw1, full0 + stage * 8, kc * 64, n_off + b_row, 0);
             } else {
               mbar_expect_tx(&full_bar[stage], TPI * 128 * 128 + B_TAP_BYTES);
-              tma_load_4d(a_dst, tsrc, &full_bar[stage], ch, 0, h0, n);
+              tma_load_4d(a_dst, &ta1, &full_bar[stage], kc * 64, 0, h0, n);
               tma_load_3d(a_dst + p.a_bytes, &tw1, &full_bar[stage], kc * 64, n_off, 0);
             }
           }
@@ -258,9 +249,6 @@ __global__ void __launch_bounds__(HALO_THREADS, 1) conv_halo_kernel(const __grid
         if (elect_one_sync()) commit(&tmem_full_bar[buf]);
         __syncwarp();
       }
-#ifdef FDM_HALO_LATE_TRIGGER
-      asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
       if (p.trace != nullptr && lane == 0) {
         p.trace[blockIdx.x * 8 + 0] = clock64() - t_begin;
         p.trace[blockIdx.x * 8 + 1] = t_wait_tmem;
@@ -436,7 +424,7 @@ static long long* g_trace = nullptr;
 
 template <int BN, int TPI, int CG, bool UP>
 static int launch_halo_cg(const CUtensorMap& ta0, const CUtensorMap& tw0, const CUtensorMap& ta1, const CUtensorMap& tw1,
-                          const CUtensorMap& ta1b, HaloParams& p, cudaStream_t st) {
+                          HaloParams& p, cudaStream_t st) {
   constexpr int SMEM_MAX = 226 * 1024;  // 227 KB per CTA minus the static barriers
   const int extra = 1024 + 8 * 32 * 16 * 4 + 2 * 2 * 4 * BN * 2 * 4;  // alignment slack + staging + statbuf (two buffers)
   p.a_bytes0 = (p.tpi * p.hbox + p.ks - 1) * p.W * 128;
@@ -463,26 +451,26 @@ static int launch_halo_cg(const CUtensorMap& ta0, const CUtensorMap& tw0, const 
   const int sms = g_num_sms > 0 ? g_num_sms : 148;
   if (CG == 2) {
     const int pairs = sms / 2, n_q = p.n_items / 2;
-    fdm::launch_cluster(conv_halo_kernel<BN, TPI, CG, UP>, dim3(2 * (n_q < pairs ? n_q : pairs)), dim3(HALO_THREADS), smem, st, 2, ta0, tw0, ta1, tw1, ta1b, p);
+    fdm::launch_cluster(conv_halo_kernel<BN, TPI, CG, UP>, dim3(2 * (n_q < pairs ? n_q : pairs)), dim3(HALO_THREADS), smem, st, 2, ta0, tw0, ta1, tw1, p);
   } else {
     const int grid = p.n_items < sms ? p.n_items : sms;
-    fdm::launch(conv_halo_kernel<BN, TPI, CG, UP>, dim3(grid), dim3(HALO_THREADS), smem, st, ta0, tw0, ta1, tw1, ta1b, p);
+    fdm::launch(conv_halo_kernel<BN, TPI, CG, UP>, dim3(grid), dim3(HALO_THREADS), smem, st, ta0, tw0, ta1, tw1, p);
   }
   return check_launch();
 }
 
 template <int BN, int TPI>
 static int launch_halo(const CUtensorMap& ta0, const CUtensorMap& tw0, const CUtensorMap& ta1, const CUtensorMap& tw1,
-                       const CUtensorMap& ta1b, HaloParams& p, bool pair, cudaStream_t st) {
+                       HaloParams& p, bool pair, cudaStream_t st) {
   if (p.up) {
     // upsample convs map C -> C channels of the U-Net's block widths: BN = 32 is not instantiated for them
     if (BN == 32) return FDM_ERR_UNSUPPORTED;
     constexpr int BU = BN == 32 ? 64 : BN;
-    if (pair) return launch_halo_cg<BU, TPI, 2, true>(ta0, tw0, ta1, tw1, ta1b, p, st);
-    return launch_halo_cg<BU, TPI, 1, true>(ta0, tw0, ta1, tw1, ta1b, p, st);
+    if (pair) return launch_halo_cg<BU, TPI, 2, true>(ta0, tw0, ta1, tw1, p, st);
+    return launch_halo_cg<BU, TPI, 1, true>(ta0, tw0, ta1, tw1, p, st);
   }
-  if (pair) return launch_halo_cg<BN, TPI, 2, false>(ta0, tw0, ta1, tw1, ta1b, p, st);
-  return launch_halo_cg<BN, TPI, 1, false>(ta0, tw0, ta1, tw1, ta1b, p, st);
+  if (pair) return launch_halo_cg<BN, TPI, 2, false>(ta0, tw0, ta1, tw1, p, st);
+  return launch_halo_cg<BN, TPI, 1, false>(ta0, tw0, ta1, tw1, p, st);
 }
 
 // FDM_ERR_UNSUPPORTED => the caller falls back to the per-tap kernel of conv_tc.cu
@@ -494,8 +482,6 @@ int conv_halo_launch(const fdm_conv_args* a, cudaStream_t st) {
   FDM_REQUIRE(!up || (a->ksize == 3 && a->a1 == nullptr && a->resid == nullptr), FDM_ERR_UNSUPPORTED);
   FDM_REQUIRE(a->resid_norm == 0, FDM_ERR_UNSUPPORTED);  // the recomputed-GroupNorm residual lives in the per-tap kernel's epilogue
   FDM_REQUIRE(a->C0 % 8 == 0 && (a->a1 == nullptr || a->C1 % 8 == 0) && a->Cout % 4 == 0 && a->Cout >= 32, FDM_ERR_UNSUPPORTED);
-  FDM_REQUIRE(a->a1b == nullptr || (a->a1 != nullptr && a->C1a % 64 == 0 && a->C1a > 0 && a->C1a < a->C1 && (a->C1 - a->C1a) % 8 == 0),
-              FDM_ERR_UNSUPPORTED);
   FDM_REQUIRE(a->y_op == nullptr || a->op_dtype == FDM_BF16, FDM_ERR_UNSUPPORTED);
   int W = a->Win, H = a->Hin, N = a->N;
   // pointwise layers without per-frame statistics see a flat pixel list: maps the row-halo tiling does not take (8x8, 4x4) run as
@@ -533,7 +519,6 @@ int conv_halo_launch(const fdm_conv_args* a, cudaStream_t st) {
   p.ks = up ? 2 : a->ksize;
   p.kchunks0 = (a->C0 + 63) / 64;
   p.kchunks1 = a->a1 ? (a->C1 + 63) / 64 : 0;
-  p.kchunks1a = a->a1b ? a->C1a / 64 : p.kchunks1;
   p.klast0 = (a->C0 - (p.kchunks0 - 1) * 64 + 15) / 16;
   p.klast1 = a->a1 ? (a->C1 - (p.kchunks1 - 1) * 64 + 15) / 16 : 0;
   const int co_pad = (a->Cout + 15) / 16 * 16;
@@ -541,11 +526,10 @@ int conv_halo_launch(const fdm_conv_args* a, cudaStream_t st) {
   // of a pair CTA holds half of the tile's rows.
   // Measured on B200 (profiles/r02_halo_cta_pairs.txt): 1.10-1.32x on layers with >= 9 pipeline stages per item (Cin >= 192 or a wide
   // skip segment; 384->384 at 32x32 reaches 1474 TFLOP/s), 0.85-1.0x on shallower ones, where the cross-CTA signalling latency of the
-  // few stages is not amortised -> pairs only for the deep layers.  FDM_HALO_CG=1 forces single CTAs, =2 pairs wherever possible.
-  static const int cg_env = [] { const char* e = getenv("FDM_HALO_CG"); return e ? atoi(e) : 0; }();
+  // few stages is not amortised -> pairs only for the deep layers.
   const int stages_per_item = p.kchunks0 * p.ks + p.kchunks1;
   // (W = 128, BN = 128: always worth it, 1.1-1.4x — only pairs can run the two-tile items there, see below)
-  bool pair = cg_env != 1 && (cg_env == 2 || stages_per_item >= 9 || (W == 128 && bn == 128)) &&
+  bool pair = (stages_per_item >= 9 || (W == 128 && bn == 128)) &&
               ((long)N * (H / (p.tpi * hbox))) % 2 == 0;
   // W = 128 with BN = 128: a single CTA's two-tile stage (64 KB of A + 48 KB of weights) fits only once -> one-tile items (3 image
   // rows loaded per row computed); a pair CTA stages 24 KB of weights, so two stages of two-tile items fit (4 rows per 2 computed)
@@ -556,27 +540,24 @@ int conv_halo_launch(const fdm_conv_args* a, cudaStream_t st) {
   p.pairs_per_frame = H / (p.tpi * hbox);
   p.n_items = N * p.pairs_per_frame * p.ntiles * p.nph;
   const int brows = pair ? bn / 2 : bn;
-  CUtensorMap ta0, tw0, ta1, tw1, ta1b;
+  CUtensorMap ta0, tw0, ta1, tw1;
   bool ok = encode4(&ta0, a->a0, N, H, W, a->C0, p.tpi * hbox + p.ks - 1) &&
             encode3w(&tw0, a->w0, up ? 16 : a->ksize * a->ksize, co_pad, p.kchunks0 * 64, brows, p.ks);
   if (ok && a->a1) {
-    ok = encode4(&ta1, a->a1, N, H, W, a->a1b ? a->C1a : a->C1, p.tpi * hbox) && encode3w(&tw1, a->w1, 1, co_pad, p.kchunks1 * 64, brows, 1);
-    if (ok && a->a1b) ok = encode4(&ta1b, a->a1b, N, H, W, a->C1 - a->C1a, p.tpi * hbox);
-    else ta1b = ta1;
+    ok = encode4(&ta1, a->a1, N, H, W, a->C1, p.tpi * hbox) && encode3w(&tw1, a->w1, 1, co_pad, p.kchunks1 * 64, brows, 1);
   } else {
     ta1 = ta0;
     tw1 = tw0;
-    ta1b = ta0;
   }
   FDM_REQUIRE(ok, FDM_ERR_UNSUPPORTED);
   if (p.tpi == 2) {
-    if (bn == 128) return launch_halo<128, 2>(ta0, tw0, ta1, tw1, ta1b, p, pair, st);
-    if (bn == 64) return launch_halo<64, 2>(ta0, tw0, ta1, tw1, ta1b, p, pair, st);
-    return launch_halo<32, 2>(ta0, tw0, ta1, tw1, ta1b, p, pair, st);
+    if (bn == 128) return launch_halo<128, 2>(ta0, tw0, ta1, tw1, p, pair, st);
+    if (bn == 64) return launch_halo<64, 2>(ta0, tw0, ta1, tw1, p, pair, st);
+    return launch_halo<32, 2>(ta0, tw0, ta1, tw1, p, pair, st);
   }
-  if (bn == 128) return launch_halo<128, 1>(ta0, tw0, ta1, tw1, ta1b, p, pair, st);
-  if (bn == 64) return launch_halo<64, 1>(ta0, tw0, ta1, tw1, ta1b, p, pair, st);
-  return launch_halo<32, 1>(ta0, tw0, ta1, tw1, ta1b, p, pair, st);
+  if (bn == 128) return launch_halo<128, 1>(ta0, tw0, ta1, tw1, p, pair, st);
+  if (bn == 64) return launch_halo<64, 1>(ta0, tw0, ta1, tw1, p, pair, st);
+  return launch_halo<32, 1>(ta0, tw0, ta1, tw1, p, pair, st);
 }
 
 }  // namespace fdm

@@ -35,7 +35,6 @@ __global__ void __launch_bounds__(HEAD_THREADS) conv_head_kernel(const __grid_co
   __shared__ __align__(8) uint64_t load_bar[HEAD_MAX_CHUNKS];
   __shared__ __align__(8) uint64_t mma_bar;
   __shared__ uint32_t tmem_slot;
-  pdl_launch_dependents();
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int n = blockIdx.x / p.strips_per_frame, h0 = (blockIdx.x - n * p.strips_per_frame) * p.R;
   const int rows = p.R + 2, PS = rows * p.W;

@@ -7,7 +7,6 @@
 // GEMM view:  Y[M = N*Ho*Wo, Cout] = sum over (segment, tap, ci) A[pixel(m, tap), ci] * W[tap][ci][co]
 // Tile 64 pixels x 64 channels x 16 k, 256 threads, 4x4 outputs per thread.
 #include "common.cuh"
-#include <stdlib.h>
 
 namespace fdm {
 
@@ -30,7 +29,6 @@ struct ConvParams {
 
 template <typename AT, typename OT>
 __global__ void __launch_bounds__(NT) conv_simt_kernel(ConvParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   __shared__ __align__(16) float As[BK][BM + 4];
   __shared__ __align__(16) float Bs[BK][BN + 4];
@@ -259,23 +257,15 @@ extern "C" int fdm_conv(const fdm_conv_args* a, void* stream) {
   FDM_REQUIRE(a->y_f32 != nullptr || a->y_op != nullptr, FDM_ERR_BAD_ARG);
   FDM_REQUIRE(!(a->out_nchw && a->y_f32 == nullptr), FDM_ERR_BAD_ARG);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  // the two-tensor skip segment exists in the tcgen05 halo kernel only: everything else fails loudly
-  const bool split1 = a->a1b != nullptr;
-  FDM_REQUIRE(!split1 || (a->a1 != nullptr && a->engine == FDM_CONV_TC && a->ksize == 3 && a->stride == 1 && !a->upsample && !a->out_nchw &&
-                          a->C1a > 0 && a->C1a < a->C1 && a->C1a % 64 == 0), FDM_ERR_UNSUPPORTED);
   if (a->engine == FDM_CONV_TC) {
     // the halo kernel also has a pointwise mode, but measured slower than the per-tap kernel for the 1x1 qkv / proj_out
     // linears on B200 (35 vs 28 us, 30 vs 17 us: two short K stages cannot amortise the persistent pipeline) -> 3x3 only
     // — but with >= 4 K chunks (Cin >= 256: the wide models' qkv / proj_out) it wins: 43.6 -> 29.2 us for 384 -> 1152 at 16x16
-    static const bool pw = getenv("FDM_HALO_POINTWISE") != nullptr;
-    static const bool no_pw = getenv("FDM_HALO_NO_POINTWISE") != nullptr;
-    static const bool no_head = getenv("FDM_NO_HEAD_KERNEL") != nullptr;
-    if (a->out_nchw && a->ksize == 3 && !no_head) {
+    if (a->out_nchw && a->ksize == 3) {
       const int rh = conv_head_launch(a, st);
       if (rh != FDM_ERR_UNSUPPORTED) return rh;
     }
-    int rc = (a->ksize == 3 || pw || (a->C0 >= 256 && !no_pw)) ? conv_halo_launch(a, st) : FDM_ERR_UNSUPPORTED;
-    if (rc == FDM_ERR_UNSUPPORTED && split1) return rc;
+    const int rc = (a->ksize == 3 || a->C0 >= 256) ? conv_halo_launch(a, st) : FDM_ERR_UNSUPPORTED;
     return rc == FDM_ERR_UNSUPPORTED ? conv_tc_launch(a, st) : rc;
   }
   if (a->engine == FDM_CONV_TC_TAP) return conv_tc_launch(a, st);

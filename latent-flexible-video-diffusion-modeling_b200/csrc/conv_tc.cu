@@ -80,7 +80,6 @@ __global__ void __launch_bounds__(TC_THREADS, RN ? 3 : 0) conv_tc_kernel(const _
   __shared__ uint32_t tmem_base_slot;
   __shared__ __align__(16) float4 rn_tab[RN ? 4 : 1][2][2][RN ? 32 : 1];  // [epilogue warp][frame half][mul | add][group]
 
-  pdl_launch_dependents();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int mt = blockIdx.x, n_off = blockIdx.y * BN;
   const int m0 = mt * TC_BM;

@@ -8,7 +8,6 @@ namespace fdm {
 __global__ void input_prep_kernel(const float* __restrict__ x, const float* __restrict__ x0,
                                   const float* __restrict__ obs, float* __restrict__ xin,
                                   __nv_bfloat16* __restrict__ xin_bf16, int N, int C, int HW, int Cpad) {
-  pdl_launch_dependents();
   pdl_wait();
   // one thread per (n, pixel); reads are coalesced across pixels per channel plane
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -34,7 +33,6 @@ __global__ void input_prep_kernel(const float* __restrict__ x, const float* __re
 // ---------------- A6 nearest x2 upsample + cast (unet.py:85) ------------------------------------------
 template <typename OT>
 __global__ void cast_kernel(const float* __restrict__ x, OT* __restrict__ out, int N, int H, int W, int C, int up) {
-  pdl_launch_dependents();
   pdl_wait();
   const int Ho = up ? 2 * H : H, Wo = up ? 2 * W : W;
   const int quads = C / 4;
@@ -59,7 +57,6 @@ __global__ void cast_kernel(const float* __restrict__ x, OT* __restrict__ out, i
 // shard against 63 MB of traffic)
 __global__ void __launch_bounds__(256) upsample2_cast_bf16_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ out, int N,
                                                                  int H, int W, int C) {
-  pdl_launch_dependents();
   pdl_wait();
   const int oct = C >> 3;
   const long long total = (long long)N * H * W * oct;
@@ -86,7 +83,6 @@ __global__ void __launch_bounds__(256) upsample2_cast_bf16_kernel(const float* _
 
 // plain fp32 -> bf16 cast of a flat tensor: 8 elements per thread (two 16-byte loads, one 16-byte store), no index arithmetic
 __global__ void __launch_bounds__(256) flat_cast_bf16_kernel(const float4* __restrict__ x, uint4* __restrict__ out, long long n8) {
-  pdl_launch_dependents();
   pdl_wait();
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += (long long)gridDim.x * blockDim.x) {
     const float4 a = __ldg(x + 2 * i), b = __ldg(x + 2 * i + 1);
@@ -105,7 +101,6 @@ __global__ void __launch_bounds__(256) flat_cast_bf16_kernel(const float4* __res
 template <typename OT>
 __global__ void __launch_bounds__(256) cast_colsum_kernel(const float* __restrict__ x, OT* __restrict__ out, float* __restrict__ cs,
                                                           float* __restrict__ cs2, long long rows, int C, long long rows_per_block) {
-  pdl_launch_dependents();
   pdl_wait();
   __shared__ float4 red[256];
   const int quads = C / 4;
@@ -172,7 +167,6 @@ __global__ void ddpm_step_kernel(const float4* x, const float4* __restrict__ eps
                                  const int64_t* __restrict__ t, float4* sample,
                                  float4* __restrict__ pred, const unsigned long long* __restrict__ philox,
                                  long long per_video4, int B, int clip) {
-  pdl_launch_dependents();
   pdl_wait();
   long long total = per_video4 * B;
   unsigned long long seed = 0ull, nonce = 0ull;
@@ -211,7 +205,6 @@ __global__ void ddpm_step_kernel(const float4* x, const float4* __restrict__ eps
 __global__ void q_sample_kernel(const float4* __restrict__ x0, const float4* __restrict__ noise,
                                 const float* __restrict__ coef2, const int64_t* __restrict__ t,
                                 float4* __restrict__ xt, long long per_video4, int B) {
-  pdl_launch_dependents();
   pdl_wait();
   long long total = per_video4 * B;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
@@ -227,7 +220,6 @@ __global__ void q_sample_kernel(const float4* __restrict__ x0, const float4* __r
 __global__ void masked_mse_kernel(const float* __restrict__ eps, const float* __restrict__ noise,
                                   const float* __restrict__ m1, const float* __restrict__ m2,
                                   float* __restrict__ mse, float* __restrict__ evl, long long per_frame, int T) {
-  pdl_launch_dependents();
   pdl_wait();
   const int f = blockIdx.y, b = f / T;
   const float* e = eps + (size_t)f * per_frame;
@@ -256,7 +248,6 @@ __global__ void masked_mse_kernel(const float* __restrict__ eps, const float* __
 __global__ void timestep_embedding_kernel(const float* __restrict__ t, const int64_t* __restrict__ t_index,
                                           const float* __restrict__ t_table, const float* __restrict__ freqs,
                                           float* __restrict__ out, int B, int dim) {
-  pdl_launch_dependents();
   pdl_wait();
   const int half = dim / 2;
   int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -277,7 +268,6 @@ __global__ void timestep_embedding_kernel(const float* __restrict__ t, const int
 constexpr int GL_SMALL_M = 8;
 __global__ void __launch_bounds__(256) grouped_linear_small_kernel(const fdm_linear_problem* __restrict__ probs) {
   extern __shared__ float gl_xs[];  // [M][K]: the (activated) input rows, computed once per block
-  pdl_launch_dependents();
   pdl_wait();
   const fdm_linear_problem pr = probs[blockIdx.y];
   const int lane = threadIdx.x & 31;
@@ -312,7 +302,6 @@ __global__ void __launch_bounds__(256) grouped_linear_small_kernel(const fdm_lin
 
 constexpr int GL_TM = 16, GL_TN = 64, GL_TK = 32;
 __global__ void __launch_bounds__(256) grouped_linear_kernel(const fdm_linear_problem* __restrict__ probs) {
-  pdl_launch_dependents();
   pdl_wait();
   const fdm_linear_problem pr = probs[blockIdx.z];
   const int m0 = blockIdx.y * GL_TM, n0 = blockIdx.x * GL_TN;
@@ -359,7 +348,6 @@ __global__ void __launch_bounds__(256) grouped_linear_kernel(const fdm_linear_pr
 template <typename OT>
 __global__ void rpe_hidden_kernel(const float* __restrict__ te, const int64_t* __restrict__ fi,
                                   const fdm_rpe_hidden_problem* __restrict__ probs, int B, int T, int te_stride) {
-  pdl_launch_dependents();
   pdl_wait();
   const fdm_rpe_hidden_problem pr = probs[blockIdx.y];
   const int C = pr.C;

@@ -114,7 +114,6 @@ __global__ void __launch_bounds__(NL_WORKERS, 1) nl_qkv_kernel(const __grid_cons
   __shared__ uint32_t tmem_slot;
   __shared__ __align__(16) float bias_s[384];
 
-  pdl_launch_dependents();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int w_bytes = p.Cout * NL_K * 2;
   uint8_t* w_s = smem;                     // [2 chunks][Cout rows][128 B]

@@ -26,7 +26,6 @@ __device__ __forceinline__ float4 gn_load4(const __nv_bfloat16* p) {
 // IT = element type of source A (bf16: single-source launches only)
 template <typename OT, typename IT>
 __global__ void gn_apply_kernel(GnParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   __shared__ float s_mean[32], s_rstd[32];
   const int n = blockIdx.y;
@@ -150,7 +149,6 @@ struct TgnParams {
 // Second pass re-reads the (L1/L2-resident) values, normalises and writes.  V = vector width of the channel accesses.
 template <typename OT, int V>
 __global__ void __launch_bounds__(256) temporal_gn_kernel(TgnParams p) {
-  pdl_launch_dependents();
   pdl_wait();
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= p.B * p.HW * 4) return;

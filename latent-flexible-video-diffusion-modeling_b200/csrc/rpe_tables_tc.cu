@@ -37,7 +37,6 @@ __global__ void __launch_bounds__(128) rpe_tables_kernel(const RtParams p) {
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   __shared__ __align__(8) uint64_t w_full[2], mma_done[2], bar_d;
   __shared__ uint32_t tmem_slot;
-  pdl_launch_dependents();
   const RtProblem pr = p.probs[blockIdx.z];
   const int C = pr.C;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;

@@ -41,7 +41,6 @@ __global__ void __launch_bounds__(128, 1) wgrad_tc_kernel(const __grid_constant_
   __shared__ __align__(8) uint64_t done_bar;
   __shared__ uint32_t tmem_base_slot;
 
-  pdl_launch_dependents();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (warp == 0 && lane == 0) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(&tx) : "memory");

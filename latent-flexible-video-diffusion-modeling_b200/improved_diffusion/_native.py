@@ -29,7 +29,7 @@ ConvArgs = _S("ConvArgs", [("a0", vp), ("w0", vp), ("a1", vp), ("w1", vp), ("bia
                            ("ksize", i32), ("stride", i32), ("upsample", i32),
                            ("a_dtype", i32), ("op_dtype", i32), ("out_nchw", i32), ("engine", i32),
                            ("resid_norm", i32), ("rn_T", i32), ("rn_eps", f32), ("rn_tstats", vp), ("rn_stats", vp),
-                           ("rn_gamma", vp), ("rn_beta", vp), ("a1b", vp), ("C1a", i32)])
+                           ("rn_gamma", vp), ("rn_beta", vp)])
 GnApplyArgs = _S("GnApplyArgs", [("xa", vp), ("xb", vp), ("stats_a", vp), ("stats_b", vp), ("gamma", vp), ("beta", vp),
                                  ("film", vp), ("out_op", vp), ("out_f32", vp), ("raw_op", vp),
                                  ("N", i32), ("HW", i32), ("Ca", i32), ("Cb", i32), ("T", i32),
@@ -166,8 +166,8 @@ def lib():
             getattr(L, name).argtypes = [vp]
         L.fdm_norm_linear_supported.restype = C.c_int
         L.fdm_norm_linear_supported.argtypes = [vp]
-        if L.fdm_abi_version() != 1:
-            raise NativeError(f"libfdm_sm100.so ABI {L.fdm_abi_version()} != 1")
+        if L.fdm_abi_version() != 2:
+            raise NativeError(f"libfdm_sm100.so ABI {L.fdm_abi_version()} != 2")
         _lib = L
     return _lib
 

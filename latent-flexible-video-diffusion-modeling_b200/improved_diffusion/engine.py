@@ -369,10 +369,7 @@ class DenoiserEngine:
         self.op_dtype = N_.BF16 if precision == "bf16" else N_.F32
         self.op_torch = th.bfloat16 if precision == "bf16" else th.float32
         self.op_size = 2 if precision == "bf16" else 4
-        # FDM_CONV_ENGINE=simt forces the CUDA-core implicit GEMM everywhere (debugging / A-B timing of the tcgen05 kernel)
-        self.use_tc = precision == "bf16" and os.environ.get("FDM_CONV_ENGINE", "tc") != "simt"
-        # temporal RPE attention on tcgen05 (attn_temporal_tc.cu); FDM_TEMPORAL_TC=0 keeps the CUDA-core kernel (A/B timing)
-        self.temporal_tc = self.use_tc and os.environ.get("FDM_TEMPORAL_TC", "1") != "0"
+        self.use_tc = precision == "bf16"
         self.plans = {}
         self._params = self._n_params = None
         self._train_probe = None
@@ -463,25 +460,11 @@ class DenoiserEngine:
 
     def up_tc_ok(self, Cc, H, W):
         """Upsample convs the halo kernel's phase mode takes (H x W = the LOW-resolution input): whole image rows per 128-pixel tile"""
-        return (self.use_tc and os.environ.get("FDM_UP_PHASES", "1") != "0" and W in (16, 32, 64, 128) and H % (128 // W) == 0
-                and Cc % 8 == 0 and Cc >= 64)  # (the 32-column tile variant is not instantiated for the phase mode)
-
-    # Measured (B200, cfg5 / cfg3 samplers): the bf16 copy costs the producing convs' epilogues what the GroupNorm pass saves (gn_apply
-    # -100..-160 us, halo convs +40..+170 us per step: those epilogues drain at ~2.6 TB/s, the GroupNorm pass at 5.7) — the step time does
-    # not move beyond run-to-run noise, with or without a >= 256-channel threshold.  So the scheme is OFF by default (no producer is asked
-    # for the copy); FDM_SPLIT_MIN_C=<channels> enables it for producers at least that wide (0: all).  Results are bit-identical.
-    split_min_c = int(os.environ.get("FDM_SPLIT_MIN_C", str(1 << 30)))
+        # (the 32-column tile variant is not instantiated for the phase mode)
+        return self.use_tc and self.halo_map_ok(H, W) and Cc % 8 == 0 and Cc >= 64
 
     def halo_map_ok(self, H, W):
         return W in (16, 32, 64, 128) and H % (128 // W) == 0
-
-    def split_ok(self, xa, xb, Co, H, W, train):
-        """ResBlock skip_connection as a two-tensor K segment of the halo conv (fdm_conv a1 | a1b): both producers stored bf16 copies"""
-        if not self.use_tc or train or os.environ.get("FDM_SPLIT_SKIP", "1") == "0" or not self.halo_map_ok(H, W):
-            return False
-        if xa.op is None or Co < 32 or Co % 4 or xa.C % 8 or xa.C < self.split_min_c:
-            return False
-        return xb is None or (xb.op is not None and xa.C % 64 == 0 and xb.C % 8 == 0)
 
     def _f32(self, p):
         key = ("f32", p.data_ptr())
@@ -760,7 +743,7 @@ class DenoiserEngine:
         hsz = self.op_size if self.use_tc else 4
         # inference plans whose temporal attentions ALL run on tcgen05: ONE fused launch produces every bf16 table (hidden layer
         # generated in shared memory as the GEMM's A operand: rpe_tables_tc.cu) instead of fdm_rpe_hidden + one GEMM per net
-        fuse_tables = (self.temporal_tc and not train and os.environ.get("FDM_FUSED_RPE_TABLES", "1") != "0" and bool(attn_blocks)
+        fuse_tables = (self.use_tc and not train and bool(attn_blocks)
                        and max(ab.channels for ab in attn_blocks) <= 512
                        and all(self._temporal_ws(B, T, ab.channels, ab.temporal_attention.num_heads, None) is not None
                                for ab in attn_blocks))
@@ -772,11 +755,11 @@ class DenoiserEngine:
                 hb = None if fuse_tables else P.buf(f"rpe_hidden", B * T * T * Cc * hsz, True)
                 # bf16 copies of the tables are the B operands of the tcgen05 temporal attention (attn_temporal_tc.cu); the fp32
                 # tables are only kept where something still reads them: the CUDA-core kernel (shapes the tcgen05 engine does not
-                # take, FDM_TEMPORAL_TC=0) and the backward kernels of training plans
+                # take) and the backward kernels of training plans
                 # (training plans keep the CUDA-core forward: its backward kernels re-form P in fp32 from the fp32 tables, and a
                 # forward that rounded P / R to bf16 would leave the analytically-zero gradients (RPE output biases: softmax shift
                 # invariance) with more noise than torch's own autocast backward — measured 0.148 vs 0.14 allowed)
-                tc_here = (self.temporal_tc and not train
+                tc_here = (self.use_tc and not train
                            and self._temporal_ws(B, T, ab.channels, ab.temporal_attention.num_heads, None) is not None)
                 rop = P.buf(f"rpe_R_op", B * T * T * Cc * 2, True) if tc_here else None
                 rb_ = P.buf(f"rpe_R", B * T * T * Cc * 4, True) if (train or not tc_here) else None
@@ -839,7 +822,7 @@ class DenoiserEngine:
 
         # ---------------- conv helper
         def conv(a0, C0, Hin, Win, w0, Cout, k, stride=1, upsample=0, a1=None, C1=0, w1=None, bias=None, resid=None,
-                 y_f32=None, y_op=None, stats=None, out_nchw=0, a_dtype=None, flop_c0=None, n_frames=None, a1b=None, C1a=0,
+                 y_f32=None, y_op=None, stats=None, out_nchw=0, a_dtype=None, flop_c0=None, n_frames=None,
                  **resid_norm):
             a_dtype = opd if a_dtype is None else a_dtype
             Nf_ = Nf if n_frames is None else n_frames
@@ -856,7 +839,7 @@ class DenoiserEngine:
             P.op("fdm_conv", N_.ConvArgs, a0=a0, w0=pack(w0), a1=a1, w1=pack(w1) if w1 is not None else None, bias=bias,
                  resid=resid, y_f32=y_f32, y_op=y_op, stats=stats, N=Nf_, Hin=Hin, Win=Win, C0=C0, C1=C1, Cout=Cout,
                  ksize=k, stride=stride, upsample=upsample, a_dtype=a_dtype, op_dtype=opd, out_nchw=out_nchw,
-                 engine=N_.CONV_TC if tc else N_.CONV_SIMT, a1b=a1b, C1a=C1a, **resid_norm)
+                 engine=N_.CONV_TC if tc else N_.CONV_SIMT, **resid_norm)
             return Ho, Wo
 
         for hb, Cc, net, rb_, rop in self._pending_rpe_tc:
@@ -936,7 +919,7 @@ class DenoiserEngine:
             Cc = xa.C + (xb.C if xb else 0)
             ab_ = P.bzero("gn_ab", Nf * Cc * 16)
             gop = None
-            if last and os.environ.get("FDM_FUSE_GRAD_CAST", "1") != "0":
+            if last:
                 gop = P.buf("g_op", Nf * xa.H * xa.W * xa.C * osz)
                 preop[id(xa.buf)] = gop
                 fused_checks.append((len(P.bops), gact(xa)))
@@ -1040,11 +1023,7 @@ class DenoiserEngine:
             hw = Hh * Ww
             has_skip = not isinstance(rb.skip_connection, nn.Identity)
             a1 = P.buf("res_a1", Nf * hw * Ci * osz)
-            # inference: the 1x1 skip_connection reads the bf16 copies its producers stored (xa.op | xb.op: a two-tensor K segment of
-            # the halo conv) instead of a raw copy of the concat written by the GroupNorm pass — 2 of that pass's 8 bytes per element,
-            # moved into conv epilogues where the store is free
-            split_raw = (has_skip and self.split_ok(xa, xb, Co, Hh, Ww, train))
-            raw = P.buf("res_raw", Nf * hw * Ci * osz) if (has_skip and not split_raw) else None
+            raw = P.buf("res_raw", Nf * hw * Ci * osz) if has_skip else None
             gn, c1 = rb.in_layers[0], rb.in_layers[2]
             P.op("fdm_gn_apply", N_.GnApplyArgs, xa=xa.buf, xb=xb.buf if xb else None, stats_a=xa.st,
                  stats_b=xb.st if xb else None, gamma=f32(gn.weight), beta=f32(gn.bias), film=None, out_op=a1, out_f32=None,
@@ -1053,7 +1032,7 @@ class DenoiserEngine:
             # the first conv's output is read by ONE consumer, the second GroupNorm: inference plans in bf16 mode store it once, in
             # bf16 (statistics still come from the fp32 accumulators in the conv epilogue): 6 instead of 10 bytes per element through
             # conv epilogue + GN-apply.  Training plans keep it in fp32 (the GroupNorm backward re-reads it).
-            h1_bf16 = self.use_tc and not train and os.environ.get("FDM_H1_BF16", "1") != "0"
+            h1_bf16 = self.use_tc and not train
             if h1_bf16:
                 h1_ = Act(P.buf("res_h1_op", Nf * hw * Co * osz), P.stats("res_h1", Nf, Co), Co, Hh, Ww)
                 conv(a1, Ci, Hh, Ww, c1.weight, Co, 3, bias=f32(c1.bias), y_op=h1_.buf, stats=h1_.st)
@@ -1074,12 +1053,8 @@ class DenoiserEngine:
             if has_skip:
                 if sk.kernel_size != (1, 1):
                     raise NotImplementedError("ResBlock(use_conv=True) 3x3 skip is never built by create_model")
-                if split_raw:
-                    conv(a2, Co, Hh, Ww, c2.weight, Co, 3, a1=xa.op, C1=Ci, w1=sk.weight, bias=bias_sum(c2.bias, sk.bias),
-                         y_f32=out.buf, y_op=yop, stats=out.st, a1b=xb.op if xb else None, C1a=xa.C if xb else 0)
-                else:
-                    conv(a2, Co, Hh, Ww, c2.weight, Co, 3, a1=raw, C1=Ci, w1=sk.weight, bias=bias_sum(c2.bias, sk.bias),
-                         y_f32=out.buf, y_op=yop, stats=out.st)
+                conv(a2, Co, Hh, Ww, c2.weight, Co, 3, a1=raw, C1=Ci, w1=sk.weight, bias=bias_sum(c2.bias, sk.bias),
+                     y_f32=out.buf, y_op=yop, stats=out.st)
             else:
                 conv(a2, Co, Hh, Ww, c2.weight, Co, 3, bias=f32(c2.bias), resid=xa.buf, y_f32=out.buf, y_op=yop, stats=out.st)
 
@@ -1113,7 +1088,7 @@ class DenoiserEngine:
             # the normalised tensor is never written) and the proj_out epilogue recomputes the residual GN(x) from x and the
             # saved statistics (fdm_conv resid_norm) — 2 launches and 24 bytes per element less per attention block.
             def nl_ok(a_mode):
-                if not self.use_tc or train or os.environ.get("FDM_FUSED_QKV", "1") == "0":
+                if not self.use_tc or train:
                     return False
                 probe = N_.NormLinearArgs(B=B, T=T, HW=hw, K=Cc, Cout=3 * Cc, a_mode=a_mode)
                 return bool(lib.fdm_norm_linear_supported(C.byref(probe)))
@@ -1141,7 +1116,7 @@ class DenoiserEngine:
                 conv(xn_op, Cc, Hh, Ww, ta.qkv.weight, 3 * Cc, 1, bias=f32(ta.qkv.bias), y_op=qkv)
             o = P.buf("ta_o", Nf * hw * Cc * osz)
             P.flops += 10 * T * T * Cc * B * hw  # QK^T, PV and the three contextual RPE einsums (rpe.py:72-83,144,166)
-            ws_bytes = self._temporal_ws(B, T, Cc, ta.num_heads, hw) if (self.temporal_tc and not train) else None
+            ws_bytes = self._temporal_ws(B, T, Cc, ta.num_heads, hw) if (self.use_tc and not train) else None
             ws = P.buf("ta_ws", ws_bytes) if ws_bytes else None
             if ws is None and R[(id(ab), "rpe_q")] is None:
                 raise NativeShapeError(f"temporal attention: no kernel takes T={T}, HW={hw}, C={Cc}, heads={ta.num_heads}")
@@ -1298,17 +1273,10 @@ class DenoiserEngine:
 
         names = {id(mod): name for name, mod in m.named_modules()}
 
-        def run_stage(stage, h, skip=None, feeds_downsample=False, out_wants_op=False):
+        def run_stage(stage, h, skip=None, feeds_downsample=False):
             layers = list(stage)
             for li, layer in enumerate(layers):
                 want_op = feeds_downsample and li == len(layers) - 1 and self.use_tc
-                if out_wants_op and li == len(layers) - 1 and self.use_tc and not train:
-                    # the stage's output is read raw by a ResBlock skip_connection later (as h or as the U-Net skip): bf16 copy from
-                    # its producer when that ResBlock's conv will run on the halo kernel (split_ok)
-                    Hi, Wi = (H, W) if h is None else (h.H, h.W)
-                    Ho_, Wo_ = (Hi // 2, Wi // 2) if isinstance(layer, Downsample) else ((Hi * 2, Wi * 2) if isinstance(layer, Upsample) else (Hi, Wi))
-                    Cout_ = getattr(layer, "out_channels", None) or (h.C if h is not None else 0)
-                    want_op = want_op or (self.halo_map_ok(Ho_, Wo_) and Cout_ >= self.split_min_c)
                 # inference: the phase-mode upsample conv reads the low-resolution bf16 operand — let the producing conv store it
                 # (one more epilogue store instead of a cast launch)
                 if (not train and h is not None and li + 1 < len(layers) and isinstance(layers[li + 1], Upsample)
@@ -1359,12 +1327,11 @@ class DenoiserEngine:
         for si, stage in enumerate(in_stages):
             nxt = in_stages[si + 1] if si + 1 < len(in_stages) else None
             feeds = nxt is not None and len(nxt) == 1 and isinstance(nxt[0], Downsample)
-            h = run_stage(stage, h, feeds_downsample=feeds, out_wants_op=True)   # pushed as a U-Net skip
+            h = run_stage(stage, h, feeds_downsample=feeds)   # pushed as a U-Net skip
             hs.append(h)
-        h = run_stage(m.middle_block, h, out_wants_op=True)
-        out_stages = list(m.output_blocks)
-        for oi, stage in enumerate(out_stages):
-            h = run_stage(stage, h, hs.pop(), out_wants_op=oi + 1 < len(out_stages))
+        h = run_stage(m.middle_block, h)
+        for stage in m.output_blocks:
+            h = run_stage(stage, h, hs.pop())
         gn, cv = m.out[0], m.out[2]
         a = P.buf("head_a", Nf * H * W * h.C * osz)
         P.op("fdm_gn_apply", N_.GnApplyArgs, xa=h.buf, xb=None, stats_a=h.st, stats_b=None, gamma=f32(gn.weight),
@@ -1442,11 +1409,10 @@ class DenoiserEngine:
                 if isinstance(b_, Buf) and id(b_) in cond_bufs:
                     return True
             return False
-        if os.environ.get("FDM_SIDE_COND", "1") != "0" and not train and P.side_end > P.side_begin:
+        if not train and P.side_end > P.side_begin:
             P.side_begin = P.temb_op
         P.join_at = next((i for i, (fn, _, f_) in enumerate(P.ops) if i >= P.side_end and reads_cond(f_)), len(P.ops))
-        if (th.device(device).type == "cuda" and P.side_end > P.side_begin and P.join_at >= P.side_end
-                and os.environ.get("FDM_SIDE_STREAM", "1") != "0"):
+        if th.device(device).type == "cuda" and P.side_end > P.side_begin and P.join_at >= P.side_end:
             P.side_stream = th.cuda.Stream(device)
             P.ev_fork, P.ev_join = th.cuda.Event(), th.cuda.Event()
         # skip-connection activations must stay alive until their consumer: handled by liveness (first/last use)
@@ -1488,7 +1454,7 @@ class DenoiserEngine:
         if train:
             P.geps_view = P.view(P.geps, (B, T, m.out_channels, H, W), th.float32)
             P.n_bwd_launches = len(P.bcalls)
-            if th.device(device).type == "cuda" and os.environ.get("FDM_BWD_SIDE_STREAM", "1") != "0":
+            if th.device(device).type == "cuda":
                 P.bwd_side_stream = th.cuda.Stream(device)
                 P.ev_bfork, P.ev_bjoin = th.cuda.Event(), th.cuda.Event()
         # typed views of the I/O buffers

@@ -154,7 +154,7 @@ class UNetVideoModel(nn.Module):
             # tcgen05 attention kernels accumulate the head-averaged maps themselves (materialising variants: attn_tc.cu,
             # attn_temporal_tc.cu).  Otherwise (fp32 parity mode, CPU, inside autograd): PyTorch expression of the same network.
             from .engine import NativeShapeError
-            if x.is_cuda and self.precision == "bf16" and not th.is_grad_enabled() and os.environ.get("FDM_ATTN_MAPS", "native") == "native":
+            if x.is_cuda and self.precision == "bf16" and not th.is_grad_enabled():
                 try:
                     return self.engine().forward(x, x0, timesteps, frame_indices, obs_mask, latent_mask, collect_attn=True)
                 except NativeShapeError:

@@ -208,31 +208,6 @@ def test_wide_model_64px_vs_oracle(precision):
     assert e <= TOL[precision]
 
 
-def test_split_skip_segment_plans_are_bit_identical():
-    """ResBlock skip_connection over the virtual concat as a two-tensor K segment of the halo conv (engine.split_ok, fdm_conv a1 | a1b;
-    off by default: measured neutral) — the same MMAs in the same order as the materialised raw copy: eps must be bit-identical."""
-    from improved_diffusion.engine import DenoiserEngine
-    over = dict(image_size=64, in_channels=4, num_channels=128, num_res_blocks=1, diffusion_steps=1000)
-    cfg = O.make_cfg(**over)
-    inp = O.synthetic_inputs(cfg, 1, 4, 2, seed=5, video_len=300)
-    ts = torch.tensor([417.0])
-    outs, launches = [], []
-    old = DenoiserEngine.split_min_c
-    try:
-        for min_c in (1 << 30, 0):
-            DenoiserEngine.split_min_c = min_c
-            model, _, _, _ = build(over, "bf16")
-            with torch.no_grad():
-                eps, _ = model(inp["x"].cuda(), timesteps=ts.cuda(), **cuda_kw(inp))
-            outs.append(eps.clone())
-            P = next(iter(model.engine().plans.values()))
-            launches.append(sum(1 for (_, _, _), st in zip(P.calls, P._structs) if getattr(st, "a1b", None)))
-    finally:
-        DenoiserEngine.split_min_c = old
-    assert launches[0] == 0 and launches[1] > 0, launches   # the second plan really uses the two-tensor segment
-    assert torch.equal(outs[0], outs[1])
-
-
 @pytest.mark.parametrize("precision", ["fp32", "bf16"])
 def test_pixel_space_128px_vs_oracle(precision):
     """cfg3's model family (128-px RGB frames: 5 resolution levels, channel_mult (1,1,2,3,4), 128-wide per-tap convs at the top,

@@ -31,7 +31,7 @@ def test_library_exports_every_declared_symbol():
     for name in declared:
         assert hasattr(lib, name), name
     assert set(_native.ENTRY_POINTS) <= declared
-    assert _native.lib().fdm_abi_version() == 1
+    assert _native.lib().fdm_abi_version() == 2
     assert _native.verify_struct_sizes()
     assert _native.lib().fdm_status_string(-2).decode().startswith("unsupported")
 
