@@ -118,6 +118,16 @@ int fdm_conv(const fdm_conv_args* a, void* stream);
  * rpe.py:113,136 (spatial attention norm).  The input may be the channel concat of two tensors
  * (th.cat skip connection, unet.py:460) which is never materialised in fp32.
  *   v = (x - mean_g) * rstd_g * gamma + beta;  if film: v = v*(1+film[b][c]) + film[b][C+c];  if silu: v*=sigmoid(v)
+ *
+ * ResBlock dropout (nn.Dropout between SiLU and the second conv, unet.py:167,203-206), on when drop_philox != NULL and
+ * drop_p > 0 (requires silu = 1).  drop_philox is a DEVICE uint64[2] = {seed, nonce}, read at run time (a captured CUDA graph
+ * draws a new mask whenever the caller rewrites it).  For the element quad starting at index o of [N][HW][C]:
+ *     r    = Philox4x32-10(counter = (lo32(o), hi32(o), drop_salt, lo32(nonce)), key = (lo32(seed), hi32(seed)))
+ *     keep = r.{x,y,z,w}[k] >= thr  for element o + k,   thr = min(ceil(drop_p * 2^32), 2^32 - 1)   (i.e. u = r / 2^32 >= p)
+ *     out  = keep ? v * s : 0,   s = fp32(1 / (1 - drop_p)), s = 0 for drop_p = 1;  the product is formed in fp32, then rounded
+ *                                to op_dtype.
+ * fdm_gn_bwd called with the same drop_philox contents, drop_p and drop_salt regenerates the same mask: that is part of this
+ * contract (the mask is never stored).
  * ---------------------------------------------------------------------------------------------- */
 typedef struct {
   const void* xa;       /* [N][HW][Ca] fp32, or bf16 when xa_bf16 != 0 */
@@ -137,6 +147,9 @@ typedef struct {
   int32_t xa_bf16;      /* 1: xa holds bf16 (a conv output that only this normalisation reads is stored once, in bf16: inference) */
   int32_t film_add;     /* 1: use_scale_shift_norm=False (unet.py:204-206): film row holds C values e, y = GN(x + e) (statistics of x + e are
                            derived from those of x); 0: scale/shift FiLM, y = GN(x) * (1 + scale) + shift */
+  const uint64_t* drop_philox; /* dropout after the SiLU (see above): device {seed, nonce}, or NULL for none */
+  float drop_p;         /* 0 <= drop_p <= 1 (FDM_ERR_BAD_ARG otherwise); 0 = no dropout */
+  int32_t drop_salt;    /* distinguishes the masks of the launches that share one drop_philox */
 } fdm_gn_apply_args; /* which = 2 */
 int fdm_gn_apply(const fdm_gn_apply_args* a, void* stream);
 
@@ -420,8 +433,9 @@ typedef struct {
 int fdm_conv_wgrad(const fdm_conv_wgrad_args* a, void* stream);
 size_t fdm_conv_wgrad_workspace(const fdm_conv_wgrad_args* a);
 
-/* B2  GroupNorm(+FiLM)(+SiLU) backward — native_group_norm_backward + silu_backward + the FiLM chain (unet.py:199-203)
- *     du = (dy_op + dy_f32) * silu'(u);  per (n,c): A = sum_hw du*xhat, B = sum_hw du  (scratch `ab`, fp64 atomics)
+/* B2  GroupNorm(+FiLM)(+SiLU)(+dropout) backward — native_group_norm_backward + silu_backward + the FiLM chain (unet.py:199-203)
+ *     du = (dy_op + dy_f32) * m * silu'(u),  m = the dropout factor (keep ? s : 0) of the fdm_gn_apply launch with the same
+ *     drop_philox contents / drop_p / drop_salt (1 without dropout);  per (n,c): A = sum_hw du*xhat, B = sum_hw du  (scratch `ab`, fp64 atomics)
  *     dx = rstd * (du*k_c - mean_g(k_c*B) - xhat * mean_g(k_c*A)),  k_c = gamma_c * (1 + scale_c);   gx (+)= dx (+ draw_op)
  *     dgamma_c = sum_n (1+scale) A;  dbeta_c = sum_n (1+scale) B;  dscale[b,c] = sum_{n in b} (gamma A + beta B);  dshift[b,c] = sum B */
 typedef struct {
@@ -446,6 +460,9 @@ typedef struct {
   int32_t phases; /* 0 = all three launches; else a mask: 1 = per-(n,c) sums, 2 = parameter gradients (reads the sums), 4 = apply
                      (reads the sums).  The parameter-gradient launch only feeds parameter gradients, so the training schedule issues it
                      on its side stream (mask 2) and keeps the activation-gradient chain (mask 5) short */
+  const uint64_t* drop_philox; /* as fdm_gn_apply_args: the forward's dropout, regenerated (NULL: none; requires silu = 1) */
+  float drop_p;
+  int32_t drop_salt;
 } fdm_gn_bwd_args; /* which = 18 */
 int fdm_gn_bwd(const fdm_gn_bwd_args* a, void* stream);
 

@@ -25,6 +25,7 @@ struct GnBwdParams {
   const float* dpass_a; void* gop_a; float* cs_a; float* cs2_a;
   int N, HW, Ca, Cb, C, T, film_stride, film_off, silu, pix_per_block, acc_a, acc_b;
   float eps;
+  DropArgs drop;  // read by the DROP instantiations only
 };
 
 // group statistics of frame n (threads < 32), as in gn_apply_kernel
@@ -45,9 +46,12 @@ __device__ __forceinline__ void gn_group_stats(const GnBwdParams& p, int n, int 
 }
 
 // MODE 0: statistics pass; MODE 1: apply pass.  grid (ceil(HW / pix_per_block), N); block (C/4) * ppi threads.
-template <typename OT, int MODE>
+// DROP: the forward's dropout mask (p.drop, regenerated) and scale are applied to the upstream gradient before silu'.
+template <typename OT, int MODE, bool DROP>
 __global__ void __launch_bounds__(256, 3) gn_bwd_kernel(GnBwdParams p) {
   pdl_wait();
+  DropMask dm;
+  if constexpr (DROP) dm = load_drop_mask(p.drop);
   __shared__ float s_mean[32], s_rstd[32], s_m1[32], s_m2[32];
   __shared__ float s_red[MODE == 0 ? 1024 * 8 : 1024];  // MODE 1: block partials of the fused bias-gradient column sums
   const int n = blockIdx.y, b = n / p.T;
@@ -126,6 +130,7 @@ __global__ void __launch_bounds__(256, 3) gn_bwd_kernel(GnBwdParams p) {
       float dy[4] = {0.f, 0.f, 0.f, 0.f};
       if (p.dy_op != nullptr) { dy[0] = d_op[u].x; dy[1] = d_op[u].y; dy[2] = d_op[u].z; dy[3] = d_op[u].w; }
       if (p.dy_f32 != nullptr) { dy[0] += d_f32[u].x; dy[1] += d_f32[u].y; dy[2] += d_f32[u].z; dy[3] += d_f32[u].w; }
+      if constexpr (DROP) dm.apply(((size_t)n * p.HW + px) * C + c, dy);
       const float x[4] = {x4[u].x, x4[u].y, x4[u].z, x4[u].w};
       float dx[4];
 #pragma unroll
@@ -350,7 +355,9 @@ extern "C" int fdm_gn_bwd(const fdm_gn_bwd_args* a, void* stream) {
   FDM_REQUIRE((a->xb == nullptr) == (a->stats_b == nullptr), FDM_ERR_BAD_ARG);
   FDM_REQUIRE(a->xb == nullptr || a->gxb != nullptr, FDM_ERR_BAD_ARG);
   FDM_REQUIRE(a->dy_op != nullptr || a->dy_f32 != nullptr, FDM_ERR_BAD_ARG);
-  GnBwdParams p;
+  FDM_REQUIRE(a->drop_p >= 0.f && a->drop_p <= 1.f, FDM_ERR_BAD_ARG);
+  FDM_REQUIRE(a->drop_philox == nullptr || a->silu == 1, FDM_ERR_BAD_ARG);
+  GnBwdParams p{};
   p.xa = a->xa; p.xb = a->xb; p.sa = a->stats_a; p.sb = a->stats_b; p.gamma = a->gamma; p.beta = a->beta; p.film = a->film;
   p.dy_op = a->dy_op; p.dy_f32 = a->dy_f32; p.draw_op = a->draw_op; p.gxa = a->gxa; p.gxb = a->gxb; p.ab = a->ab;
   p.dgamma = a->dgamma; p.dbeta = a->dbeta; p.dfilm = a->dfilm;
@@ -371,14 +378,18 @@ extern "C" int fdm_gn_bwd(const fdm_gn_bwd_args* a, void* stream) {
   dim3 grid((a->HW + ppb - 1) / ppb, a->N);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const int ph = a->phases == 0 ? 7 : a->phases;
+  // the sums pass and the apply pass both read du; the parameter-gradient pass reads only the (masked) sums
+  const bool drop = a->drop_philox != nullptr && a->drop_p > 0.f;
+  if (drop) p.drop = drop_args(a->drop_philox, a->drop_p, a->drop_salt);
+  const bool bf = a->op_dtype == FDM_BF16;
   if (ph & 1) {
-    if (a->op_dtype == FDM_BF16) fdm::launch(gn_bwd_kernel<__nv_bfloat16, 0>, grid, dim3(threads), 0, st, p);
-    else fdm::launch(gn_bwd_kernel<float, 0>, grid, dim3(threads), 0, st, p);
+    fdm::launch(bf ? (drop ? gn_bwd_kernel<__nv_bfloat16, 0, true> : gn_bwd_kernel<__nv_bfloat16, 0, false>)
+                   : (drop ? gn_bwd_kernel<float, 0, true> : gn_bwd_kernel<float, 0, false>), grid, dim3(threads), 0, st, p);
   }
   if (ph & 2) fdm::launch(gn_bwd_params_kernel, dim3((p.C + 31) / 32), dim3(32, 8), 0, st, p);
   if (ph & 4) {
-    if (a->op_dtype == FDM_BF16) fdm::launch(gn_bwd_kernel<__nv_bfloat16, 1>, grid, dim3(threads), 0, st, p);
-    else fdm::launch(gn_bwd_kernel<float, 1>, grid, dim3(threads), 0, st, p);
+    fdm::launch(bf ? (drop ? gn_bwd_kernel<__nv_bfloat16, 1, true> : gn_bwd_kernel<__nv_bfloat16, 1, false>)
+                   : (drop ? gn_bwd_kernel<float, 1, true> : gn_bwd_kernel<float, 1, false>), grid, dim3(threads), 0, st, p);
   }
   return check_launch();
 }

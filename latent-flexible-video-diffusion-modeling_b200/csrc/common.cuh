@@ -107,6 +107,60 @@ inline void launch_cluster(void (*kernel)(KArgs...), dim3 grid, dim3 block, size
   cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 
+// Philox4x32-10 (Salmon et al. 2011; the counter-based generator cuRAND / PyTorch use): 4 x 32 random bits per (counter, key).
+// Shared by the sampler's in-kernel noise (fdm_ddpm_step) and the ResBlock dropout mask (fdm_gn_apply / fdm_gn_bwd).
+__device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    const uint32_t hi0 = __umulhi(0xD2511F53u, ctr.x), lo0 = 0xD2511F53u * ctr.x;
+    const uint32_t hi1 = __umulhi(0xCD9E8D57u, ctr.z), lo1 = 0xCD9E8D57u * ctr.z;
+    ctr = make_uint4(hi1 ^ ctr.y ^ key.x, lo1, hi0 ^ ctr.w ^ key.y, lo0);
+    key.x += 0x9E3779B9u;
+    key.y += 0xBB67AE85u;
+  }
+  return ctr;
+}
+
+// ResBlock dropout (the nn.Dropout between SiLU and the second conv): the keep mask of the four channels c..c+3 of one
+// [N][HW][C] element quad, first element index `o`, regenerated bit for bit by the GroupNorm backward (include/fdm_b200.h).
+struct DropMask {
+  uint2 key;             // seed = philox[0]
+  uint32_t salt, nonce;  // per-launch salt, step nonce = low word of philox[1]
+  uint32_t thr;          // keep iff the 32-bit draw >= thr = min(ceil(p * 2^32), 2^32 - 1)
+  float scale;           // 1 / (1 - p); 0 for p = 1
+  __device__ __forceinline__ void apply(size_t o, float* v) const {
+    const uint4 r = philox4x32_10(make_uint4((uint32_t)o, (uint32_t)((unsigned long long)o >> 32), salt, nonce), key);
+    v[0] = r.x >= thr ? v[0] * scale : 0.f;
+    v[1] = r.y >= thr ? v[1] * scale : 0.f;
+    v[2] = r.z >= thr ? v[2] * scale : 0.f;
+    v[3] = r.w >= thr ? v[3] * scale : 0.f;
+  }
+};
+
+// host: the mask parameters of (philox, p, salt); the seed / nonce words are read on the device at run time
+struct DropArgs {
+  const unsigned long long* philox;
+  uint32_t salt, thr;
+  float scale;
+};
+
+inline DropArgs drop_args(const uint64_t* philox, float p, int32_t salt) {
+  DropArgs d{reinterpret_cast<const unsigned long long*>(philox), (uint32_t)salt, 0u, 1.f};
+  if (p < 1.f) {
+    d.thr = (uint32_t)fmin(ceil((double)p * 4294967296.0), 4294967295.0);
+    d.scale = (float)(1.0 / (1.0 - (double)p));
+  } else {
+    d.thr = 0xffffffffu;
+    d.scale = 0.f;
+  }
+  return d;
+}
+
+__device__ __forceinline__ DropMask load_drop_mask(const DropArgs& d) {
+  const unsigned long long seed = d.philox[0], nonce = d.philox[1];
+  return DropMask{make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)), d.salt, (uint32_t)nonce, d.thr, d.scale};
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

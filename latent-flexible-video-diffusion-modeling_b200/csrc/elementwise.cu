@@ -134,19 +134,7 @@ __global__ void __launch_bounds__(256) cast_colsum_kernel(const float* __restric
 }
 
 // ---------------- A16-A18 fused DDPM posterior update -------------------------------------------------
-// Philox4x32-10 (Salmon et al. 2011; the counter-based generator cuRAND / PyTorch use): 4 x 32 random bits per (counter, key)
-__device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const uint32_t hi0 = __umulhi(0xD2511F53u, ctr.x), lo0 = 0xD2511F53u * ctr.x;
-    const uint32_t hi1 = __umulhi(0xCD9E8D57u, ctr.z), lo1 = 0xCD9E8D57u * ctr.z;
-    ctr = make_uint4(hi1 ^ ctr.y ^ key.x, lo1, hi0 ^ ctr.w ^ key.y, lo0);
-    key.x += 0x9E3779B9u;
-    key.y += 0xBB67AE85u;
-  }
-  return ctr;
-}
-
+// (philox4x32_10: common.cuh)
 // two standard normals from two 32-bit words (Box-Muller; u1 in (0,1], precise logf / sincosf)
 __device__ __forceinline__ float2 box_muller(uint32_t a, uint32_t b) {
   const float u1 = ((float)a + 1.0f) * 2.3283064365386963e-10f;  // (a + 1) / 2^32; a = 2^32-1 rounds to 1.0 -> log = 0

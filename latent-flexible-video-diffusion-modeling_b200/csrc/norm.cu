@@ -14,6 +14,7 @@ struct GnParams {
   float eps;
   double inv_cnt;  // 1 / (channels per group * HW)
   int film_add;  // 1: use_scale_shift_norm=False (unet.py:204-206): the embedding is ADDED before the norm, h = GN(x + e[n, c])
+  DropArgs drop;  // read by the DROP instantiations only
 };
 
 __device__ __forceinline__ float4 gn_load4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
@@ -23,11 +24,13 @@ __device__ __forceinline__ float4 gn_load4(const __nv_bfloat16* p) {
 }
 
 // grid: (ceil(HW / pix_per_block), N); block: (C/4) * ppi threads  (ppi pixels per iteration)
-// IT = element type of source A (bf16: single-source launches only)
-template <typename OT, typename IT>
+// IT = element type of source A (bf16: single-source launches only).  DROP: ResBlock dropout after the SiLU (p.drop).
+template <typename OT, typename IT, bool DROP>
 __global__ void gn_apply_kernel(GnParams p) {
   pdl_wait();
   __shared__ float s_mean[32], s_rstd[32];
+  DropMask dm;
+  if constexpr (DROP) dm = load_drop_mask(p.drop);
   const int n = blockIdx.y;
   const int C = p.C, cpg = C / 32;
   const int quads = C / 4;
@@ -127,6 +130,7 @@ __global__ void gn_apply_kernel(GnParams p) {
         }
       }
       size_t o = ((size_t)n * p.HW + pp) * C + c;
+      if constexpr (DROP) dm.apply(o, v);
       float4 v4 = make_float4(v[0], v[1], v[2], v[3]);
       if (p.out_op != nullptr) OpType<OT>::store4(reinterpret_cast<OT*>(p.out_op) + o, v4);
       if (p.out_f32 != nullptr) *reinterpret_cast<float4*>(p.out_f32 + o) = v4;
@@ -215,7 +219,9 @@ extern "C" int fdm_gn_apply(const fdm_gn_apply_args* a, void* stream) {
   using namespace fdm;
   FDM_REQUIRE(a && a->xa && a->stats_a && a->gamma && a->beta, FDM_ERR_BAD_ARG);
   FDM_REQUIRE((a->xb == nullptr) == (a->stats_b == nullptr), FDM_ERR_BAD_ARG);
-  GnParams p;
+  FDM_REQUIRE(a->drop_p >= 0.f && a->drop_p <= 1.f, FDM_ERR_BAD_ARG);
+  FDM_REQUIRE(a->drop_philox == nullptr || a->silu == 1, FDM_ERR_BAD_ARG);
+  GnParams p{};
   p.xa = a->xa; p.xb = a->xb; p.sa = reinterpret_cast<const double*>(a->stats_a); p.sb = reinterpret_cast<const double*>(a->stats_b); p.gamma = a->gamma; p.beta = a->beta;
   p.film = a->film; p.out_op = a->out_op; p.out_f32 = a->out_f32; p.raw_op = a->raw_op;
   p.N = a->N; p.HW = a->HW; p.Ca = a->Ca; p.Cb = a->xb ? a->Cb : 0; p.C = p.Ca + p.Cb; p.T = a->T > 0 ? a->T : 1;
@@ -235,11 +241,18 @@ extern "C" int fdm_gn_apply(const fdm_gn_apply_args* a, void* stream) {
   p.pix_per_block = ppb;
   dim3 grid((a->HW + ppb - 1) / ppb, a->N);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const bool drop = a->drop_philox != nullptr && a->drop_p > 0.f;
+  if (drop) p.drop = drop_args(a->drop_philox, a->drop_p, a->drop_salt);
   if (a->xa_bf16) {
     FDM_REQUIRE(a->xb == nullptr && a->op_dtype == FDM_BF16, FDM_ERR_UNSUPPORTED);
-    fdm::launch(gn_apply_kernel<__nv_bfloat16, __nv_bfloat16>, dim3(grid), dim3(threads), 0, st, p);
-  } else if (a->op_dtype == FDM_BF16) fdm::launch(gn_apply_kernel<__nv_bfloat16, float>, dim3(grid), dim3(threads), 0, st, p);
-  else fdm::launch(gn_apply_kernel<float, float>, dim3(grid), dim3(threads), 0, st, p);
+    fdm::launch(drop ? gn_apply_kernel<__nv_bfloat16, __nv_bfloat16, true> : gn_apply_kernel<__nv_bfloat16, __nv_bfloat16, false>,
+                dim3(grid), dim3(threads), 0, st, p);
+  } else if (a->op_dtype == FDM_BF16) {
+    fdm::launch(drop ? gn_apply_kernel<__nv_bfloat16, float, true> : gn_apply_kernel<__nv_bfloat16, float, false>, dim3(grid),
+                dim3(threads), 0, st, p);
+  } else {
+    fdm::launch(drop ? gn_apply_kernel<float, float, true> : gn_apply_kernel<float, float, false>, dim3(grid), dim3(threads), 0, st, p);
+  }
   return check_launch();
 }
 

@@ -34,7 +34,7 @@ GnApplyArgs = _S("GnApplyArgs", [("xa", vp), ("xb", vp), ("stats_a", vp), ("stat
                                  ("film", vp), ("out_op", vp), ("out_f32", vp), ("raw_op", vp),
                                  ("N", i32), ("HW", i32), ("Ca", i32), ("Cb", i32), ("T", i32),
                                  ("film_stride", i32), ("film_off", i32), ("silu", i32), ("op_dtype", i32), ("eps", f32),
-                                 ("xa_bf16", i32), ("film_add", i32)])
+                                 ("xa_bf16", i32), ("film_add", i32), ("drop_philox", vp), ("drop_p", f32), ("drop_salt", i32)])
 TemporalGnArgs = _S("TemporalGnArgs", [("x", vp), ("gamma", vp), ("beta", vp), ("out_f32", vp), ("out_op", vp),
                                        ("B", i32), ("T", i32), ("HW", i32), ("C", i32), ("op_dtype", i32), ("eps", f32)])
 TimestepEmbeddingArgs = _S("TimestepEmbeddingArgs", [("t", vp), ("t_index", vp), ("t_table", vp), ("freqs", vp), ("out", vp),
@@ -74,7 +74,8 @@ GnBwdArgs = _S("GnBwdArgs", [("xa", vp), ("xb", vp), ("stats_a", vp), ("stats_b"
                              ("dgamma", vp), ("dbeta", vp), ("dfilm", vp),
                              ("N", i32), ("HW", i32), ("Ca", i32), ("Cb", i32), ("T", i32), ("film_stride", i32),
                              ("film_off", i32), ("silu", i32), ("op_dtype", i32), ("acc_a", i32), ("acc_b", i32), ("eps", f32),
-                             ("dpass_a", vp), ("gop_a", vp), ("cs_a", vp), ("cs2_a", vp), ("phases", i32)])
+                             ("dpass_a", vp), ("gop_a", vp), ("cs_a", vp), ("cs2_a", vp), ("phases", i32),
+                             ("drop_philox", vp), ("drop_p", f32), ("drop_salt", i32)])
 TemporalGnBwdArgs = _S("TemporalGnBwdArgs", [("x", vp), ("gamma", vp), ("dy_op", vp), ("dy_f32", vp), ("gx", vp),
                                              ("dgamma", vp), ("dbeta", vp),
                                              ("B", i32), ("T", i32), ("HW", i32), ("C", i32), ("op_dtype", i32),

@@ -64,6 +64,18 @@ class Plan:
         self.attn_maps = {"spatial": [], "temporal": [], "mixed": []}  # collect_attn plans: (Buf in the zeroed arena, shape)
         self.flops = 0       # algorithmic 2*MAC of every conv / linear / attention matmul of one forward
         self.conv_flops = 0
+        self.res_a2 = []     # (Buf, C, H, W) of every ResBlock's second GroupNorm output (conv2's operand; dropout applied), in order
+        self.drop_p = 0.0    # training plans: ResBlock dropout probability, with its device {seed, nonce} buffer
+        self.drop_philox = None
+        self.drop_nonce = 0
+
+    def refresh_dropout(self):
+        """New dropout masks for the next training forward: {seed, nonce} written on the current stream (the kernels read the buffer
+        at run time, so captured forward / backward graphs pick it up).  The seed is one draw of torch's default generator, so
+        torch.manual_seed decides the masks; the nonce counts this plan's forwards."""
+        self.drop_nonce += 1
+        self.drop_philox[0].fill_(int(th.randint(0, 2 ** 62, ()).item()))
+        self.drop_philox[1].fill_(self.drop_nonce)
 
     # ---- buffers
     def buf(self, name, nbytes, persistent=False):
@@ -298,7 +310,9 @@ class _DenoiserFn(th.autograd.Function):
     @staticmethod
     def forward(ctx, engine, x, x0, timesteps, frame_indices, obs_mask, latent_mask, *params):
         B, T, Cx, H, W = x.shape
-        P = engine.plan_for(B, T, H, W, x.device, train=True)
+        P = engine.plan_for(B, T, H, W, x.device, train=True, drop_p=engine.train_dropout())
+        if P.drop_philox is not None:
+            P.refresh_dropout()
         engine.load_conditioning(P, x0, frame_indices, obs_mask, latent_mask)
         P.set_t_source(None)
         P.x_view.copy_(x)
@@ -479,24 +493,25 @@ class DenoiserEngine:
         return self.packed[key]
 
     # ------------------------------------------------------------------ plan compiler
-    def plan_for(self, B, T, H, W, device, train=False, slot=0, collect_attn=False):
-        """`slot`: distinct plans (own arena, own streams) of the same shape — sub-batches run concurrently by the sampler"""
+    def plan_for(self, B, T, H, W, device, train=False, slot=0, collect_attn=False, drop_p=0.0):
+        """`slot`: distinct plans (own arena, own streams) of the same shape — sub-batches run concurrently by the sampler.
+        `drop_p`: ResBlock dropout of a training plan (part of its key: a plan built without dropout never serves one with it)"""
         if train:
             # training plans survive optimizer steps: their packed weights are refreshed by ONE fdm_pack_weights launch at the
             # head of every forward; they are rebuilt only when a parameter's storage moves (.to(), re-materialisation)
             # parameter storage moves as a whole (.to(), FlatAdamW flattening): three probes decide whether the full signature
             # (390 data_ptr() calls, ~0.2 ms of host time on the launch-bound small model) has to be rebuilt
             pl = self.param_list()
-            probe = (B, T, H, W, str(device), pl[0].data_ptr(), pl[len(pl) // 2].data_ptr(), pl[-1].data_ptr())
+            probe = (B, T, H, W, str(device), drop_p, pl[0].data_ptr(), pl[len(pl) // 2].data_ptr(), pl[-1].data_ptr())
             if self._train_probe is not None and self._train_probe[0] == probe:
                 return self._train_probe[1]
-            key = (B, T, H, W, str(device), tuple(p.data_ptr() for p in pl))
+            key = (B, T, H, W, str(device), drop_p, tuple(p.data_ptr() for p in pl))
             if key in self.train_plans:
                 self._train_probe = (probe, self.train_plans[key])
             if key not in self.train_plans:
                 self.train_plans.clear()
                 with th.cuda.device(device):
-                    self.train_plans[key] = self._compile(B, T, H, W, device, train=True)
+                    self.train_plans[key] = self._compile(B, T, H, W, device, train=True, drop_p=drop_p)
                 self._train_probe = (probe, self.train_plans[key])
             return self.train_plans[key]
         self.refresh_weights()
@@ -583,11 +598,14 @@ class DenoiserEngine:
             return 128 % Wo == 0 and hw % 128 == 0
         return 128 % hw == 0 and (hw % 32 == 0 or 32 % hw == 0)
 
-    def _compile(self, B, T, H, W, device, train=False, collect_attn=False):
+    def _compile(self, B, T, H, W, device, train=False, collect_attn=False, drop_p=0.0):
         m = self.model
         from .unet import ResBlock, FactorizedAttentionBlock, Downsample, Upsample
         P = Plan(self, B, T, H, W)
         P.train = train
+        if train and drop_p > 0:
+            P.drop_p = drop_p
+            P.drop_philox = th.zeros(2, dtype=th.int64, device=device)
         Nf = B * T
         opd, osz = self.op_dtype, self.op_size
         mc, ted = m.model_channels, m.model_channels * 4
@@ -912,10 +930,11 @@ class DenoiserEngine:
                  dbias=pg(biases[0]) if biases else None,
                  dbias2=pg(biases[1]) if len(biases) > 1 else None, workspace=P.wg_ws, workspace_bytes=need, **fields)
 
-        def gn_bwd(xa, xb, gn, foff, dy_op, dy_f32, draw, silu, last=False, dpass=None):
+        def gn_bwd(xa, xb, gn, foff, dy_op, dy_f32, draw, silu, last=False, dpass=None, dropf=None):
             """`last`: this GroupNorm is the LAST contributor (in backward order) to xa's gradient — true for the first forward
             consumer of a tensor — so the launch also emits the operand copy + bias sums its producer needs (checked after the
-            schedule is complete: no later launch may write that gradient)."""
+            schedule is complete: no later launch may write that gradient).  `dropf`: the dropout fields of the forward launch,
+            whose mask the backward regenerates."""
             Cc = xa.C + (xb.C if xb else 0)
             ab_ = P.bzero("gn_ab", Nf * Cc * 16)
             gop = None
@@ -931,7 +950,7 @@ class DenoiserEngine:
                           film_off=foff if foff is not None else 0, silu=silu, op_dtype=opd, acc_a=acc(xa),
                           acc_b=acc(xb) if xb else 0, eps=gn.eps, dpass_a=dpass, gop_a=gop,
                           cs_a=pg(xa.biases[0]) if (gop is not None and xa.biases) else None,
-                          cs2_a=pg(xa.biases[1]) if (gop is not None and len(xa.biases) > 1) else None)
+                          cs2_a=pg(xa.biases[1]) if (gop is not None and len(xa.biases) > 1) else None, **(dropf or {}))
             # sums + apply on the main chain; the parameter-gradient launch (dgamma, dbeta, FiLM scale/shift gradients) only reads
             # the sums and feeds parameter gradients / the conditioning-path backward at the very end: side stream
             P.op("fdm_gn_bwd", N_.GnBwdArgs, phases=5, **fields)
@@ -1042,10 +1061,13 @@ class DenoiserEngine:
             h1_.biases = (c1.bias,)
             gn2, c2 = rb.out_layers[0], rb.out_layers[3]
             a2 = P.buf("res_a2", Nf * hw * Co * osz)
+            P.res_a2.append((a2, Co, Hh, Ww))
+            # dropout (train mode, p > 0): one salt per ResBlock; the backward regenerates the mask from the same fields
+            dropf = dict(drop_philox=P.drop_philox, drop_p=P.drop_p, drop_salt=len(P.res_a2)) if P.drop_philox is not None else {}
             P.op("fdm_gn_apply", N_.GnApplyArgs, xa=h1_.buf, xb=None, stats_a=h1_.st, stats_b=None, gamma=f32(gn2.weight),
                  beta=f32(gn2.bias), film=cond, out_op=a2, out_f32=None, raw_op=None, N=Nf, HW=hw, Ca=Co, Cb=0, T=T,
                  film_stride=cond_cols, film_off=film_off[id(rb)], silu=1, op_dtype=opd, eps=gn2.eps, xa_bf16=1 if h1_bf16 else 0,
-                 film_add=0 if m.use_scale_shift_norm else 1)
+                 film_add=0 if m.use_scale_shift_norm else 1, **dropf)
             out = new_act("res_out", Co, Hh, Ww)
             yop = with_op_copy(out) if want_op else None
             sk = rb.skip_connection
@@ -1071,7 +1093,7 @@ class DenoiserEngine:
                     wgrad(raw, opd, Ci, Ci, Hh, Ww, go, Co, 1, 1, sk.weight)
                 else:
                     wgrad(a2, opd, Co, Co, Hh, Ww, go, Co, 3, 1, c2.weight)  # identity residual: g_xa += g_out inside the last gn_bwd
-                gn_bwd(h1_, None, gn2, film_off[id(rb)], da2, None, None, 1, last=True)
+                gn_bwd(h1_, None, gn2, film_off[id(rb)], da2, None, None, 1, last=True, dropf=dropf)
                 gh = get_op(h1_)
                 da1 = P.buf("d_a1", Nf * hw * Ci * osz)
                 dgrad(gh, Co, Hh, Ww, c1.weight, Ci, 3, out_op=da1)
@@ -1478,6 +1500,14 @@ class DenoiserEngine:
         P.obs_view.copy_(obs_mask.reshape(P.B, P.T))
         th.clamp(obs_mask.reshape(P.B, P.T) + latent_mask.reshape(P.B, P.T), max=1, out=P.mask_view)
 
+    def train_dropout(self):
+        """Dropout probability of the ResBlocks in a training forward (unet.py:167,203-206): the model's `dropout` in train mode,
+        0 in eval mode."""
+        p = float(getattr(self.model, "dropout", 0) or 0) if self.model.training else 0.0
+        if not 0.0 <= p <= 1.0:
+            raise ValueError(f"dropout probability has to be between 0 and 1, but got {p}")
+        return p
+
     def forward_train(self, x, x0, timesteps, frame_indices, obs_mask, latent_mask):
         """Differentiable forward (w.r.t. the parameters) through the native forward + backward schedules."""
         if frame_indices is None:
@@ -1485,11 +1515,11 @@ class DenoiserEngine:
         if not self.model.use_scale_shift_norm:
             raise NotImplementedError("native training implements use_scale_shift_norm=True (the reference default, script_util.py:34); "
                                       "use FDM_TRAIN_ENGINE=autograd for the additive-embedding ResBlocks (unet.py:204-206)")
-        if self.model.training and float(getattr(self.model, "dropout", 0) or 0) > 0:
-            # the reference applies nn.Dropout between SiLU and the second conv of every ResBlock (unet.py:167,203-206); the
-            # native schedules have no dropout mask yet -> refuse loudly instead of silently training without it
-            raise NotImplementedError(f"native training implements dropout=0 (the reference default); dropout={self.model.dropout} "
-                                      "needs FDM_TRAIN_ENGINE=autograd (PyTorch expression of the network) or model.eval()")
+        p = self.train_dropout()
+        if p > 0 and not x.is_cuda:
+            # the masks exist only inside the sm_100a GroupNorm kernels: refuse loudly rather than train without them
+            raise NotImplementedError(f"native ResBlock dropout (dropout={p}) draws its masks on a CUDA device; for CPU tensors use the "
+                                      "PyTorch expression of the network (FDM_ALLOW_TORCH_TRAIN=1), which applies nn.Dropout")
         sink = getattr(self.model, "_fdm_flat_sink", None)
         if sink is not None:  # flat-gradient mode: ONE anchor tensor stands in for the 390 parameters in the autograd graph
             return _DenoiserFn.apply(self, x, x0, timesteps, frame_indices, obs_mask, latent_mask, sink.anchor)
