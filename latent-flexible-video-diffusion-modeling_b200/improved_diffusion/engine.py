@@ -347,14 +347,11 @@ class _DenoiserFn(th.autograd.Function):
         P = engine.plan_for(B, T, H, W, x.device, train=True, drop_p=engine.train_dropout())
         if P.drop_philox is not None:
             P.refresh_dropout()
-        engine.load_conditioning(P, x0, frame_indices, obs_mask, latent_mask)
-        P.set_t_source(None)
-        P.x_view.copy_(x)
-        P.t_view.copy_(timesteps.reshape(B).float())
+        engine.load_inputs(P, x, x0, timesteps, frame_indices, obs_mask, latent_mask)
         P.run_graphed("fwd", x.device)
         P.generation = getattr(P, "generation", 0) + 1
-        ctx.plan, ctx.generation, ctx.engine = P, P.generation, engine
-        ctx.sink = getattr(engine.model, "_fdm_flat_sink", None)
+        ctx.plan, ctx.generation = P, P.generation
+        ctx.route = grad_route(engine.model)
         return P.eps_view.clone()
 
     @staticmethod
@@ -364,48 +361,83 @@ class _DenoiserFn(th.autograd.Function):
             raise RuntimeError("the activations of this forward were overwritten by a later forward of the same shape "
                                "(the training plan keeps ONE set of saved activations): call backward before the next forward")
         P.geps_view.copy_(g)
-        sink = ctx.sink
-        model = ctx.engine.model
-        sync = getattr(model, "_fdm_grad_sync", None)
-        bucket_sync = getattr(model, "_fdm_grad_sync_bucket", None)
-        overlap = (sink is not None and sync is not None and bucket_sync is not None and getattr(model, "_fdm_grad_sync_on", True)
-                   and not getattr(sink, "unsynced", False) and len(P.grad_buckets) > 1)
-        if overlap:
-            # overlapped gradient exchange (reference: DDP's bucketed allreduce during backward, train_util.py:118-125): the backward
-            # schedule runs as one CUDA graph per gradient bucket; as soon as a segment is enqueued, the bucket that is final at its
-            # end is all-reduced (NCCL's stream waits for the segment, the next segment does not wait for NCCL)
-            pending = []
-            for lo, hi, (b_lo, b_hi) in P.backward_segments():
-                P.run_graphed("bwd", g.device, seg=(lo, hi))
-                pending.append(bucket_sync(P.pgrad[b_lo:b_hi]))
-            for finish in pending:
-                finish()
-            sink.receive(P.pgrad)
-            return (None,) * 8
-        P.run_graphed("bwd", g.device)
-        if sink is not None:
-            # flat-gradient mode (optim.FlatAdamW(..., model=model)): the parameters' .grad are persistent views of the optimizer's
-            # flat gradient buffer, so the whole hand-over is ONE allreduce (in place, on the plan's buffer) and ONE copy / add —
-            # no per-parameter views, AccumulateGrad nodes or zero_grad loops (1.5 ms of host time per step for 390 tensors)
-            if sync is None:
-                sink.receive(P.pgrad)
-            elif not getattr(ctx.engine.model, "_fdm_grad_sync_on", True):  # FlatGradDataParallel.no_sync(): accumulate locally
-                sink.receive(P.pgrad)
-                sink.unsynced = True
-            elif getattr(sink, "unsynced", False):  # first synchronised backward after no_sync(): reduce the accumulated total
-                sink.receive(P.pgrad)
-                sync(sink.flat_g)
-                sink.unsynced = False
+        return (None,) * 7 + ctx.route.hand_over(P, g.device)
+
+
+class GradRoute:
+    """Where the native backward's flat parameter gradient (`Plan.pgrad`) goes: one per model, see `grad_route(model)`.
+
+      sink          the optim.FlatAdamW bound to the model (flat-gradient mode), or None
+      reduce        reduce(flat): blocking in-place mean-allreduce (sharding.FlatGradDataParallel), or None
+      reduce_async  reduce_async(view) -> finish: starts a bucket's mean-allreduce, finish() makes the current stream wait for it;
+                    or None (one allreduce after the whole backward)
+      synced        False inside FlatGradDataParallel.no_sync()
+      pending       the sink holds gradients accumulated under no_sync() that have not been reduced yet (FlatAdamW.zero_grad
+                    clears it)
+    """
+    __slots__ = ("sink", "reduce", "reduce_async", "synced", "pending")
+
+    def __init__(self):
+        self.sink = self.reduce = self.reduce_async = None
+        self.synced, self.pending = True, False
+
+    def hand_over(self, P, device):
+        """Run the backward schedule of the training plan `P` and deliver its gradient.  Returns the gradients of the parameter
+        inputs of _DenoiserFn: per-parameter views without a sink, (None,) for the sink's anchor otherwise.
+
+        | sink | reduce        | state                       | what happens                                                     |
+        |------|---------------|-----------------------------|------------------------------------------------------------------|
+        | no   | no            | –                           | run bwd; return per-parameter views of P.pgrad.clone()           |
+        | no   | yes           | –                           | run bwd; clone; reduce(clone); return views                      |
+        | yes  | no            | –                           | run bwd; sink.receive(P.pgrad)                                   |
+        | yes  | yes           | not synced                  | run bwd; receive; pending = True                                 |
+        | yes  | yes           | synced, pending             | run bwd; receive; reduce(sink.flat_g); pending = False           |
+        | yes  | yes + async,  | synced, not pending         | one bwd graph per P.backward_segments() entry, each followed by  |
+        |      | > 1 bucket    |                             | reduce_async(P.pgrad[b_lo:b_hi]); then every finish(); receive   |
+        | yes  | yes           | synced, not pending, else   | run bwd; reduce(P.pgrad); receive                                |
+        """
+        sink, reduce = self.sink, self.reduce
+        if sink is None:
+            P.run_graphed("bwd", device)
+            flat = P.pgrad.clone()  # the plan's buffer is reused by the next backward; autograd owns this copy
+            if reduce is not None:
+                reduce(flat)
+            views = th._C._nn.unflatten_dense_tensors(flat, P.unflat)
+            return tuple(views[i] for i in P.unflat_pick)
+        # flat-gradient mode (optim.FlatAdamW(..., model=model)): the parameters' .grad are persistent views of the optimizer's flat
+        # gradient buffer, so the whole hand-over is ONE allreduce (in place, on the plan's buffer) and ONE copy / add — no
+        # per-parameter views, AccumulateGrad nodes or zero_grad loops (1.5 ms of host time per step for 390 tensors)
+        if reduce is not None and self.synced and not self.pending:
+            if self.reduce_async is not None and len(P.grad_buckets) > 1:
+                # overlapped gradient exchange (reference: DDP's bucketed allreduce during backward, train_util.py:118-125): the
+                # backward schedule runs as one CUDA graph per gradient bucket; as soon as a segment is enqueued, the bucket that is
+                # final at its end is all-reduced (NCCL's stream waits for the segment, the next segment does not wait for NCCL)
+                finishes = []
+                for lo, hi, (b_lo, b_hi) in P.backward_segments():
+                    P.run_graphed("bwd", device, seg=(lo, hi))
+                    finishes.append(self.reduce_async(P.pgrad[b_lo:b_hi]))
+                for finish in finishes:
+                    finish()
             else:
-                sync(P.pgrad)
-                sink.receive(P.pgrad)
-            return (None,) * 8
-        flat = P.pgrad.clone()  # the plan's buffer is reused by the next backward; autograd owns this copy
-        sync = getattr(ctx.engine.model, "_fdm_grad_sync", None)
-        if sync is not None:  # sharding.FlatGradDataParallel: ONE allreduce over the whole flat gradient
-            sync(flat)
-        views = th._C._nn.unflatten_dense_tensors(flat, P.unflat)
-        return (None,) * 7 + tuple(views[i] for i in P.unflat_pick)
+                P.run_graphed("bwd", device)
+                reduce(P.pgrad)
+            sink.receive(P.pgrad)
+            return (None,)
+        P.run_graphed("bwd", device)
+        sink.receive(P.pgrad)
+        if reduce is not None:
+            if self.synced:  # first synchronised backward after no_sync(): reduce the accumulated total once
+                reduce(sink.flat_g)
+            self.pending = not self.synced
+        return (None,)
+
+
+def grad_route(model):
+    """The GradRoute of `model` (any nn.Module), created on first use."""
+    route = getattr(model, "_grad_route", None)
+    if route is None:
+        route = model._grad_route = GradRoute()
+    return route
 
 
 class DenoiserEngine:
@@ -501,6 +533,13 @@ class DenoiserEngine:
         P.obs_view.copy_(obs_mask.reshape(P.B, P.T))
         th.clamp(obs_mask.reshape(P.B, P.T) + latent_mask.reshape(P.B, P.T), max=1, out=P.mask_view)
 
+    def load_inputs(self, P, x, x0, timesteps, frame_indices, obs_mask, latent_mask):
+        """Copy one denoiser call's inputs into the plan's static buffers, with the float `t` buffer as the timestep source."""
+        self.load_conditioning(P, x0, frame_indices, obs_mask, latent_mask)
+        P.set_t_source(None)
+        P.x_view.copy_(x)
+        P.t_view.copy_(timesteps.reshape(P.B).float())
+
     def train_dropout(self):
         """Dropout probability of the ResBlocks in a training forward (unet.py:167,203-206): the model's `dropout` in train mode,
         0 in eval mode."""
@@ -521,7 +560,7 @@ class DenoiserEngine:
             # the masks exist only inside the sm_100a GroupNorm kernels: refuse loudly rather than train without them
             raise NotImplementedError(f"native ResBlock dropout (dropout={p}) draws its masks on a CUDA device; for CPU tensors use the "
                                       "PyTorch expression of the network (FDM_ALLOW_TORCH_TRAIN=1), which applies nn.Dropout")
-        sink = getattr(self.model, "_fdm_flat_sink", None)
+        sink = grad_route(self.model).sink
         if sink is not None:  # flat-gradient mode: ONE anchor tensor stands in for the 390 parameters in the autograd graph
             return _DenoiserFn.apply(self, x, x0, timesteps, frame_indices, obs_mask, latent_mask, sink.anchor)
         return _DenoiserFn.apply(self, x, x0, timesteps, frame_indices, obs_mask, latent_mask, *self.param_list())
@@ -535,10 +574,7 @@ class DenoiserEngine:
             raise ValueError("frame_indices is required (temporal RPE, rpe.py:146)")
         with N_.device_guard(x.device):
             P = self.plan_for(B, T, H, W, x.device, collect_attn=collect_attn)
-            self.load_conditioning(P, x0, frame_indices, obs_mask, latent_mask)
-            P.set_t_source(None)
-            P.x_view.copy_(x)
-            P.t_view.copy_(timesteps.reshape(B).float())
+            self.load_inputs(P, x, x0, timesteps, frame_indices, obs_mask, latent_mask)
             P.run(th.cuda.current_stream(x.device).cuda_stream)
             eps = P.eps_view.clone()
             if not collect_attn:

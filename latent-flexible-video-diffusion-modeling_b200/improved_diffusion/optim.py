@@ -16,16 +16,18 @@ graphs) are gathered into a flat buffer with one foreach copy first.  CUDA only:
 `FlatAdamW(model.parameters(), ..., model=model, bind=False)` only adopts the model's flat layout (gradient-completion order, the
 layout of the native backward's buffer: its per-parameter gradient views are then used in place, without a gather copy).
 `FlatAdamW(model.parameters(), ..., model=model)` additionally BINDS the model's gradient path to the optimizer ("flat-gradient
-mode"): every `p.grad` becomes a persistent view of the optimizer's flat gradient buffer, the native backward node takes ONE
-anchor tensor instead of the 390 parameters and hands its flat gradient over with one (allreduce +) copy — or add, when several
-backwards run between `zero_grad()` calls (gradient accumulation).  `p.grad` stays readable / clippable as usual; torch DDP
-(per-parameter hooks) does not apply in this mode — use `sharding.FlatGradDataParallel`.
+mode": it becomes the `sink` of the model's `engine.GradRoute`): every `p.grad` becomes a persistent view of the optimizer's flat
+gradient buffer, the native backward node takes ONE anchor tensor instead of the 390 parameters and hands its flat gradient over
+with one (allreduce +) copy — or add, when several backwards run between `zero_grad()` calls (gradient accumulation).
+`p.grad` stays readable / clippable as usual; torch DDP (per-parameter hooks) does not apply in this mode — use
+`sharding.FlatGradDataParallel`.
 """
 import ctypes as C
 
 import torch as th
 
 from . import _native as N_
+from .engine import grad_route
 
 
 def completion_order(names):
@@ -108,16 +110,15 @@ class FlatAdamW(th.optim.Optimizer):
         self._step = 0
         self.ema_rates = tuple(float(r) for r in ema_rates)
         self.flat_ema = [self.flat_p.clone() for _ in self.ema_rates]
-        self.bound = None
+        self.route = None  # the model's engine.GradRoute once bound
         if model is not None and bind:
-            self.bound = model
             self.flat_g = th.zeros_like(self.flat_p)
             for p, gview in zip(ps, self._views(self.flat_g)):
                 p.grad = gview  # persistent: the native backward refreshes flat_g, never these tensor objects
             self.anchor = th.zeros(1, device=dev, requires_grad=True)
             self._fresh = True
-            self.unsynced = False  # set by the backward node under FlatGradDataParallel.no_sync()
-            model._fdm_flat_sink = self
+            self.route = grad_route(model)
+            self.route.sink = self
 
     def receive(self, flat):
         """Called by the native backward node with the plan's flat gradient (same slot layout): copy, or add when accumulating."""
@@ -130,18 +131,18 @@ class FlatAdamW(th.optim.Optimizer):
             self.flat_g.add_(flat)
 
     def zero_grad(self, set_to_none=True):
-        if self.bound is None:
+        if self.route is None:
             return super().zero_grad(set_to_none=set_to_none)
         self.flat_g.zero_()  # one memset: gradients that arrive through AccumulateGrad (CPU-style autograd path) add into the views
         self._fresh = True   # the native backward overwrites (copy) on its first hand-over, adds on later ones
-        self.unsynced = False
+        self.route.pending = False
 
     def ema_params(self, i):
         """Per-parameter views of the i-th EMA copy (same shapes / order as the parameters)."""
         return self._views(self.flat_ema[i])
 
     def _flat_grad(self, ps):
-        if self.bound is not None:
+        if self.route is not None:
             return self.flat_g.data_ptr(), None
         g0 = ps[0].grad
         if g0 is None:

@@ -9,12 +9,16 @@ Multi-GPU data parallelism for the hot path (SURVEY §8e), one process per GPU u
     over NVLink/NVSwitch, 128 MB buckets, broadcast_buffers=False); `wrap_ddp` is that call with the reference's arguments.
     `FlatGradDataParallel` is the B200-native alternative for the native training path: the backward schedule leaves ALL
     parameter gradients in one flat fp32 buffer, so the exchange is ONE NCCL allreduce over that buffer (no per-parameter
-    hooks, no bucket copies) issued from inside the autograd node.
+    hooks, no bucket copies) issued from inside the autograd node: the wrapper sets the `reduce` / `reduce_async` of the
+    model's `engine.GradRoute`, and `no_sync()` its `synced`.
 """
 import contextlib
+import os
 
 import torch as th
 import torch.distributed as dist
+
+from .engine import grad_route
 
 
 def shard_bounds(n, rank, world):
@@ -114,15 +118,14 @@ class FlatGradDataParallel(th.nn.Module):
             # p.data writes do not bump the parameters' version counters: drop any packed inference weights / sampler graphs
             for eng in getattr(model, "_engines", {}).values():
                 eng.invalidate()
-        model._fdm_grad_sync = lambda flat: allreduce_mean_(flat, group)
-        model._fdm_grad_sync_on = True
-        # bucketed exchange overlapped with the backward schedule (engine._DenoiserFn.backward); `overlap=False` / FDM_DDP_OVERLAP=0
+        self.route = route = grad_route(model)
+        route.reduce = lambda flat: allreduce_mean_(flat, group)
+        # bucketed exchange overlapped with the backward schedule (engine.GradRoute.hand_over); `overlap=False` / FDM_DDP_OVERLAP=0
         # keeps the single allreduce after the whole backward
-        import os
         if overlap and os.environ.get("FDM_DDP_OVERLAP", "1") != "0":
-            model._fdm_grad_sync_bucket = lambda flat: allreduce_mean_async(flat, group)
-        elif hasattr(model, "_fdm_grad_sync_bucket"):
-            del model._fdm_grad_sync_bucket
+            route.reduce_async = lambda flat: allreduce_mean_async(flat, group)
+        else:
+            route.reduce_async = None
 
     @contextlib.contextmanager
     def no_sync(self):
@@ -130,13 +133,13 @@ class FlatGradDataParallel(th.nn.Module):
         accumulated gradient once.  Needs the flat-gradient mode (optim.FlatAdamW(..., model=model)), whose flat buffer is what
         gets reduced; as with DDP, do not mix synchronised and unsynchronised backwards between two zero_grad() calls other than
         `no_sync ... no_sync, sync`."""
-        if getattr(self.module, "_fdm_flat_sink", None) is None:
+        if self.route.sink is None:
             raise NotImplementedError("FlatGradDataParallel.no_sync() needs optim.FlatAdamW(..., model=model) (flat-gradient mode)")
-        self.module._fdm_grad_sync_on = False
+        self.route.synced = False
         try:
             yield
         finally:
-            self.module._fdm_grad_sync_on = True
+            self.route.synced = True
 
     def forward(self, x, **kwargs):
         if not x.is_cuda:

@@ -23,6 +23,8 @@ What changes is the cost once forward+backward takes ~3 ms (cfg2) instead of ~50
 
 This module owns no kernels; it calls the hot path through the same public API a user does.
 """
+import contextlib
+
 import numpy as np
 import torch as th
 import torch.distributed as dist
@@ -198,7 +200,7 @@ class NativeTrainStep:
             last = i + mb >= batch1.shape[0]
             t, weights = self.schedule_sampler.sample(micro.shape[0], dev)
             no_sync = getattr(self.net, "no_sync", None) if not last else None
-            ctx = no_sync() if no_sync is not None else _null()
+            ctx = no_sync() if no_sync is not None else contextlib.nullcontext()
             with ctx:
                 losses = self.diffusion.training_losses(
                     self.net, micro, t, model_kwargs=dict(frame_indices=frame_indices, obs_mask=obs_mask, latent_mask=latent_mask,
@@ -371,11 +373,3 @@ class NativeTrainStep:
             self.opt.load_state_dict(th.load(path, map_location=dev))
         self.step = step
         return step
-
-
-class _null:
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        return False

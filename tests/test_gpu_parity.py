@@ -598,7 +598,7 @@ def test_native_train_step_matches_torch_stack(monkeypatch, tmp_path):
     # allreduce is the identity, the deferred-synchronisation bookkeeping is what runs): the same numbers
     acc, _, model_a, _ = run("flat", "native", microbatch=1, steps=2)
     accw, _, model_w, runner_w = run("flat", "native", microbatch=1, wrap=True, steps=2)
-    assert runner_w.opt.unsynced is False
+    assert runner_w.opt.route.pending is False
     for a, b in zip(acc, accw):  # not bit-identical: the backward's fp32 atomics (RPE tables, split reductions) reorder run to run
         for k in a:
             assert abs(a[k] - b[k]) <= 1e-5 * max(abs(b[k]), 1e-6), (k, a[k], b[k])
@@ -624,9 +624,10 @@ def test_native_train_step_matches_torch_stack(monkeypatch, tmp_path):
 
 def test_bucketed_backward_segments_match_the_single_graph(monkeypatch):
     """The overlapped gradient exchange runs the backward schedule as one CUDA graph per gradient bucket and hands each bucket to the
-    collective as soon as its segment is enqueued (engine._DenoiserFn.backward).  With an identity 'collective' on one GPU the
+    collective as soon as its segment is enqueued (engine.GradRoute.hand_over).  With an identity 'collective' on one GPU the
     segmented path must reproduce the single-graph gradients exactly, bucket views must tile the flat buffer, and every bucket
     must be handed over exactly once, in completion order."""
+    from improved_diffusion.engine import grad_route
     from improved_diffusion.optim import FlatAdamW
     over = dict(image_size=32, in_channels=4, num_channels=32, num_res_blocks=1, diffusion_steps=32)
     monkeypatch.setenv("FDM_TRAIN_ENGINE", "native")
@@ -653,9 +654,9 @@ def test_bucketed_backward_segments_match_the_single_graph(monkeypatch):
     def bucket_sync(view):
         seen.append((view.data_ptr(), view.numel()))
         return lambda: None
-    model._fdm_grad_sync = lambda flat: flat
-    model._fdm_grad_sync_on = True
-    model._fdm_grad_sync_bucket = bucket_sync
+    route = grad_route(model)
+    route.reduce = lambda flat: flat
+    route.reduce_async = bucket_sync
     seg = grads()
     P = next(iter(model.engine().train_plans.values()))
     nb = len(P.grad_buckets)

@@ -95,6 +95,7 @@ def _worker(rank, world, port, what, out_dir):
             worst = max(float((p.grad - ref[k]).norm()) / max(float(ref[k].norm()), floor) for k, p in model.named_parameters())
             assert worst <= 1e-4, worst
         elif what == "flat":
+            from improved_diffusion.engine import grad_route
             # the collective of FlatGradDataParallel (one mean-allreduce over a flat gradient buffer) and its parameter broadcast
             flat = torch.arange(10, dtype=torch.float32) * (rank + 1)
             sharding.allreduce_mean_(flat)
@@ -103,9 +104,10 @@ def _worker(rank, world, port, what, out_dir):
             with torch.no_grad():
                 m.w.fill_(float(rank + 3))
             wrapped = sharding.FlatGradDataParallel(m)
-            assert float(m.w) == 3.0 and callable(m._fdm_grad_sync) and wrapped.module is m
+            route = grad_route(m)
+            assert float(m.w) == 3.0 and callable(route.reduce) and wrapped.module is m and wrapped.route is route
             g = torch.full((4,), float(rank))
-            m._fdm_grad_sync(g)
+            route.reduce(g)
             assert torch.allclose(g, torch.full((4,), (world - 1) / 2))
         elif what == "trainstep":
             # train_step.NativeTrainStep (host side of TrainLoop.run_step) under DDP, torch arm: per-rank data and masks, two
