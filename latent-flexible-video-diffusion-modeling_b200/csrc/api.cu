@@ -1,5 +1,6 @@
-// C-ABI housekeeping: version, status strings, struct sizes (so the ctypes mirror can be verified on CPU).
-#include "common.cuh"
+// C-ABI housekeeping: version, status strings, struct sizes (so the ctypes mirror can be verified on CPU); the tensor-map encoder.
+#include "tc_common.cuh"
+#include <cudaTypedefs.h>
 #include <string.h>
 #include <stdlib.h>
 
@@ -16,6 +17,28 @@ bool pdl_enabled() {
     return !(e != nullptr && e[0] == '0');
   }();
   return on;
+}
+
+bool encode_bf16_map(CUtensorMap* map, const void* ptr, int rank, const cuuint64_t* dims, const cuuint32_t* box,
+                     CUtensorMapL2promotion l2, CUtensorMapSwizzle swz, const cuuint64_t* strides, const cuuint32_t* elem_strides) {
+  static const PFN_cuTensorMapEncodeTiled encode = [] {
+    void* fn = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    const bool found = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) == cudaSuccess &&
+                       q == cudaDriverEntryPointSuccess;
+    return found ? reinterpret_cast<PFN_cuTensorMapEncodeTiled>(fn) : nullptr;
+  }();
+  if (encode == nullptr || rank > 5) return false;  // 5: the largest rank of a tiled tensor map
+  cuuint64_t dense[4];
+  if (strides == nullptr) {
+    cuuint64_t s = sizeof(__nv_bfloat16);
+    for (int i = 0; i + 1 < rank; ++i) dense[i] = s *= dims[i];
+    strides = dense;
+  }
+  const cuuint32_t ones[5] = {1, 1, 1, 1, 1};
+  return encode(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(ptr), dims, strides, box,
+                elem_strides != nullptr ? elem_strides : ones, CU_TENSOR_MAP_INTERLEAVE_NONE, swz, l2,
+                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 }  // namespace fdm
 

@@ -13,7 +13,6 @@
 //   KV = false: rows = queries (Q, dO), columns = keys (K, V);   out1 = dS K            -> dQ        (row statistics)
 //   KV = true : rows = keys (K, V),    columns = queries (Q, dO); out1 = dS^T Q -> dK, out2 = P^T dO -> dV   (column statistics)
 #include "tc_common.cuh"
-#include <mutex>
 
 namespace fdm {
 
@@ -65,18 +64,15 @@ __global__ void __launch_bounds__(128) attn_spatial_bwd_tc_kernel(const __grid_c
   uint8_t* p_s = ds_s + 2 * 16384;               // [2][128][128 B]   P tile (KV only)
 
   if (tid == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tq) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&td) : "memory");
+    prefetch_tmap(&tq);
+    prefetch_tmap(&td);
     mbar_init(&bar_rows, 1);
     mbar_init(&bar_cols, 1);
     mbar_init(&bar_s, 1);
     mbar_init(&bar_o, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "n"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc<1, 512>(&tmem_slot);
   tcgen05_fence_before();
   __syncthreads();
   tcgen05_fence_after();
@@ -251,19 +247,8 @@ __global__ void __launch_bounds__(128) attn_spatial_bwd_tc_kernel(const __grid_c
   __syncthreads();
   if (warp == 1) {
     tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(512));
+    tmem_dealloc<1, 512>(tmem);
   }
-}
-
-static bool sab_encode(CUtensorMap* m, const void* ptr, int N, int L, int Cs, int rows) {
-  EncodeTiledFn enc = get_tensormap_encoder();
-  if (!enc) return false;
-  cuuint64_t dims[3] = {(cuuint64_t)Cs, (cuuint64_t)L, (cuuint64_t)N};
-  cuuint64_t strides[2] = {(cuuint64_t)Cs * 2, (cuuint64_t)L * Cs * 2};
-  cuuint32_t box[3] = {64, (cuuint32_t)rows, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
 // returns FDM_ERR_UNSUPPORTED for shapes outside the kernel (the caller then uses the CUDA-core kernels)
@@ -282,21 +267,17 @@ int attn_spatial_bwd_tc_launch(const fdm_attn_spatial_bwd_args* a, cudaStream_t 
   p.cf = (F + 63) / 64;
   p.scale = 1.0f / sqrtf((float)F);
   p.scale_log2e = 1.4426950408889634f * p.scale;
+  // qkv [N][L][3C] and dout [N][L][C] as (channel, row, frame) tensors; box (64, rows, 1)
+  const cuuint64_t qdims[3] = {(cuuint64_t)3 * a->C, (cuuint64_t)L, (cuuint64_t)a->N};
+  const cuuint64_t ddims[3] = {(cuuint64_t)a->C, (cuuint64_t)L, (cuuint64_t)a->N};
+  const cuuint32_t box[3] = {64, (cuuint32_t)p.rows, 1};
   CUtensorMap tq, td;
-  FDM_REQUIRE(sab_encode(&tq, a->qkv, a->N, L, 3 * a->C, p.rows) && sab_encode(&td, a->dout, a->N, L, a->C, p.rows), FDM_ERR_UNSUPPORTED);
+  FDM_REQUIRE(encode_bf16_map(&tq, a->qkv, 3, qdims, box, CU_TENSOR_MAP_L2_PROMOTION_L2_128B) &&
+                  encode_bf16_map(&td, a->dout, 3, ddims, box, CU_TENSOR_MAP_L2_PROMOTION_L2_128B), FDM_ERR_UNSUPPORTED);
   const int smem = 4 * p.cf * 16384 + 4 * 16384 + 1024;
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] {
-    attr_err = cudaFuncSetAttribute(attn_spatial_bwd_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (attr_err == cudaSuccess)
-      attr_err = cudaFuncSetAttribute(attn_spatial_bwd_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-  });
-  if (attr_err != cudaSuccess) {
-    set_last_error(attr_err);
-    return FDM_ERR_CUDA;
-  }
   FDM_REQUIRE(smem <= 200 * 1024, FDM_ERR_UNSUPPORTED);
+  if (int rc = allow_smem(attn_spatial_bwd_tc_kernel<false>, 200 * 1024)) return rc;
+  if (int rc = allow_smem(attn_spatial_bwd_tc_kernel<true>, 200 * 1024)) return rc;
   dim3 grid((L + 127) / 128, a->heads, a->N);
   fdm::launch(attn_spatial_bwd_tc_kernel<false>, grid, dim3(128), smem, st, tq, td, p);
   fdm::launch(attn_spatial_bwd_tc_kernel<true>, grid, dim3(128), smem, st, tq, td, p);

@@ -230,8 +230,9 @@ static int launch_temporal_cfg(TAParams& p, cudaStream_t st) {
   p.tgroups = (slots + p.nw - 1) / p.nw;
   dim3 grid((p.HW + 31) / 32, p.heads, p.B * p.tgroups);
   const size_t smem = ((size_t)p.T * KvTile<QT>::WORDS_PER_S + (size_t)p.nw * 2 * TPW * p.T * TA_FC) * sizeof(float);
-  if (smem > 48 * 1024)
-    cudaFuncSetAttribute(attn_temporal_kernel<TP, TPW, QT, OT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (smem > 48 * 1024) {
+    if (int rc = allow_smem(attn_temporal_kernel<TP, TPW, QT, OT>, (int)smem)) return rc;
+  }
   fdm::launch(attn_temporal_kernel<TP, TPW, QT, OT>, dim3(grid), dim3(p.nw * 32), smem, st, p);
   return check_launch();
 }

@@ -17,7 +17,6 @@
 //                      -> TMEM columns [0, F) (aliasing S, which every thread has finished reading)
 //   5. O / rowsum -> bf16 -> out[N][L][C]
 #include "tc_common.cuh"
-#include <mutex>
 
 namespace fdm {
 
@@ -70,17 +69,14 @@ __global__ void __launch_bounds__(256) attn_spatial_tc_kernel(const __grid_const
   uint8_t* p_s = q_s;                          // [ceil(L/64)][128][128 B], aliases Q and K once S is complete
 
   if (tid == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tq) : "memory");
+    prefetch_tmap(&tq);
     mbar_init(&bar_load, 1);
     mbar_init(&bar_v, 1);
     mbar_init(&bar_s, 1);
     mbar_init(&bar_o, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"(p.tmem_cols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc(&tmem_slot, p.tmem_cols);
   tcgen05_fence_before();
   __syncthreads();
   tcgen05_fence_after();
@@ -273,7 +269,7 @@ __global__ void __launch_bounds__(256) attn_spatial_tc_kernel(const __grid_const
   __syncthreads();
   if (warp == 1) {
     tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(p.tmem_cols));
+    tmem_dealloc(tmem, p.tmem_cols);
   }
 }
 
@@ -298,30 +294,16 @@ int attn_spatial_tc_launch(const fdm_attn_spatial_args* a, cudaStream_t st) {
   p.scale_log2e = 1.4426950408889634f / sqrtf((float)F);
   p.lse = a->lse;
   p.attn_mean = a->attn_mean;
-  EncodeTiledFn enc = get_tensormap_encoder();
-  FDM_REQUIRE(enc != nullptr, FDM_ERR_UNSUPPORTED);
   CUtensorMap tq;
-  cuuint64_t dims[3] = {(cuuint64_t)3 * a->C, (cuuint64_t)L, (cuuint64_t)a->N};
-  cuuint64_t strides[2] = {(cuuint64_t)3 * a->C * 2, (cuuint64_t)L * 3 * a->C * 2};
-  cuuint32_t box[3] = {64, (cuuint32_t)p.rows, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  FDM_REQUIRE(enc(&tq, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(a->qkv), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS, FDM_ERR_UNSUPPORTED);
+  const cuuint64_t dims[3] = {(cuuint64_t)3 * a->C, (cuuint64_t)L, (cuuint64_t)a->N};
+  const cuuint32_t box[3] = {64, (cuuint32_t)p.rows, 1};
+  FDM_REQUIRE(encode_bf16_map(&tq, a->qkv, 3, dims, box, CU_TENSOR_MAP_L2_PROMOTION_L2_128B), FDM_ERR_UNSUPPORTED);
   const int kv_tile = L * 128;
   const int pbytes = ((L + 63) / 64) * 16384;
   const int qk = p.cf * (16384 + kv_tile);
   const int smem = p.cf * kv_tile + (qk > pbytes ? qk : pbytes) + 1024;
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] {
-    attr_err = cudaFuncSetAttribute(attn_spatial_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-  });
-  if (attr_err != cudaSuccess) {
-    set_last_error(attr_err);
-    return FDM_ERR_CUDA;
-  }
   FDM_REQUIRE(smem <= 200 * 1024, FDM_ERR_UNSUPPORTED);
+  if (int rc = allow_smem(attn_spatial_tc_kernel, 200 * 1024)) return rc;
   dim3 grid((L + 127) / 128, a->heads, a->N);
   // rows of >= SA_SPLIT_MIN_L keys: two threads per query row (256-thread CTAs)
   fdm::launch(attn_spatial_tc_kernel, dim3(grid), dim3(L >= SA_SPLIT_MIN_L ? 256 : 128), smem, st, tq, p);

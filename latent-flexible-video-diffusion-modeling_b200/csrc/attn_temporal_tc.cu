@@ -22,7 +22,6 @@
 //
 // Data never changes layout on the way: the two row orders are two TMA views (tensor maps) of the same [B*T][HW][3C] qkv tensor.
 #include "tc_common.cuh"
-#include <mutex>
 
 namespace fdm {
 
@@ -98,17 +97,14 @@ __global__ void __launch_bounds__(128) rpe_bias_kernel(const __grid_constant__ C
   uint8_t* rk_s = k_s + p.cf * 16384;        // [cf][Tn][128 B]
   uint8_t* rq_s = rk_s + p.cf * rtile;
   if (tid == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tq) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&trk) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&trq) : "memory");
+    prefetch_tmap(&tq);
+    prefetch_tmap(&trk);
+    prefetch_tmap(&trq);
     mbar_init(&bar_load, 1);
     mbar_init(&bar_d, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"(p.tmem_cols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc(&tmem_slot, p.tmem_cols);
   tcgen05_fence_before();
   __syncthreads();
   tcgen05_fence_after();
@@ -197,7 +193,7 @@ __global__ void __launch_bounds__(128) rpe_bias_kernel(const __grid_constant__ C
   __syncthreads();
   if (warp == 1) {
     tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(p.tmem_cols));
+    tmem_dealloc(tmem, p.tmem_cols);
   }
 }
 
@@ -221,16 +217,13 @@ __global__ void __launch_bounds__(128) attn_rows_kernel(const __grid_constant__ 
   uint8_t* k_s = q_s + p.cf * 16384;      // [cf][128][128 B]
   uint8_t* p_s = q_s;                     // [2][128][128 B]: aliases Q (and K) once S is complete
   if (tid == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tq4) : "memory");
+    prefetch_tmap(&tq4);
     mbar_init(&bar_load, 1);
     mbar_init(&bar_s, 1);
     mbar_init(&bar_o, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"(128));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc(&tmem_slot, 128);
   tcgen05_fence_before();
   __syncthreads();
   tcgen05_fence_after();
@@ -444,7 +437,7 @@ __global__ void __launch_bounds__(128) attn_rows_kernel(const __grid_constant__ 
   __syncthreads();
   if (warp == 1) {
     tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(128));
+    tmem_dealloc(tmem, 128);
   }
 }
 
@@ -469,17 +462,14 @@ __global__ void __launch_bounds__(128) rpe_pv_kernel(const __grid_constant__ CUt
   // global read-modify-write in the epilogue was 85 % of this kernel's stall samples): [rows][F] bf16, not swizzled
   __nv_bfloat16* o_s = reinterpret_cast<__nv_bfloat16*>(rv_s + p.cf * rtile);
   if (tid == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tp4) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&trv) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&to) : "memory");
+    prefetch_tmap(&tp4);
+    prefetch_tmap(&trv);
+    prefetch_tmap(&to);
     mbar_init(&bar_load, 1);
     mbar_init(&bar_d, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"(p.tmem_cols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc(&tmem_slot, p.tmem_cols);
   tcgen05_fence_before();
   __syncthreads();
   tcgen05_fence_after();
@@ -549,7 +539,7 @@ __global__ void __launch_bounds__(128) rpe_pv_kernel(const __grid_constant__ CUt
   __syncthreads();
   if (warp == 1) {
     tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(p.tmem_cols));
+    tmem_dealloc(tmem, p.tmem_cols);
   }
 }
 
@@ -590,24 +580,6 @@ size_t attn_temporal_tc_workspace(const fdm_attn_temporal_args* a) {
   return 2 * rows * TS * sizeof(__nv_bfloat16) + rows * 64 * sizeof(__nv_bfloat16);
 }
 
-template <typename Kern>
-static int tt_set_smem(Kern k, int bytes) {
-  cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-  if (e != cudaSuccess) {
-    set_last_error(e);
-    return FDM_ERR_CUDA;
-  }
-  return FDM_OK;
-}
-
-static bool tt_encode(CUtensorMap* m, const void* ptr, int rank, const cuuint64_t* dims, const cuuint64_t* strides, const cuuint32_t* box) {
-  EncodeTiledFn enc = get_tensormap_encoder();
-  if (!enc) return false;
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, rank, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 // returns FDM_ERR_UNSUPPORTED for shapes outside these kernels (the caller then runs the CUDA-core kernel)
 int attn_temporal_tc_launch(const fdm_attn_temporal_args* a, cudaStream_t st) {
   if (!tt_shape_ok(a) || !a->Rq_op || !a->Rk_op || !a->Rv_op || !a->workspace) return FDM_ERR_UNSUPPORTED;
@@ -631,75 +603,55 @@ int attn_temporal_tc_launch(const fdm_attn_temporal_args* a, cudaStream_t st) {
   const int TP = T <= 8 ? 8 : (T <= 16 ? 16 : (T <= 32 ? 32 : 64));
   const int PL = 128 / TP;
 
-  CUtensorMap tq3, tq4, trq, trk, trv, tp4;
+  const CUtensorMapL2promotion L2 = CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
+  CUtensorMap tq3, tq4, trq, trk, trv, tp4, to;
   {
-    cuuint64_t dims[3] = {(cuuint64_t)3 * C, (cuuint64_t)HW, (cuuint64_t)B * T};
-    cuuint64_t strides[2] = {(cuuint64_t)3 * C * 2, (cuuint64_t)HW * 3 * C * 2};
-    cuuint32_t box[3] = {64, (cuuint32_t)p.rows, 1};
-    FDM_REQUIRE(tt_encode(&tq3, a->qkv, 3, dims, strides, box), FDM_ERR_UNSUPPORTED);
+    const cuuint64_t dims[3] = {(cuuint64_t)3 * C, (cuuint64_t)HW, (cuuint64_t)B * T};
+    const cuuint32_t box[3] = {64, (cuuint32_t)p.rows, 1};
+    FDM_REQUIRE(encode_bf16_map(&tq3, a->qkv, 3, dims, box, L2), FDM_ERR_UNSUPPORTED);
   }
   {
     // the same tensor with rows ordered (pixel, frame): dims (channel, frame, pixel, video)
-    cuuint64_t dims[4] = {(cuuint64_t)3 * C, (cuuint64_t)T, (cuuint64_t)HW, (cuuint64_t)B};
-    cuuint64_t strides[3] = {(cuuint64_t)HW * 3 * C * 2, (cuuint64_t)3 * C * 2, (cuuint64_t)T * HW * 3 * C * 2};
-    cuuint32_t box[4] = {64, (cuuint32_t)TP, (cuuint32_t)PL, 1};
-    FDM_REQUIRE(tt_encode(&tq4, a->qkv, 4, dims, strides, box), FDM_ERR_UNSUPPORTED);
+    const cuuint64_t dims[4] = {(cuuint64_t)3 * C, (cuuint64_t)T, (cuuint64_t)HW, (cuuint64_t)B};
+    const cuuint64_t strides[3] = {(cuuint64_t)HW * 3 * C * 2, (cuuint64_t)3 * C * 2, (cuuint64_t)T * HW * 3 * C * 2};
+    const cuuint32_t box[4] = {64, (cuuint32_t)TP, (cuuint32_t)PL, 1};
+    FDM_REQUIRE(encode_bf16_map(&tq4, a->qkv, 4, dims, box, L2, CU_TENSOR_MAP_SWIZZLE_128B, strides), FDM_ERR_UNSUPPORTED);
   }
   {
-    cuuint64_t dims[3] = {(cuuint64_t)C, (cuuint64_t)T, (cuuint64_t)B * T};
-    cuuint64_t strides[2] = {(cuuint64_t)C * 2, (cuuint64_t)T * C * 2};
-    cuuint32_t box[3] = {64, (cuuint32_t)p.Tn, 1};
-    FDM_REQUIRE(tt_encode(&trq, a->Rq_op, 3, dims, strides, box) && tt_encode(&trk, a->Rk_op, 3, dims, strides, box) &&
-                    tt_encode(&trv, a->Rv_op, 3, dims, strides, box), FDM_ERR_UNSUPPORTED);
+    const cuuint64_t dims[3] = {(cuuint64_t)C, (cuuint64_t)T, (cuuint64_t)B * T};
+    const cuuint32_t box[3] = {64, (cuuint32_t)p.Tn, 1};
+    FDM_REQUIRE(encode_bf16_map(&trq, a->Rq_op, 3, dims, box, L2) && encode_bf16_map(&trk, a->Rk_op, 3, dims, box, L2) &&
+                    encode_bf16_map(&trv, a->Rv_op, 3, dims, box, L2), FDM_ERR_UNSUPPORTED);
   }
   {
-    cuuint64_t dims[4] = {64, (cuuint64_t)T, (cuuint64_t)HW, (cuuint64_t)B * heads};
-    cuuint64_t strides[3] = {128, (cuuint64_t)T * 128, (cuuint64_t)HW * T * 128};
-    cuuint32_t box[4] = {64, 1, (cuuint32_t)p.rows, 1};
-    FDM_REQUIRE(tt_encode(&tp4, p.P, 4, dims, strides, box), FDM_ERR_UNSUPPORTED);
+    const cuuint64_t dims[4] = {64, (cuuint64_t)T, (cuuint64_t)HW, (cuuint64_t)B * heads};
+    const cuuint32_t box[4] = {64, 1, (cuuint32_t)p.rows, 1};
+    FDM_REQUIRE(encode_bf16_map(&tp4, p.P, 4, dims, box, L2), FDM_ERR_UNSUPPORTED);
   }
-  CUtensorMap to;
   {
     // `out` as (channel, pixel, frame): box = one head's F channels x the tile's pixels, no swizzle (read by plain ld.shared)
-    EncodeTiledFn enc = get_tensormap_encoder();
-    cuuint64_t dims[3] = {(cuuint64_t)C, (cuuint64_t)HW, (cuuint64_t)B * T};
-    cuuint64_t strides[2] = {(cuuint64_t)C * 2, (cuuint64_t)HW * C * 2};
-    cuuint32_t box[3] = {(cuuint32_t)F, (cuuint32_t)p.rows, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    FDM_REQUIRE(enc != nullptr && enc(&to, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, a->out, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                                      CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS, FDM_ERR_UNSUPPORTED);
+    const cuuint64_t dims[3] = {(cuuint64_t)C, (cuuint64_t)HW, (cuuint64_t)B * T};
+    const cuuint32_t box[3] = {(cuuint32_t)F, (cuuint32_t)p.rows, 1};
+    FDM_REQUIRE(encode_bf16_map(&to, a->out, 3, dims, box, L2, CU_TENSOR_MAP_SWIZZLE_NONE), FDM_ERR_UNSUPPORTED);
   }
   const int smem1 = p.cf * (2 * 16384 + 2 * p.Tn * 128) + 1024;
   const int smem2 = p.cf * 3 * 16384 + 2 * PL * T * p.TS * (int)sizeof(__nv_bfloat16) + 1024;  // P (32 KB) aliases Q + K; + bias tiles
   const int smem3 = 16384 + p.cf * p.Tn * 128 + p.rows * F * 2 + 1024;
-  static std::once_flag once;
-  static int attr_rc = FDM_OK;
-  std::call_once(once, [] {
-    int rc = tt_set_smem(rpe_bias_kernel, 100 * 1024);
-    if (rc == FDM_OK) rc = tt_set_smem(attn_rows_kernel<8>, 200 * 1024);
-    if (rc == FDM_OK) rc = tt_set_smem(attn_rows_kernel<16>, 200 * 1024);
-    if (rc == FDM_OK) rc = tt_set_smem(attn_rows_kernel<32>, 200 * 1024);
-    if (rc == FDM_OK) rc = tt_set_smem(attn_rows_kernel<64>, 200 * 1024);
-    if (rc == FDM_OK) rc = tt_set_smem(rpe_pv_kernel, 100 * 1024);
-    attr_rc = rc;
-  });
-  if (attr_rc != FDM_OK) return attr_rc;
   FDM_REQUIRE(smem1 <= 100 * 1024 && smem2 <= 200 * 1024 && smem3 <= 100 * 1024, FDM_ERR_UNSUPPORTED);
+  const auto rows_kernel =
+      TP == 8 ? attn_rows_kernel<8> : TP == 16 ? attn_rows_kernel<16> : TP == 32 ? attn_rows_kernel<32> : attn_rows_kernel<64>;
+  int rc = allow_smem(rpe_bias_kernel, 100 * 1024);
+  if (rc == FDM_OK) rc = allow_smem(rows_kernel, 200 * 1024);
+  if (rc == FDM_OK) rc = allow_smem(rpe_pv_kernel, 100 * 1024);
+  if (rc != FDM_OK) return rc;
 
   TtParams p1 = p;
   p1.tmem_cols = tt_pow2(2 * p.Tn, 32);
   dim3 gridA((HW + 127) / 128, T, B * heads);
   fdm::launch(rpe_bias_kernel, gridA, dim3(128), smem1, st, tq3, trk, trq, p1);
-  int rc = check_launch();
+  rc = check_launch();
   if (rc != FDM_OK) return rc;
-  dim3 gridB(HW / PL, heads, B);
-  switch (TP) {
-    case 8: fdm::launch(attn_rows_kernel<8>, gridB, dim3(128), smem2, st, tq4, p); break;
-    case 16: fdm::launch(attn_rows_kernel<16>, gridB, dim3(128), smem2, st, tq4, p); break;
-    case 32: fdm::launch(attn_rows_kernel<32>, gridB, dim3(128), smem2, st, tq4, p); break;
-    default: fdm::launch(attn_rows_kernel<64>, gridB, dim3(128), smem2, st, tq4, p); break;
-  }
+  fdm::launch(rows_kernel, dim3(HW / PL, heads, B), dim3(128), smem2, st, tq4, p);
   rc = check_launch();
   if (rc != FDM_OK) return rc;
   TtParams p3 = p;

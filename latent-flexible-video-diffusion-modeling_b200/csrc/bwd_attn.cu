@@ -756,8 +756,8 @@ extern "C" int fdm_attn_spatial_bwd(const fdm_attn_spatial_bwd_args* a, void* st
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
 #define FDM_SA_BWD(QT)                                                                                                  \
   do {                                                                                                                  \
-    cudaFuncSetAttribute(attn_spatial_bwd_q_kernel<QT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_q);      \
-    cudaFuncSetAttribute(attn_spatial_bwd_kv_kernel<QT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_kv);    \
+    if (int rc = allow_smem(attn_spatial_bwd_q_kernel<QT>, (int)smem_q)) return rc;                                     \
+    if (int rc = allow_smem(attn_spatial_bwd_kv_kernel<QT>, (int)smem_kv)) return rc;                                   \
     fdm::launch(attn_spatial_bwd_q_kernel<QT>, grid, dim3(256), smem_q, st, p);                                         \
     fdm::launch(attn_spatial_bwd_kv_kernel<QT>, grid, dim3(256), smem_kv, st, p);                                       \
   } while (0)
@@ -767,7 +767,7 @@ extern "C" int fdm_attn_spatial_bwd(const fdm_attn_spatial_bwd_args* a, void* st
 }
 
 template <int TP, typename QT>
-static void launch_ta_bwd(const TABwdParams& p, cudaStream_t st) {
+static int launch_ta_bwd(const TABwdParams& p, cudaStream_t st) {
   const int T = p.T;
   // frames (warps) per CTA.  Fewer warps per CTA (more CTAs on the small feature maps, where 8-warp CTAs number only 48-192) was
   // measured SLOWER on B200 (cfg3: 3.7 -> 4.9 ms per step): every CTA re-stages all T key/value frames, so halving the frames
@@ -775,10 +775,11 @@ static void launch_ta_bwd(const TABwdParams& p, cudaStream_t st) {
   const size_t smem_q = ((size_t)2 * T * TB_FC * TB_LD + (size_t)TB_WARPS * (3 * T * TB_FC + T * TB_LD + TB_FC * TB_LD)) * sizeof(float);
   const size_t smem_kv = ((size_t)2 * T * TB_FC * TB_LD + (size_t)TB_WARPS * (3 * T * TB_FC + 2 * T * TB_LD + TB_FC * TB_LD)) * sizeof(float);
   dim3 grid((p.HW + 31) / 32, p.heads, p.B * ((T + TB_WARPS - 1) / TB_WARPS));
-  cudaFuncSetAttribute(attn_temporal_bwd_q_kernel<TP, QT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_q);
-  cudaFuncSetAttribute(attn_temporal_bwd_kv_kernel<TP, QT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_kv);
+  if (int rc = allow_smem(attn_temporal_bwd_q_kernel<TP, QT>, (int)smem_q)) return rc;
+  if (int rc = allow_smem(attn_temporal_bwd_kv_kernel<TP, QT>, (int)smem_kv)) return rc;
   fdm::launch(attn_temporal_bwd_q_kernel<TP, QT>, grid, dim3(TB_WARPS * 32), smem_q, st, p);
   fdm::launch(attn_temporal_bwd_kv_kernel<TP, QT>, grid, dim3(TB_WARPS * 32), smem_kv, st, p);
+  return check_launch();
 }
 
 extern "C" int fdm_attn_temporal_bwd(const fdm_attn_temporal_bwd_args* a, void* stream) {
@@ -792,13 +793,12 @@ extern "C" int fdm_attn_temporal_bwd(const fdm_attn_temporal_bwd_args* a, void* 
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
 #define FDM_TA_BWD(QT)                                      \
   do {                                                      \
-    if (a->T <= 8) launch_ta_bwd<8, QT>(p, st);             \
-    else if (a->T <= 16) launch_ta_bwd<16, QT>(p, st);      \
-    else if (a->T <= 24) launch_ta_bwd<24, QT>(p, st);      \
-    else if (a->T <= 32) launch_ta_bwd<32, QT>(p, st);      \
-    else launch_ta_bwd<40, QT>(p, st);                      \
+    if (a->T <= 8) return launch_ta_bwd<8, QT>(p, st);      \
+    if (a->T <= 16) return launch_ta_bwd<16, QT>(p, st);    \
+    if (a->T <= 24) return launch_ta_bwd<24, QT>(p, st);    \
+    if (a->T <= 32) return launch_ta_bwd<32, QT>(p, st);    \
+    return launch_ta_bwd<40, QT>(p, st);                    \
   } while (0)
   if (a->dtype == FDM_BF16) FDM_TA_BWD(__nv_bfloat16);
-  else FDM_TA_BWD(float);
-  return check_launch();
+  FDM_TA_BWD(float);
 }

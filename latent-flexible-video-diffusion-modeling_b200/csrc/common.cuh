@@ -18,6 +18,19 @@ inline int check_launch() {
   return FDM_OK;
 }
 
+// Lets `kernel` use `bytes` of dynamic shared memory (above the 48 KB default) on the CURRENT device: a kernel's attributes belong
+// to its instance in each device's context, so this is called before every launch that needs it (CUDA-graph replays do not
+// repeat it).  FDM_ERR_CUDA when the runtime refuses.
+template <typename... KArgs>
+inline int allow_smem(void (*kernel)(KArgs...), int bytes) {
+  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  if (e != cudaSuccess) {
+    set_last_error(e);
+    return FDM_ERR_CUDA;
+  }
+  return FDM_OK;
+}
+
 #define FDM_REQUIRE(cond, code) \
   do {                          \
     if (!(cond)) return (code); \

@@ -25,7 +25,6 @@
 // CTAs, so the release would come at kernel start and the next kernel's CTAs would sit on the SMs for the whole run (measured: +4 %
 // on the cfg5 / cfg3 steps).
 #include "tc_common.cuh"
-#include <mutex>
 
 namespace fdm {
 
@@ -82,11 +81,11 @@ __global__ void __launch_bounds__(HALO_THREADS, 1) conv_halo_kernel(const __grid
   float* statbuf = staging + 8 * 32 * 16;                                              // [2 buffers][2 tiles][4 lane groups][BN][2]
 
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&ta0) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tw0) : "memory");
+    prefetch_tmap(&ta0);
+    prefetch_tmap(&tw0);
     if (p.kchunks1) {
-      asm volatile("prefetch.tensormap [%0];" ::"l"(&ta1) : "memory");
-      asm volatile("prefetch.tensormap [%0];" ::"l"(&tw1) : "memory");
+      prefetch_tmap(&ta1);
+      prefetch_tmap(&tw1);
     }
   }
   if (warp == 1 && lane == 0) {
@@ -98,17 +97,9 @@ __global__ void __launch_bounds__(HALO_THREADS, 1) conv_halo_kernel(const __grid
       mbar_init(&tmem_full_bar[i], 1);
       mbar_init(&tmem_empty_bar[i], 8 * CG);  // one arrival per epilogue warp (of both CTAs: the leader's copy is the live one)
     }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
-  if (warp == 2) {
-    if (CG == 2) {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)), "n"(TMEM_COLS));
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)), "n"(TMEM_COLS));
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
-  }
+  if (warp == 2) tmem_alloc<CG, TMEM_COLS>(&tmem_base_slot);
   tcgen05_fence_before();
   __syncthreads();
   if (CG == 2) cluster_sync_all();  // the peer's barriers are initialised before anything signals them
@@ -392,34 +383,11 @@ __global__ void __launch_bounds__(HALO_THREADS, 1) conv_halo_kernel(const __grid
   if (CG == 2) cluster_sync_all();  // neither CTA leaves while the other may still signal its barriers or read its shared memory
   if (warp == 2) {
     tcgen05_fence_after();
-    if (CG == 2) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS));
-    else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS));
+    tmem_dealloc<CG, TMEM_COLS>(tmem_base);
   }
 }
 
 // ---------------------------------------------------------------- host side
-static bool encode4(CUtensorMap* m, const void* ptr, int N, int H, int W, int C, int rows) {
-  EncodeTiledFn enc = get_tensormap_encoder();
-  if (!enc) return false;
-  cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
-  cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
-  cuuint32_t box[4] = {64, (cuuint32_t)W, (cuuint32_t)rows, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-static bool encode3w(CUtensorMap* m, const void* ptr, int taps, int co_pad, int ci_pad, int bn, int box_taps) {
-  EncodeTiledFn enc = get_tensormap_encoder();
-  if (!enc) return false;
-  cuuint64_t dims[3] = {(cuuint64_t)ci_pad, (cuuint64_t)co_pad, (cuuint64_t)taps};
-  cuuint64_t strides[2] = {(cuuint64_t)ci_pad * 2, (cuuint64_t)co_pad * ci_pad * 2};
-  cuuint32_t box[3] = {64, (cuuint32_t)bn, (cuuint32_t)box_taps};
-  cuuint32_t estr[3] = {1, 1, 1};
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
-static int g_num_sms = 0;
 static long long* g_trace = nullptr;
 
 template <int BN, int TPI, int CG, bool UP>
@@ -434,21 +402,11 @@ static int launch_halo_cg(const CUtensorMap& ta0, const CUtensorMap& tw0, const 
   if (p.stages > HALO_MAX_STAGES) p.stages = HALO_MAX_STAGES;
   if (p.stages < 2) return FDM_ERR_UNSUPPORTED;
   const int smem = p.stages * p.stage_bytes + extra;
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] {
-    attr_err = cudaFuncSetAttribute(conv_halo_kernel<BN, TPI, CG, UP>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_MAX);
-    if (g_num_sms == 0) {
-      int dev = 0;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev);
-    }
-  });
-  if (attr_err != cudaSuccess) {
-    set_last_error(attr_err);
-    return FDM_ERR_CUDA;
-  }
-  const int sms = g_num_sms > 0 ? g_num_sms : 148;
+  if (int rc = allow_smem(conv_halo_kernel<BN, TPI, CG, UP>, SMEM_MAX)) return rc;
+  int dev = 0, sms = 0;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  if (sms <= 0) sms = 148;
   if (CG == 2) {
     const int pairs = sms / 2, n_q = p.n_items / 2;
     fdm::launch_cluster(conv_halo_kernel<BN, TPI, CG, UP>, dim3(2 * (n_q < pairs ? n_q : pairs)), dim3(HALO_THREADS), smem, st, 2, ta0, tw0, ta1, tw1, p);
@@ -540,11 +498,21 @@ int conv_halo_launch(const fdm_conv_args* a, cudaStream_t st) {
   p.pairs_per_frame = H / (p.tpi * hbox);
   p.n_items = N * p.pairs_per_frame * p.ntiles * p.nph;
   const int brows = pair ? bn / 2 : bn;
+  // activations [N][H][W][C] as a (C, W, H, N) tensor, box (64, W, rows, 1); weights [taps][co_pad][ci_pad] as a
+  // (ci_pad, co_pad, taps) tensor, box (64, brows, ks taps)
+  const CUtensorMapL2promotion L2_ACT = CU_TENSOR_MAP_L2_PROMOTION_L2_128B, L2_W = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
+  const cuuint64_t adims0[4] = {(cuuint64_t)a->C0, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
+  const cuuint32_t abox0[4] = {64, (cuuint32_t)W, (cuuint32_t)(p.tpi * hbox + p.ks - 1), 1};
+  const cuuint64_t wdims0[3] = {(cuuint64_t)p.kchunks0 * 64, (cuuint64_t)co_pad, (cuuint64_t)(up ? 16 : a->ksize * a->ksize)};
+  const cuuint32_t wbox0[3] = {64, (cuuint32_t)brows, (cuuint32_t)p.ks};
   CUtensorMap ta0, tw0, ta1, tw1;
-  bool ok = encode4(&ta0, a->a0, N, H, W, a->C0, p.tpi * hbox + p.ks - 1) &&
-            encode3w(&tw0, a->w0, up ? 16 : a->ksize * a->ksize, co_pad, p.kchunks0 * 64, brows, p.ks);
+  bool ok = encode_bf16_map(&ta0, a->a0, 4, adims0, abox0, L2_ACT) && encode_bf16_map(&tw0, a->w0, 3, wdims0, wbox0, L2_W);
   if (ok && a->a1) {
-    ok = encode4(&ta1, a->a1, N, H, W, a->C1, p.tpi * hbox) && encode3w(&tw1, a->w1, 1, co_pad, p.kchunks1 * 64, brows, 1);
+    const cuuint64_t adims1[4] = {(cuuint64_t)a->C1, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
+    const cuuint32_t abox1[4] = {64, (cuuint32_t)W, (cuuint32_t)(p.tpi * hbox), 1};
+    const cuuint64_t wdims1[3] = {(cuuint64_t)p.kchunks1 * 64, (cuuint64_t)co_pad, 1};
+    const cuuint32_t wbox1[3] = {64, (cuuint32_t)brows, 1};
+    ok = encode_bf16_map(&ta1, a->a1, 4, adims1, abox1, L2_ACT) && encode_bf16_map(&tw1, a->w1, 3, wdims1, wbox1, L2_W);
   } else {
     ta1 = ta0;
     tw1 = tw0;

@@ -10,7 +10,6 @@
 // strip's pixels are covered by 128-row MMA tiles whose 48-column accumulators all stay in TMEM, then Z is spilled to shared memory
 // (over the dead input tile) and every thread gathers the 9 shifted float4s of its output pixels and writes coalesced NCHW rows.
 #include "tc_common.cuh"
-#include <mutex>
 
 namespace fdm {
 
@@ -41,15 +40,12 @@ __global__ void __launch_bounds__(HEAD_THREADS) conv_head_kernel(const __grid_co
   uint8_t* b_s = smem;                               // [nchunks][48 rows][128 B], K-major, 128-byte swizzle
   uint8_t* a_s = smem + p.nchunks * HEAD_NC * 128;   // [nchunks][ntile * 128 pixels][128 B]; later Z: [pixels][36] fp32
   if (tid == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&ta) : "memory");
+    prefetch_tmap(&ta);
     for (int c = 0; c < p.nchunks; ++c) mbar_init(&load_bar[c], 1);
     mbar_init(&mma_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"(p.tmem_cols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc(&tmem_slot, p.tmem_cols);
   // weight tile: rows (tap, co < 4) of the packed weights, written in the swizzled K-major layout; rows 36..47 are zero.
   // (parameters are never written by the preceding launch of the stream, so this runs before the dependency wait)
   for (int i = tid; i < p.nchunks * HEAD_NC * 8; i += HEAD_THREADS) {
@@ -116,7 +112,7 @@ __global__ void __launch_bounds__(HEAD_THREADS) conv_head_kernel(const __grid_co
   __syncthreads();
   if (warp == 1) {
     tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(p.tmem_cols));
+    tmem_dealloc(tmem, p.tmem_cols);
   }
   float bias[4];
 #pragma unroll
@@ -140,17 +136,6 @@ __global__ void __launch_bounds__(HEAD_THREADS) conv_head_kernel(const __grid_co
     for (int co = 0; co < 4; ++co)
       if (co < p.Cout) y[(size_t)co * HW] = acc[co];
   }
-}
-
-static bool head_encode(CUtensorMap* m, const void* ptr, int N, int H, int W, int C, int rows) {
-  EncodeTiledFn enc = get_tensormap_encoder();
-  if (!enc) return false;
-  cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
-  cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
-  cuuint32_t box[4] = {64, (cuuint32_t)W, (cuuint32_t)rows, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
 // FDM_ERR_UNSUPPORTED => the caller falls back to the per-tap kernel
@@ -195,15 +180,12 @@ int conv_head_launch(const fdm_conv_args* a, cudaStream_t st) {
   while (p.tmem_cols < p.ntile * HEAD_NC) p.tmem_cols *= 2;
   const long a_bytes = (long)p.nchunks * p.ntile * 16384, z_bytes = (long)p.ntile * 128 * HEAD_ZW * 4;
   const int smem = 1024 + p.nchunks * HEAD_NC * 128 + (int)(a_bytes > z_bytes ? a_bytes : z_bytes);
+  // activations [N][H][W][C] as a (C, W, H, N) tensor, box (64, W, R + 2 rows, 1)
+  const cuuint64_t dims[4] = {(cuuint64_t)a->C0, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)a->N};
+  const cuuint32_t box[4] = {64, (cuuint32_t)W, (cuuint32_t)(p.R + 2), 1};
   CUtensorMap ta;
-  FDM_REQUIRE(head_encode(&ta, a->a0, a->N, H, W, a->C0, p.R + 2), FDM_ERR_UNSUPPORTED);
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] { attr_err = cudaFuncSetAttribute(conv_head_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024); });
-  if (attr_err != cudaSuccess) {
-    set_last_error(attr_err);
-    return FDM_ERR_CUDA;
-  }
+  FDM_REQUIRE(encode_bf16_map(&ta, a->a0, 4, dims, box, CU_TENSOR_MAP_L2_PROMOTION_L2_128B), FDM_ERR_UNSUPPORTED);
+  if (int rc = allow_smem(conv_head_kernel, smem_cap)) return rc;
   fdm::launch(conv_head_kernel, dim3(a->N * p.strips_per_frame), dim3(HEAD_THREADS), (size_t)smem, st, ta, p);
   return check_launch();
 }

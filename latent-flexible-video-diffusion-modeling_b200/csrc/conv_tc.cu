@@ -16,7 +16,6 @@
 //   The staging buffer aliases the operand ring (all MMAs have retired when the epilogue starts; one tile per CTA),
 //   so two CTAs fit per SM and one CTA's epilogue overlaps the other's main loop.
 #include "tc_common.cuh"
-#include <mutex>
 
 namespace fdm {
 
@@ -89,11 +88,11 @@ __global__ void __launch_bounds__(TC_THREADS, RN ? 3 : 0) conv_tc_kernel(const _
   constexpr int B_TAP_BYTES = BN * 128;
 
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&ta0) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tw0) : "memory");
+    prefetch_tmap(&ta0);
+    prefetch_tmap(&tw0);
     if (p.kchunks1) {
-      asm volatile("prefetch.tensormap [%0];" ::"l"(&ta1) : "memory");
-      asm volatile("prefetch.tensormap [%0];" ::"l"(&tw1) : "memory");
+      prefetch_tmap(&ta1);
+      prefetch_tmap(&tw1);
     }
   }
   if (warp == 1 && lane == 0) {
@@ -102,12 +101,9 @@ __global__ void __launch_bounds__(TC_THREADS, RN ? 3 : 0) conv_tc_kernel(const _
       mbar_init(&empty_bar[i], 1);
     }
     mbar_init(&tmem_full_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
-  if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)), "n"(S::TMEM_COLS));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 2) tmem_alloc<1, S::TMEM_COLS>(&tmem_base_slot);
   tcgen05_fence_before();
   __syncthreads();
   tcgen05_fence_after();
@@ -418,62 +414,16 @@ __global__ void __launch_bounds__(TC_THREADS, RN ? 3 : 0) conv_tc_kernel(const _
   __syncthreads();
   if (warp == 2) {
     tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(S::TMEM_COLS));
+    tmem_dealloc<1, S::TMEM_COLS>(tmem_base);
   }
 }
 
 // ---------------------------------------------------------------- host side
-EncodeTiledFn get_tensormap_encoder() {
-  static EncodeTiledFn fn = nullptr;
-  static std::once_flag once;
-  std::call_once(once, [] {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  });
-  return fn;
-}
-
-// activations [N][H][W][C] bf16 as a (C, W, H, N) tensor; box (64, wbox*sw, hbox*sh, nbox) traversed with stride (1, s, s, 1)
-static bool encode_act(CUtensorMap* m, const void* ptr, int N, int H, int W, int C, int wbox, int hbox, int nbox, int stride) {
-  EncodeTiledFn enc = get_tensormap_encoder();
-  if (!enc) return false;
-  cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
-  cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
-  cuuint32_t box[4] = {(cuuint32_t)TC_BK, (cuuint32_t)(wbox * stride), (cuuint32_t)(hbox * stride), (cuuint32_t)nbox};
-  cuuint32_t estr[4] = {1, (cuuint32_t)stride, (cuuint32_t)stride, 1};
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
-// weights [taps][co_pad][ci_pad] bf16 as a (ci_pad, co_pad, taps) tensor; box (64, BN, 1)
-static bool encode_w(CUtensorMap* m, const void* ptr, int taps, int co_pad, int ci_pad, int bn, int box_taps) {
-  EncodeTiledFn enc = get_tensormap_encoder();
-  if (!enc) return false;
-  cuuint64_t dims[3] = {(cuuint64_t)ci_pad, (cuuint64_t)co_pad, (cuuint64_t)taps};
-  cuuint64_t strides[2] = {(cuuint64_t)ci_pad * 2, (cuuint64_t)co_pad * ci_pad * 2};
-  cuuint32_t box[3] = {(cuuint32_t)TC_BK, (cuuint32_t)bn, (cuuint32_t)box_taps};
-  cuuint32_t estr[3] = {1, 1, 1};
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 template <int BN, bool RN = false>
 static int launch_tc(const CUtensorMap& ta0, const CUtensorMap& tw0, const CUtensorMap& ta1, const CUtensorMap& tw1,
                      TcParams& p, cudaStream_t st) {
   using S = TcSmem<BN>;
   constexpr int SMEM_MAX = (RN ? 216 : 226) * 1024;  // RN: 8.3 KB of static shared memory (the coefficient table)
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] {
-    attr_err = cudaFuncSetAttribute(conv_tc_kernel<BN, RN>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_MAX);
-  });
-  if (attr_err != cudaSuccess) {
-    set_last_error(attr_err);
-    return FDM_ERR_CUDA;
-  }
   dim3 grid((p.M + TC_BM - 1) / TC_BM, (p.Cout + BN - 1) / BN);
   // pipeline depth: a grid that cannot even fill the SMs once is latency-bound -> one CTA per SM with as many operand
   // stages in flight as the K loop has iterations (up to 8); otherwise two CTAs per SM share the shared memory.
@@ -486,6 +436,7 @@ static int launch_tc(const CUtensorMap& ta0, const CUtensorMap& tw0, const CUten
   if (stages > iters) stages = iters;
   if (stages < 1) return FDM_ERR_UNSUPPORTED;
   p.stages = stages;
+  if (int rc = allow_smem(conv_tc_kernel<BN, RN>, SMEM_MAX)) return rc;
   fdm::launch(conv_tc_kernel<BN, RN>, dim3(grid), dim3(TC_THREADS), stages * p.stage_bytes + S::EXTRA_BYTES, st, ta0, tw0, ta1, tw1, p);
   return check_launch();
 }
@@ -549,12 +500,23 @@ int conv_tc_launch(const fdm_conv_args* a, cudaStream_t st) {
   // filter rows of a filter column into one stage so a single weight box serves three taps
   const long ctas = (long)mtiles * ((a->Cout + bn - 1) / bn);
   p.nr = (a->ksize == 3 && ctas <= 148) ? 3 : 1;
+  // activations [N][H][W][C] as a (C, W, H, N) tensor, box (64, wbox * s, hbox * s, nbox) traversed with element strides
+  // (1, s, s, 1); weights [taps][co_pad][ci_pad] as a (ci_pad, co_pad, taps) tensor, box (64, BN, nr taps)
+  const CUtensorMapL2promotion L2_ACT = CU_TENSOR_MAP_L2_PROMOTION_L2_128B, L2_W = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
+  const cuuint32_t s = (cuuint32_t)a->stride;
+  const cuuint64_t adims0[4] = {(cuuint64_t)a->C0, (cuuint64_t)a->Win, (cuuint64_t)a->Hin, (cuuint64_t)a->N};
+  const cuuint32_t abox0[4] = {TC_BK, p.wbox * s, p.hbox * s, (cuuint32_t)p.nbox}, aestr0[4] = {1, s, s, 1};
+  const cuuint64_t wdims0[3] = {(cuuint64_t)round_up(a->C0, TC_BK), (cuuint64_t)co_pad, (cuuint64_t)p.taps};
+  const cuuint32_t wbox0[3] = {TC_BK, (cuuint32_t)bn, (cuuint32_t)p.nr};
   CUtensorMap ta0, tw0, ta1, tw1;
-  bool ok = encode_act(&ta0, a->a0, a->N, a->Hin, a->Win, a->C0, p.wbox, p.hbox, p.nbox, a->stride) &&
-            encode_w(&tw0, a->w0, p.taps, co_pad, round_up(a->C0, TC_BK), bn, p.nr);
+  bool ok = encode_bf16_map(&ta0, a->a0, 4, adims0, abox0, L2_ACT, CU_TENSOR_MAP_SWIZZLE_128B, nullptr, aestr0) &&
+            encode_bf16_map(&tw0, a->w0, 3, wdims0, wbox0, L2_W);
   if (ok && a->a1) {
-    ok = encode_act(&ta1, a->a1, a->N, Ho, Wo, a->C1, p.wbox, p.hbox, p.nbox, 1) &&
-         encode_w(&tw1, a->w1, 1, co_pad, round_up(a->C1, TC_BK), bn, 1);
+    const cuuint64_t adims1[4] = {(cuuint64_t)a->C1, (cuuint64_t)Wo, (cuuint64_t)Ho, (cuuint64_t)a->N};
+    const cuuint32_t abox1[4] = {TC_BK, (cuuint32_t)p.wbox, (cuuint32_t)p.hbox, (cuuint32_t)p.nbox};
+    const cuuint64_t wdims1[3] = {(cuuint64_t)round_up(a->C1, TC_BK), (cuuint64_t)co_pad, 1};
+    const cuuint32_t wbox1[3] = {TC_BK, (cuuint32_t)bn, 1};
+    ok = encode_bf16_map(&ta1, a->a1, 4, adims1, abox1, L2_ACT) && encode_bf16_map(&tw1, a->w1, 3, wdims1, wbox1, L2_W);
   } else {
     ta1 = ta0;
     tw1 = tw0;

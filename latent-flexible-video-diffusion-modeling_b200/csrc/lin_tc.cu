@@ -31,7 +31,6 @@
 // Shapes: K = C = 128 (two 64-channel chunks; a GroupNorm group = 4 channels = one float4), Cout = 128 / 256 / 384, HW % 16 == 0,
 // a_mode 2: T <= 20 (a pixel's T rows live in one warp's registers).
 #include "tc_common.cuh"
-#include <mutex>
 
 namespace fdm {
 
@@ -121,17 +120,14 @@ __global__ void __launch_bounds__(NL_WORKERS, 1) nl_qkv_kernel(const __grid_cons
   uint8_t* stg_s = a_s + NL_A_BYTES;       // [Cout / 64 blocks][128 rows][128 B]: the whole output tile, drained by TMA stores
 
   if (threadIdx.x == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tw) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&ty) : "memory");
+    prefetch_tmap(&tw);
+    prefetch_tmap(&ty);
     mbar_init(&w_bar, 1);
     mbar_init(&a_ready, 8);
     for (int i = 0; i < 3; ++i) mbar_init(&mma_bar[i], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "n"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc<1, 512>(&tmem_slot);
   for (int i = threadIdx.x; i < p.Cout; i += NL_WORKERS) bias_s[i] = p.bias[i];  // parameters: not written by the previous kernel
   tcgen05_fence_before();
   __syncthreads();
@@ -323,20 +319,11 @@ __global__ void __launch_bounds__(NL_WORKERS, 1) nl_qkv_kernel(const __grid_cons
   if (threadIdx.x == 0) NL_TRACE(3);
   if (warp == 1) {
     tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(512));
+    tmem_dealloc<1, 512>(tmem_base);
   }
 }
 
 // ---------------------------------------------------------------------------------------------------------------- host
-static bool nl_encode(CUtensorMap* m, CUtensorMapDataType dt, const void* ptr, int rank, const cuuint64_t* dims,
-                      const cuuint64_t* strides, const cuuint32_t* box, CUtensorMapSwizzle swz) {
-  EncodeTiledFn enc = get_tensormap_encoder();
-  if (!enc) return false;
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  return enc(m, dt, rank, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
-             CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 static long long* g_nl_trace = nullptr;
 
 // pixels per a_mode 2 tile: one pixel per worker warp (its T rows live in that warp's registers), PL * T rows <= 128
@@ -384,36 +371,27 @@ extern "C" int fdm_norm_linear(const fdm_norm_linear_args* a, void* stream) {
   } else {
     p.tiles = (p.M + 127) / 128;
   }
-  const CUtensorMapDataType BF = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+  const CUtensorMapL2promotion L2 = CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
   CUtensorMap tw, ty;
   {
-    cuuint64_t dims[3] = {(cuuint64_t)NL_K, (cuuint64_t)a->Cout, 1};
-    cuuint64_t strides[2] = {(cuuint64_t)NL_K * 2, (cuuint64_t)a->Cout * NL_K * 2};
-    cuuint32_t box[3] = {64, 128, 1};
-    FDM_REQUIRE(nl_encode(&tw, BF, a->w, 3, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B), FDM_ERR_UNSUPPORTED);
+    const cuuint64_t dims[3] = {(cuuint64_t)NL_K, (cuuint64_t)a->Cout, 1};
+    const cuuint32_t box[3] = {64, 128, 1};
+    FDM_REQUIRE(encode_bf16_map(&tw, a->w, 3, dims, box, L2), FDM_ERR_UNSUPPORTED);
   }
   if (a->a_mode == 1) {
-    cuuint64_t ydims[3] = {(cuuint64_t)a->Cout, (cuuint64_t)p.M, 1};
-    cuuint64_t ystrides[2] = {(cuuint64_t)a->Cout * 2, (cuuint64_t)p.M * a->Cout * 2};
-    cuuint32_t ybox[3] = {64, 128, 1};
-    FDM_REQUIRE(nl_encode(&ty, BF, a->y_op, 3, ydims, ystrides, ybox, CU_TENSOR_MAP_SWIZZLE_128B), FDM_ERR_UNSUPPORTED);
+    const cuuint64_t ydims[3] = {(cuuint64_t)a->Cout, (cuuint64_t)p.M, 1};
+    const cuuint32_t ybox[3] = {64, 128, 1};
+    FDM_REQUIRE(encode_bf16_map(&ty, a->y_op, 3, ydims, ybox, L2), FDM_ERR_UNSUPPORTED);
   } else {
     // [B*T][HW][Cout] as (channel, pixel, frame, video): a tile = PL pixels x all T frames of one video, rows ordered (frame, pixel)
-    cuuint64_t ydims[4] = {(cuuint64_t)a->Cout, (cuuint64_t)a->HW, (cuuint64_t)a->T, (cuuint64_t)a->B};
-    cuuint64_t ystrides[3] = {(cuuint64_t)a->Cout * 2, (cuuint64_t)a->HW * a->Cout * 2, (cuuint64_t)a->T * a->HW * a->Cout * 2};
-    cuuint32_t ybox[4] = {64, (cuuint32_t)p.PL, (cuuint32_t)a->T, 1};
-    FDM_REQUIRE(nl_encode(&ty, BF, a->y_op, 4, ydims, ystrides, ybox, CU_TENSOR_MAP_SWIZZLE_128B), FDM_ERR_UNSUPPORTED);
+    const cuuint64_t ydims[4] = {(cuuint64_t)a->Cout, (cuuint64_t)a->HW, (cuuint64_t)a->T, (cuuint64_t)a->B};
+    const cuuint32_t ybox[4] = {64, (cuuint32_t)p.PL, (cuuint32_t)a->T, 1};
+    FDM_REQUIRE(encode_bf16_map(&ty, a->y_op, 4, ydims, ybox, L2), FDM_ERR_UNSUPPORTED);
   }
   constexpr int SMEM_MAX = 225 * 1024;  // + ~1.6 KB of static shared memory (barriers, bias) <= 227 KB
   const int smem = a->Cout * NL_K * 2 + NL_A_BYTES + (a->Cout / 64) * NL_STG_BLOCK + 1024;
   FDM_REQUIRE(smem <= SMEM_MAX, FDM_ERR_UNSUPPORTED);
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] { attr_err = cudaFuncSetAttribute(nl_qkv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_MAX); });
-  if (attr_err != cudaSuccess) {
-    set_last_error(attr_err);
-    return FDM_ERR_CUDA;
-  }
+  if (int rc = allow_smem(nl_qkv_kernel, SMEM_MAX)) return rc;
   const int items = p.tiles * p.NS;
   const int grid = items < 148 ? items : 148;
   fdm::launch(nl_qkv_kernel, dim3(grid), dim3(NL_WORKERS), (size_t)smem, reinterpret_cast<cudaStream_t>(stream), tw, ty, p);

@@ -7,7 +7,6 @@
 // and the epilogue writes the bf16 (and/or fp32) table with coalesced row segments.  Replaces fdm_rpe_hidden + one fdm_conv per
 // net (22 launches, the hidden tensors written and re-read) on inference plans.
 #include "tc_common.cuh"
-#include <mutex>
 #include <string.h>
 
 namespace fdm {
@@ -53,18 +52,15 @@ __global__ void __launch_bounds__(128) rpe_tables_kernel(const RtParams p) {
   if (tid == 0) {
     // the tensor map lives in global memory (written by the host before the first launch): make it visible to the TMA unit
     asm volatile("fence.proxy.tensormap::generic.acquire.gpu [%0], 128;" ::"l"(wmap) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(wmap) : "memory");
+    prefetch_tmap(wmap);
     for (int i = 0; i < 2; ++i) {
       mbar_init(&w_full[i], 1);
       mbar_init(&mma_done[i], 1);
     }
     mbar_init(&bar_d, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"(tmem_cols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc(&tmem_slot, tmem_cols);
   const int kchunks = (C + 63) / 64;
   for (int c = tid; c < kchunks * 64; c += 128)  // parameters: not produced by the previous kernel, safe before pdl_wait
     coef_s[c] = c < C ? make_float4(__ldg(pr.wd + c * 3), __ldg(pr.wd + c * 3 + 1), __ldg(pr.wd + c * 3 + 2), __ldg(pr.bd + c))
@@ -178,7 +174,7 @@ __global__ void __launch_bounds__(128) rpe_tables_kernel(const RtParams p) {
   __syncthreads();
   if (warp == 1) {
     tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(tmem_cols));
+    tmem_dealloc(tmem, tmem_cols);
   }
 }
 
@@ -196,21 +192,15 @@ extern "C" int fdm_rpe_tables_prepare(const fdm_rpe_table_problem* problems, int
   FDM_REQUIRE(problems && count > 0 && host_blob, FDM_ERR_BAD_ARG);
   FDM_REQUIRE(blob_bytes >= fdm_rpe_tables_blob_bytes(count), FDM_ERR_BAD_ARG);
   static_assert(sizeof(CUtensorMap) == 128, "CUtensorMap is 128 bytes");
-  EncodeTiledFn enc = get_tensormap_encoder();
-  FDM_REQUIRE(enc != nullptr, FDM_ERR_UNSUPPORTED);
   uint8_t* blob = reinterpret_cast<uint8_t*>(host_blob);
   for (int i = 0; i < count; ++i) {
     const fdm_rpe_table_problem& q = problems[i];
     FDM_REQUIRE(q.wd && q.bd && q.bo && q.w_packed && (q.out_op || q.out_f32) && q.C > 0 && q.C % 8 == 0 && q.te_off % 4 == 0, FDM_ERR_BAD_ARG);
     const int ci_pad = (q.C + 63) / 64 * 64, co_pad = (q.C + 15) / 16 * 16;
     CUtensorMap m;
-    cuuint64_t dims[3] = {(cuuint64_t)ci_pad, (cuuint64_t)co_pad, 1};
-    cuuint64_t strides[2] = {(cuuint64_t)ci_pad * 2, (cuuint64_t)co_pad * ci_pad * 2};
-    cuuint32_t box[3] = {64, 128, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    FDM_REQUIRE(enc(&m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(q.w_packed), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS, FDM_ERR_UNSUPPORTED);
+    const cuuint64_t dims[3] = {(cuuint64_t)ci_pad, (cuuint64_t)co_pad, 1};
+    const cuuint32_t box[3] = {64, 128, 1};
+    FDM_REQUIRE(encode_bf16_map(&m, q.w_packed, 3, dims, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B), FDM_ERR_UNSUPPORTED);
     memcpy(blob + (size_t)i * sizeof(CUtensorMap), &m, sizeof(CUtensorMap));
     RtProblem d{q.wd, q.bd, q.bo, reinterpret_cast<__nv_bfloat16*>(q.out_op), q.out_f32, q.C, q.te_off};
     memcpy(blob + (size_t)count * sizeof(CUtensorMap) + (size_t)i * sizeof(RtProblem), &d, sizeof(RtProblem));
@@ -226,17 +216,11 @@ extern "C" int fdm_rpe_tables(const fdm_rpe_tables_args* a, void* stream) {
   p.probs = reinterpret_cast<const RtProblem*>(reinterpret_cast<const uint8_t*>(a->blob) + (size_t)a->count * sizeof(CUtensorMap));
   p.te = a->te; p.fi = a->frame_indices; p.B = a->B; p.T = a->T; p.te_stride = a->te_stride;
   p.M = a->B * a->T * a->T;
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] { attr_err = cudaFuncSetAttribute(rpe_tables_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); });
-  if (attr_err != cudaSuccess) {
-    set_last_error(attr_err);
-    return FDM_ERR_CUDA;
-  }
   FDM_REQUIRE(a->max_C <= 512 && a->te_stride % 4 == 0, FDM_ERR_UNSUPPORTED);  // one CTA holds all C output channels of its rows in TMEM (512 columns)
   p.wstage = (a->max_C + 127) / 128 * 128 * 128;
   const int smem_bytes = 2 * 16384 + 2 * p.wstage + (a->max_C + 63) / 64 * 64 * 16 + 1024;
   dim3 grid((p.M + 127) / 128, 1, a->count);
+  if (int rc = allow_smem(rpe_tables_kernel, 200 * 1024)) return rc;
   fdm::launch(rpe_tables_kernel, grid, dim3(128), smem_bytes, (cudaStream_t)stream, p);
   return check_launch();
 }

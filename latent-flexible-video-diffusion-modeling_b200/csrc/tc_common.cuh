@@ -1,4 +1,4 @@
-// tcgen05 / TMA / mbarrier PTX wrappers shared by the tensor-core kernels (conv_tc.cu, attn_tc.cu).  sm_100a only.
+// tcgen05 / TMA / mbarrier PTX wrappers and the tensor-map encoder shared by the tensor-core kernels.  sm_100a only.
 #pragma once
 #include "common.cuh"
 #include <cuda.h>
@@ -34,6 +34,38 @@ __device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, u
   asm volatile(
       "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
       ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2) : "memory");
+}
+// barrier initialisation made visible to the async proxy (TMA, tcgen05.commit) and to the other CTAs of the cluster
+__device__ __forceinline__ void fence_mbarrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
+__device__ __forceinline__ void prefetch_tmap(const CUtensorMap* map) { asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory"); }
+// TMEM columns (a power of two >= 32) for this CTA (CG = 1) or this CTA pair (CG = 2), allocated by one whole warp; the base address
+// is written to `slot` in shared memory.  The allocation permit is relinquished at once, so the next CTA on the SM can allocate.
+// tmem_dealloc is issued by the same warp with the same column count.  A compile-time count is passed as an immediate: a register
+// operand moves the register allocation of the kernels around it.
+template <int CG, uint32_t COLS>
+__device__ __forceinline__ void tmem_alloc(uint32_t* slot) {
+  static_assert(CG == 1 || CG == 2, "cta_group::1 or ::2");
+  if constexpr (CG == 2) {
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "n"(COLS));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;");
+  } else {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "n"(COLS));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+  }
+}
+template <int CG, uint32_t COLS>
+__device__ __forceinline__ void tmem_dealloc(uint32_t base) {
+  static_assert(CG == 1 || CG == 2, "cta_group::1 or ::2");
+  if constexpr (CG == 2) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(base), "n"(COLS));
+  else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "n"(COLS));
+}
+// a column count known at run time, single CTA
+__device__ __forceinline__ void tmem_alloc(uint32_t* slot, uint32_t cols) {
+  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "r"(cols));
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+}
+__device__ __forceinline__ void tmem_dealloc(uint32_t base, uint32_t cols) {
+  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "r"(cols));
 }
 __device__ __forceinline__ void tcgen05_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tcgen05_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
@@ -205,9 +237,11 @@ __device__ __forceinline__ uint32_t pack2_bf16(float a, float b) {
   return *reinterpret_cast<uint32_t*>(&v);
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_tensormap_encoder();  // conv_tc.cu
+// Encodes a TMA tensor map over bf16 elements at `ptr`: `rank` dims (innermost first) and box sizes, no interleave, zero fill out
+// of bounds.  `strides` (rank - 1 byte strides of dims 1..rank-1) default to the dense layout of `dims`, `elem_strides` to 1.
+// False when the driver has no encoder or rejects the map.  api.cu
+bool encode_bf16_map(CUtensorMap* map, const void* ptr, int rank, const cuuint64_t* dims, const cuuint32_t* box,
+                     CUtensorMapL2promotion l2, CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_128B,
+                     const cuuint64_t* strides = nullptr, const cuuint32_t* elem_strides = nullptr);
 
 }  // namespace fdm

@@ -15,7 +15,6 @@
 // range of pixel chunks): accumulators stay in TMEM for the whole range (<= 3 x 128 columns), then go to fp32 partials that
 // wgrad_reduce_kernel (bwd_conv.cu) sums in a fixed order.  Roofline: tensor (2*9*Cin*Cout FLOP per pixel).
 #include "tc_common.cuh"
-#include <mutex>
 
 namespace fdm {
 
@@ -43,8 +42,8 @@ __global__ void __launch_bounds__(128, 1) wgrad_tc_kernel(const __grid_constant_
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tx) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tdy) : "memory");
+    prefetch_tmap(&tx);
+    prefetch_tmap(&tdy);
   }
   if (warp == 1 && lane == 0) {
     for (int i = 0; i < p.stages; ++i) {
@@ -52,12 +51,9 @@ __global__ void __launch_bounds__(128, 1) wgrad_tc_kernel(const __grid_constant_
       mbar_init(&empty_bar[i], 1);
     }
     mbar_init(&done_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
-  if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)), "n"(WG_TMEM_COLS));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 2) tmem_alloc<1, WG_TMEM_COLS>(&tmem_base_slot);
   tcgen05_fence_before();
   __syncthreads();
   tcgen05_fence_after();
@@ -140,21 +136,7 @@ __global__ void __launch_bounds__(128, 1) wgrad_tc_kernel(const __grid_constant_
   }
   tcgen05_fence_before();
   __syncthreads();
-  if (warp == 2) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(WG_TMEM_COLS));
-  }
-}
-
-// activations [N][H][W][C] bf16 as a (C, W, H, N) tensor; box (64, W, hrows, 1), 128-byte swizzle, zero fill out of bounds
-static bool wg_encode(CUtensorMap* m, const void* ptr, int N, int H, int W, int C, int hrows) {
-  EncodeTiledFn enc = get_tensormap_encoder();
-  if (!enc) return false;
-  cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
-  cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
-  cuuint32_t box[4] = {64u, (cuuint32_t)W, (cuuint32_t)hrows, 1u};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+  if (warp == 2) tmem_dealloc<1, WG_TMEM_COLS>(tmem_base);
 }
 
 struct WgTcGeom {
@@ -216,16 +198,14 @@ size_t conv_wgrad_tc_partial_bytes(const fdm_conv_wgrad_args* a) {
 int conv_wgrad_tc(const fdm_conv_wgrad_args* a, float* part, int* splits_out, cudaStream_t st) {
   const WgTcGeom g = wg_tc_geom(a);
   if (!g.ok) return FDM_ERR_UNSUPPORTED;
+  // activations [N][H][W][C] as (C, W, H, N) tensors; boxes of 64 channels x W x (hbox + ks - 1 | hbox) rows x 1
+  const cuuint64_t xdims[4] = {(cuuint64_t)a->C, (cuuint64_t)a->Win, (cuuint64_t)a->Hin, (cuuint64_t)a->N};
+  const cuuint64_t dydims[4] = {(cuuint64_t)a->Cout, (cuuint64_t)a->Win, (cuuint64_t)a->Hin, (cuuint64_t)a->N};
+  const cuuint32_t xbox[4] = {64, (cuuint32_t)a->Win, (cuuint32_t)(g.hbox + a->ksize - 1), 1};
+  const cuuint32_t dybox[4] = {64, (cuuint32_t)a->Win, (cuuint32_t)g.hbox, 1};
   CUtensorMap tx, tdy;
-  if (!wg_encode(&tx, a->a, a->N, a->Hin, a->Win, a->C, g.hbox + a->ksize - 1)) return FDM_ERR_UNSUPPORTED;
-  if (!wg_encode(&tdy, a->dy, a->N, a->Hin, a->Win, a->Cout, g.hbox)) return FDM_ERR_UNSUPPORTED;
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] { attr_err = cudaFuncSetAttribute(wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024); });
-  if (attr_err != cudaSuccess) {
-    set_last_error(attr_err);
-    return FDM_ERR_CUDA;
-  }
+  if (!encode_bf16_map(&tx, a->a, 4, xdims, xbox, CU_TENSOR_MAP_L2_PROMOTION_L2_128B)) return FDM_ERR_UNSUPPORTED;
+  if (!encode_bf16_map(&tdy, a->dy, 4, dydims, dybox, CU_TENSOR_MAP_L2_PROMOTION_L2_128B)) return FDM_ERR_UNSUPPORTED;
   WgTcParams p{};
   p.part = part;
   p.C = a->C; p.Cout = a->Cout; p.ks = a->ksize; p.taps = a->ksize * a->ksize;
@@ -246,6 +226,7 @@ int conv_wgrad_tc(const fdm_conv_wgrad_args* a, float* part, int* splits_out, cu
   if (p.a_lbo16 >= (1u << 14) || p.b_lbo16 >= (1u << 14)) return FDM_ERR_UNSUPPORTED;
   dim3 grid(g.ci_chunks * g.co_chunks, a->ksize, g.splits);
   const size_t smem = (size_t)g.stages * g.stage_bytes + 1024;
+  if (int rc = allow_smem(wgrad_tc_kernel, 226 * 1024)) return rc;
   fdm::launch(wgrad_tc_kernel, grid, dim3(128), smem, st, tx, tdy, p);
   *splits_out = g.splits;
   return check_launch();

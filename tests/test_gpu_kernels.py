@@ -4,6 +4,8 @@ reference calls at that site (torch fp32 on the same device).  bf16 tensor-core 
 fp32 op fed the SAME bf16-rounded operands, so the tolerance only has to cover accumulation order (1e-3 rel-L2);
 fp32 CUDA-core results are held to 1e-5.
 """
+import re
+
 import pytest
 import torch
 import torch.nn.functional as F
@@ -150,6 +152,19 @@ def test_wide_pointwise_vs_torch(case):
         assert rel(stats, ref_stats) <= 1e-3
 
 
+def run_head_conv(x, w0p, bias, Co, engine):
+    """fdm_conv in the head form: 3x3, NCHW fp32 output.  x [N,H,W,C0] bf16, w0p packed by pack_tc.  Returns y [N,Co,H,W]."""
+    from improved_diffusion import _native as N_
+    N, H, W, C0 = x.shape
+    y = torch.full((N, Co, H, W), float("nan"), device="cuda")
+    a = N_.ConvArgs(a0=x.data_ptr(), w0=w0p.data_ptr(), a1=None, w1=None, bias=bias.data_ptr(), resid=None, y_f32=y.data_ptr(),
+                    y_op=None, stats=None, N=N, Hin=H, Win=W, C0=C0, C1=0, Cout=Co, ksize=3, stride=1, upsample=0,
+                    a_dtype=N_.BF16, op_dtype=N_.BF16, out_nchw=1, engine=engine)
+    N_.call("fdm_conv", a, torch.cuda.current_stream().cuda_stream)
+    torch.cuda.synchronize()
+    return y
+
+
 @pytest.mark.parametrize("case", [
     # N, H, W, C0, Cout
     (20, 32, 32, 64, 4),    # cfg4 head
@@ -170,17 +185,10 @@ def test_head_conv_vs_torch(case):
     w0p = pack_tc(w)
     outs = []
     for engine in (N_.CONV_TC, N_.CONV_TC_TAP):
-        y = torch.full((N, Co, H, W), float("nan"), device="cuda")
-        a = N_.ConvArgs(a0=x.data_ptr(), w0=w0p.data_ptr(), a1=None, w1=None, bias=bias.data_ptr(), resid=None, y_f32=y.data_ptr(),
-                        y_op=None, stats=None, N=N, Hin=H, Win=W, C0=C0, C1=0, Cout=Co, ksize=3, stride=1, upsample=0,
-                        a_dtype=N_.BF16, op_dtype=N_.BF16, out_nchw=1, engine=engine)
         try:
-            N_.call("fdm_conv", a, torch.cuda.current_stream().cuda_stream)
+            outs.append(run_head_conv(x, w0p, bias, Co, engine))
         except N_.NativeError:
             assert engine == N_.CONV_TC_TAP  # the per-tap kernel does not take every map shape; the head kernel must
-            continue
-        torch.cuda.synchronize()
-        outs.append(y)
     ref = F.conv2d(x.float().permute(0, 3, 1, 2), w.to(torch.bfloat16).float(), bias, padding=1)
     assert rel(outs[0], ref) <= 1e-3, rel(outs[0], ref)
     if len(outs) > 1:
@@ -526,12 +534,8 @@ def test_norm_linear_qkv(B, T, HW, a_mode):
         assert rel(tstats[..., 1], (var + eps).rsqrt().float()) <= 1e-4
 
 
-@pytest.mark.parametrize("B,T,HW", NL_SHAPES)
-@pytest.mark.parametrize("resid_norm", [2, 3])
-def test_conv_proj_recomputed_groupnorm_residual(B, T, HW, resid_norm):
-    """fdm_conv (per-tap tcgen05 engine), proj_out form: the residual is GroupNorm(x) RECOMPUTED in the epilogue — temporal GN from
-    the saved (mean, rstd) pairs (resid_norm 2) / per-frame GN from the sums (resid_norm 3) — instead of a normalised fp32 copy
-    (rpe.py:136,173); fp32 + bf16 outputs and the GroupNorm statistics of the result."""
+def run_proj_recomputed_gn(B, T, HW, resid_norm):
+    """fdm_conv in the proj_out form with resid_norm 2 | 3 on the inputs of _nl_inputs.  Returns (y, y_op, stats, torch reference)."""
     from improved_diffusion import _native as N_
     C, eps = 128, 1e-5
     x, gamma, beta, w, bias, g = _nl_inputs(B, T, HW, C, seed=B * 1000 + T * 10 + resid_norm + 5)
@@ -553,8 +557,70 @@ def test_conv_proj_recomputed_groupnorm_residual(B, T, HW, resid_norm):
                     rn_beta=beta.data_ptr())
     N_.call("fdm_conv", a, torch.cuda.current_stream().cuda_stream)
     torch.cuda.synchronize()
-    ref = h.float() @ wp.float().t() + bias + r
+    return y, yop, ostats, h.float() @ wp.float().t() + bias + r
+
+
+@pytest.mark.parametrize("B,T,HW", NL_SHAPES)
+@pytest.mark.parametrize("resid_norm", [2, 3])
+def test_conv_proj_recomputed_groupnorm_residual(B, T, HW, resid_norm):
+    """fdm_conv (per-tap tcgen05 engine), proj_out form: the residual is GroupNorm(x) RECOMPUTED in the epilogue — temporal GN from
+    the saved (mean, rstd) pairs (resid_norm 2) / per-frame GN from the sums (resid_norm 3) — instead of a normalised fp32 copy
+    (rpe.py:136,173); fp32 + bf16 outputs and the GroupNorm statistics of the result."""
+    y, yop, ostats, ref = run_proj_recomputed_gn(B, T, HW, resid_norm)
     assert rel(y, ref) <= 2e-5, rel(y, ref)
     assert rel(yop.float(), ref) <= 4e-3
-    rs = _frame_stats(ref.view(B * T, HW, C))
+    rs = _frame_stats(ref.view(B * T, HW, -1))
     assert rel(ostats, rs) <= 1e-5, rel(ostats, rs)
+
+
+def _fdm_kernels(fn):
+    """names of the library's kernels (namespace fdm) that torch.profiler records while fn() runs"""
+    from torch.profiler import ProfilerActivity, profile
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    return [e.name for e in prof.events() if "fdm::" in e.name]
+
+
+def _run_conv_case(case, **kw):
+    """run_conv (tcgen05 engines) on random operands of a (N, H, W, C0, Cout, k) case"""
+    from improved_diffusion import _native as N_
+    N, H, W, C0, Co, k = case
+    g = torch.Generator(device="cuda").manual_seed(sum(case))
+    x = torch.randn(N, H, W, C0, device="cuda", generator=g).to(torch.bfloat16)
+    w = torch.randn(Co, C0, k, k, device="cuda", generator=g) / (C0 * k * k) ** 0.5
+    bias = 0.1 * torch.randn(Co, device="cuda", generator=g)
+    return run_conv(x, w, bias, engine=N_.CONV_TC, want_op=True, **kw)
+
+
+def _run_head_case(case):
+    from improved_diffusion import _native as N_
+    N, H, W, C0, Co = case
+    g = torch.Generator(device="cuda").manual_seed(sum(case))
+    x = torch.randn(N, H, W, C0, device="cuda", generator=g).to(torch.bfloat16)
+    w = torch.randn(Co, C0, 3, 3, device="cuda", generator=g) / (9 * C0) ** 0.5
+    return run_head_conv(x, pack_tc(w), 0.1 * torch.randn(Co, device="cuda", generator=g), Co, N_.CONV_TC)
+
+
+# route -> (launch, pattern of the demangled kernel name: template arguments <BN, TPI, CG, UP> of the halo kernel, <BN, RN> of the
+# per-tap kernel), with case shapes of test_head_conv_vs_torch, test_conv_tc_vs_torch, test_wide_pointwise_vs_torch and
+# test_conv_proj_recomputed_groupnorm_residual
+CONV_ROUTES = {
+    "head": (lambda: _run_head_case((20, 32, 32, 64, 4)), r"\bconv_head_kernel\("),
+    "halo": (lambda: _run_conv_case((5, 32, 32, 64, 64, 3)), r"\bconv_halo_kernel<\d+, \d+, 1, false>"),
+    "halo_cta_pair": (lambda: _run_conv_case((80, 32, 32, 192, 64, 3)), r"\bconv_halo_kernel<\d+, \d+, 2, false>"),
+    "halo_pointwise": (lambda: _run_conv_case((16, 16, 16, 384, 1152, 1), want_stats=False), r"\bconv_halo_kernel<\d+, \d+, 1, false>"),
+    "tap_3x3_8x8": (lambda: _run_conv_case((5, 8, 8, 128, 128, 3)), r"\bconv_tc_kernel<\d+, false>"),
+    "tap_1x1_resid_norm": (lambda: run_proj_recomputed_gn(8, 20, 256, 2), r"\bconv_tc_kernel<\d+, true>"),
+}
+
+
+@pytest.mark.parametrize("route", list(CONV_ROUTES))
+def test_conv_dispatch_runs_the_expected_kernel(route):
+    """fdm_conv with engine FDM_CONV_TC picks one of three tcgen05 kernels by shape, and a kernel that refuses a shape (including a
+    tensor map the driver rejects) hands it on to the per-tap kernel, which computes the same result more slowly.  The result
+    tests cannot tell the kernels apart: this pins which one each route launches, and that it is the only launch."""
+    run, kernel = CONV_ROUTES[route]
+    names = _fdm_kernels(run)
+    assert len(names) == 1 and re.search(kernel, names[0]), names
